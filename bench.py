@@ -3,6 +3,9 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            one rank per GPU (torchrun for N > 1)
     python bench.py --impl reference ...                           the reference's own CPU code on the host cores
+    python bench.py --dump-outputs DIR ...                         also write the last timed step's film to DIR/*.npy
+                                                                   (one GPU, or N > 1 with --merge nccl: the default sharded
+                                                                   merge leaves the film split over the ranks, and is refused)
 
 One "step" is one complete render of the workload: every pixel, all its samples, film accumulated, and (N > 1) the
 per-GPU films combined.  Default workload = BASELINE.json configs[1] / the north-star target: init_cornell.scn, 1024x1024,
@@ -23,6 +26,7 @@ import threading
 import time
 
 REPO = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True          # the tree may be read-only: the benchmark leaves nothing in it
 sys.path.insert(0, REPO)
 sys.path.insert(0, os.path.join(REPO, "tests"))
 
@@ -60,7 +64,15 @@ def parse_args():
     ap.add_argument("--merge", default="sharded", choices=["sharded", "nccl"],
                     help="multi-GPU film combination: sharded = render kernel scatters finished pixels to their owner over NVLink, "
                          "device-side flags, local merge, film stays sharded (default); nccl = 2 all_reduce + 1 reduce")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the film of the last timed step to DIR/<plane>.npy (float32; a fixed, seeded "
+                         "sample of pixels when the whole film is over 60 MB, their indices in pixel_index.npy) to compare two builds")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.gpus > 1 and a.merge == "sharded":
+        ap.error("--dump-outputs needs one GPU or --merge nccl (the sharded film is never whole on one device)")
+    return a
 
 
 def samples(a, world):
@@ -475,6 +487,8 @@ def run_b200_arm(a):
     ms_step, launches_step, ev = timed(prm, a.steps)
     t1 = time.perf_counter()
     clocks = sampler.stop(t0, t1) if sampler else None
+    if a.dump_outputs and rank == 0:
+        dump_film(a.dump_outputs, film, npix, n, a.seed)
     kernel_ms = sum(m["start"].elapsed_time(m["render"]) for m in ev) / len(ev)
     exchange_ms = None
     if group is not None:
@@ -684,6 +698,21 @@ def run_b200_arm(a):
     ctx.close()
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_film(out_dir, film, npix, n, seed, budget=60_000_000):
+    """The four film planes a caller of the render receives, as float32 .npy files.  A film over `budget` bytes is sampled: the
+    same pixels (drawn from `seed`) every run, so that two builds can be compared plane by plane."""
+    import numpy as np
+    import torch
+    per_pixel = (3 * n + 1) * 4 + 8
+    k = min(npix, budget // per_pixel)
+    idx = np.arange(npix) if k == npix else np.sort(np.random.default_rng(seed).choice(npix, k, replace=False))
+    sel = torch.from_numpy(idx).to(film.sum.device)
+    os.makedirs(out_dir, exist_ok=True)
+    for name in ("sum", "filter", "mean", "m2"):
+        np.save(os.path.join(out_dir, name + ".npy"), getattr(film, name).index_select(0, sel).cpu().numpy())
+    np.save(os.path.join(out_dir, "pixel_index.npy"), idx.astype(np.float64))
 
 
 def image_check(a, arm, ctx, common, cfg, planes, n, spp_total, world):

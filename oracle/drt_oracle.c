@@ -573,14 +573,10 @@ static void cast_ray(ctx *c, double *dst, v3 origin, v3 dir, uint32_t max_depth)
     else c->count->reached_depth_cap += 1;
 }
 
-/* sample_scene, daily_ray_trace.c:571-618 (sample_pixel_point :550-569) */
-static void sample_scene(ctx *c, double *contribution, double *filter, uint32_t x, uint32_t y, uint32_t max_depth, int scheme)
+/* the camera ray of sample_scene, daily_ray_trace.c:571-612 (sample_pixel_point :550-569) */
+static void camera_ray(ctx *c, uint32_t x, uint32_t y, int scheme, v3 *origin_out, v3 *dir_out)
 {
     const drt_camera *cam = c->cam;
-    int n = c->n;
-    memset(contribution, 0, sizeof(double) * (size_t)n);
-    c->count->paths += 1;
-
     double px = 0.0, py = 0.0;
     if(scheme == DRT_PIXEL_CENTER) { px = 0.5; py = 0.5; }
     else if(scheme == DRT_PIXEL_RANDOM) { px = rng(c); py = rng(c); }
@@ -610,6 +606,19 @@ static void sample_scene(ctx *c, double *contribution, double *filter, uint32_t 
         origin = point;
         dir = v3_normalise(v3_sub(aperture, origin));   /* Q1: film sits behind the pinhole, image comes out rotated */
     }
+    *origin_out = origin;
+    *dir_out = dir;
+}
+
+/* sample_scene, daily_ray_trace.c:571-618 */
+static void sample_scene(ctx *c, double *contribution, double *filter, uint32_t x, uint32_t y, uint32_t max_depth, int scheme)
+{
+    int n = c->n;
+    memset(contribution, 0, sizeof(double) * (size_t)n);
+    c->count->paths += 1;
+
+    v3 origin, dir, forward = v3_make(c->cam->forward);
+    camera_ray(c, x, y, scheme, &origin, &dir);
     cast_ray(c, contribution, origin, dir, max_depth);
 
     double vignette = v3_dot(dir, forward);   /* Q20 */
@@ -661,4 +670,38 @@ void drt_oracle_render_tile(const drt_scene *scene, const drt_camera *camera, co
             d_m2[i] = d_m2[i] + (delta * (contribution[i] - d_avg[i]));
         }
     }
+}
+
+/* The material the camera ray of sample `sample` of pixel (x, y) hits first (the escape material when it hits nothing). */
+int drt_oracle_primary_material(const drt_scene *scene, const drt_camera *camera, const drt_render_params *params,
+                                uint32_t x, uint32_t y, uint32_t sample)
+{
+    drt_oracle_counters local;
+    memset(&local, 0, sizeof(local));
+    ctx c = { scene, camera, scene->num_wavelengths, {0}, &local };
+    drt_rng_begin(&c.rng, params->seed, y * params->width + x, sample);
+    v3 origin, dir;
+    camera_ray(&c, x, y, params->pixel_scheme, &origin, &dir);
+    hit_point hit;
+    memset(&hit, 0, sizeof(hit));
+    find_intersection(&c, &hit, origin, dir);
+    return (int)(hit.surface_material - scene->materials);
+}
+
+/* bdsf() at a hand-built hit point, set up as oracle/ref_perpath.c's ref_bdsf does (on_dot = n.out, trans_wl 630 nm):
+ * the CPU-tier check of the classed kernel's factorisation where the reference build is absent. */
+void drt_oracle_bdsf(const drt_scene *scene, uint32_t surface_material, uint32_t incident_material, uint32_t transmit_material,
+                     const double *normal, const double *out_dir, const double *in_dir, double *result)
+{
+    ctx c = { scene, NULL, scene->num_wavelengths, {0}, NULL };
+    hit_point p;
+    memset(&p, 0, sizeof(p));
+    p.normal = v3_make(normal);
+    p.out = v3_make(out_dir);
+    p.on_dot = v3_dot(p.normal, p.out);
+    p.trans_wl = 630.0;
+    p.surface_material = &scene->materials[surface_material];
+    p.incident_material = &scene->materials[incident_material];
+    p.transmit_material = &scene->materials[transmit_material];
+    bdsf(&c, result, &p, v3_make(in_dir));
 }

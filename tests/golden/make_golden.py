@@ -30,13 +30,14 @@ CASES = [
     ("cornell_downward", 48, 48, (16, 16, 32, 32), 2, 4, "pixel_random", 14),
     ("first_scene", 32, 32, (8, 8, 24, 24), 2, 4, "pixel_center", 15),
     ("example_scene", 32, 32, (8, 8, 24, 24), 1, 3, "pixel_random", 16),
-    ("stress_all", 64, 48, (16, 8, 40, 24), 2, 6, "pixel_random", 17),
+    # tiles of stress_all and classed_all are sized to keep each fixture under 1 MB; classed_all's still sees all nine materials
+    ("stress_all", 64, 48, (16, 8, 39, 24), 2, 6, "pixel_random", 17),
     ("rotated_room", 64, 48, (20, 12, 44, 28), 2, 5, "pixel_random", 18),
     # pinhole camera + EMISSIVE escape material (Q19 environment light): the tile straddles the scene's screen-space edge
     ("sky_cornell", 64, 48, (0, 8, 24, 24), 2, 4, "pixel_random", 19),
     # one light, pinhole: every material class of the classed compact-record kernel (plastics with repeated / single lobes and a
     # uniform-hemisphere sampler, mirror, fs_conductor, glass R+T, transmittance only, ct_conductor)
-    ("classed_all", 64, 48, (8, 8, 56, 32), 2, 6, "pixel_random", 20),
+    ("classed_all", 64, 48, (12, 20, 48, 30), 2, 6, "pixel_random", 20),
 ]
 
 

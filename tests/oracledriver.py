@@ -26,8 +26,8 @@ _lib = None
 def lib():
     global _lib
     if _lib is None:
-        if not os.path.exists(ORACLE_LIB):
-            subprocess.check_call(["make", "-C", ORACLE_DIR, "oracle"])
+        # make rebuilds a library older than drt_oracle.c (one without the newer exports) and does nothing otherwise
+        subprocess.check_call(["make", "-s", "-C", ORACLE_DIR, "oracle"], stdout=subprocess.DEVNULL)
         L = C.CDLL(ORACLE_LIB)
         dp = C.POINTER(C.c_double)
         L.drt_oracle_sample.argtypes = [C.POINTER(_structs.Scene), C.POINTER(_structs.Camera), C.POINTER(_structs.RenderParams),
@@ -36,6 +36,11 @@ def lib():
         L.drt_oracle_render_tile.argtypes = [C.POINTER(_structs.Scene), C.POINTER(_structs.Camera), C.POINTER(_structs.RenderParams),
                                              C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, dp, dp, dp, dp, C.POINTER(Counters)]
         L.drt_oracle_render_tile.restype = None
+        L.drt_oracle_bdsf.argtypes = [C.POINTER(_structs.Scene), C.c_uint32, C.c_uint32, C.c_uint32, dp, dp, dp, dp]
+        L.drt_oracle_bdsf.restype = None
+        L.drt_oracle_primary_material.argtypes = [C.POINTER(_structs.Scene), C.POINTER(_structs.Camera), C.POINTER(_structs.RenderParams),
+                                                  C.c_uint32, C.c_uint32, C.c_uint32]
+        L.drt_oracle_primary_material.restype = C.c_int
         _lib = L
     return _lib
 
@@ -53,6 +58,19 @@ def sample(scene, camera, prm, x, y, s):
     filt = C.c_double()
     lib().drt_oracle_sample(C.byref(scene), C.byref(camera), C.byref(prm), x, y, s, _p(out), C.byref(filt), None)
     return out
+
+
+def primary_material(scene, camera, prm, x, y, s):
+    """Index of the material the camera ray of path (x, y, s) hits first."""
+    return lib().drt_oracle_primary_material(C.byref(scene), C.byref(camera), C.byref(prm), x, y, s)
+
+
+def bdsf(scene, surf_mat, inc_mat, trans_mat, normal, out_dir, in_dir):
+    """The material's bdsf() sum for one incoming direction (the arguments of refdriver.Ref.bdsf)."""
+    a = [np.ascontiguousarray(v, dtype=np.float64) for v in (normal, out_dir, in_dir)]
+    res = np.zeros(scene.num_wavelengths)
+    lib().drt_oracle_bdsf(C.byref(scene), surf_mat, inc_mat, trans_mat, _p(a[0]), _p(a[1]), _p(a[2]), _p(res))
+    return res
 
 
 def render_tile(scene, camera, prm, x0, y0, x1, y1, want_paths=False):

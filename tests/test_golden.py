@@ -61,12 +61,55 @@ def test_host_setup_matches_reference_fixture(host, name):
 
 
 @pytest.mark.parametrize("name", NAMES)
+def test_spectral_helpers_match_reference_fixture(host, name):
+    """drt_rgb_to_spectrum and drt_blackbody_spectrum called directly on every rgb / blackbody input of the scene, bit-for-bit
+    against the reference's material spectra (init_spd, daily_ray_trace.c:79-123: blackbody normalised to its peak, then the scale)."""
+    import ctypes as C
+    z, meta, cfg, tables, scene, cam = _load(name)
+    parsed = host.parse_scene_text(open(common.scene_path(name)).read())
+    inputs = {parsed.materials[j].name: parsed.materials[j] for j in range(parsed.num_materials)}
+    L = host.lib()
+    dp = C.POINTER(C.c_double)
+    n = scene.num_wavelengths
+    checked = 0
+    for i in range(scene.num_materials):
+        m = inputs.get(scene.materials[i].name)
+        for k in range(6) if m is not None else ():
+            spd = m.spd[k]
+            out = np.zeros(n)
+            if spd.method == 1:
+                rgb = np.array(spd.rgb[:])
+                L.drt_rgb_to_spectrum(C.byref(tables), rgb.ctypes.data_as(dp), out.ctypes.data_as(dp))
+            elif spd.method == 3:
+                L.drt_blackbody_spectrum(C.byref(tables), spd.value, out.ctypes.data_as(dp))
+                out = out / out.max()
+            else:
+                continue
+            if spd.has_scale:
+                out = out * spd.scale
+            assert np.array_equal(out, z["mat_spds"][i][k]), (scene.materials[i].name, k)
+            checked += 1
+    assert checked > 0
+    print(f"\n{name}: {checked} rgb / blackbody spectra")
+
+
+@pytest.mark.parametrize("name", NAMES)
 def test_oracle_matches_reference_fixture(name):
     z, (w, h, x0, y0, x1, y1, spp, depth, scheme, seed), cfg, tables, scene, cam = _load(name)
     prm = oracledriver.params(w, h, 0, spp, depth, scheme, seed)
     o_sum, o_avg, o_m2, o_paths, cnt = oracledriver.render_tile(scene, cam, prm, x0, y0, x1, y1, want_paths=True)
     assert _same(o_paths, z["paths"])
     assert _same(o_sum, z["film_sum"]) and _same(o_avg, z["film_mean"]) and _same(o_m2, z["film_m2"])
+
+
+def test_classed_all_tile_sees_every_material():
+    """The classed_all fixture's tile is cut to stay under 1 MB; its camera rays must still hit every material of the scene's surfaces
+    (all classes of the classed kernel) other than the light, which the tile does not see."""
+    z, (w, h, x0, y0, x1, y1, spp, depth, scheme, seed), cfg, tables, scene, cam = _load("classed_all")
+    prm = oracledriver.params(w, h, 0, spp, depth, scheme, seed)
+    hit = {oracledriver.primary_material(scene, cam, prm, x, y, s) for y in range(y0, y1) for x in range(x0, x1) for s in range(spp)}
+    want = {scene.surfaces[i].material for i in range(scene.num_surfaces) if not scene.materials[scene.surfaces[i].material].is_emissive}
+    assert len(want) == 9 and want <= hit, sorted(scene.materials[m].name.decode() for m in want - hit)
 
 
 @pytest.mark.gpu

@@ -1,7 +1,8 @@
 """Host C front-end (product) pinned bit-for-bit against the unmodified reference's own parse/setup code.
 
-Needs oracle/_ref (built where /root/reference exists); the committed fixtures in tests/golden cover the same
-ground on machines without it (test_golden.py)."""
+The comparisons with the reference need oracle/_ref (built by oracle/Makefile where the reference sources are present).  Without
+it, test_golden.py compares scene, camera, tables and the rgb / blackbody spectra with stored reference fixtures; material names,
+spectrum -> RGB and the 8-bit conversion are compared with the reference only here."""
 import os
 
 import numpy as np
@@ -9,7 +10,7 @@ import pytest
 
 import refdriver
 
-pytestmark = pytest.mark.skipif(not refdriver.available(), reason="oracle/_ref not built")
+needs_ref = pytest.mark.skipif(not refdriver.available(), reason="oracle/_ref not built")
 
 SCENES = ["cornell_plane_light", "init_cornell", "cornell_large_box", "cornell_downward", "first_scene", "example_scene"]
 
@@ -24,15 +25,25 @@ def _load_both(host, assets, tmp_path, scene, w=48, h=32):
     cfg = host.parse_config_text(cfg_text)
     tables = host.load_tables(cfg, assets)
     mine = host.load_scene_file(assets, f"scenes/{scene}.scn", tables, w, h)
-    # the upgraded text must parse to the same scene under the STRICT (reference) grammar
-    again = host.load_scene_file(root, "scenes/upgraded.scn", tables, w, h, flags=0)
-    return ref, tables, mine, again
+    return ref, tables, mine
 
 
 @pytest.mark.parametrize("scene", SCENES)
-def test_scene_and_camera_bit_exact(host, assets, tmp_path, scene):
-    ref, tables, (sc, cam), (sc2, cam2) = _load_both(host, assets, tmp_path, scene)
+def test_upgraded_text_reparses_to_the_same_scene(host, assets, tmp_path, scene):
+    """The text scene_to_text upgrades a legacy scene to parses to the same scene and camera under the STRICT (reference) grammar."""
+    w, h = 48, 32
+    parsed = host.parse_scene_text(open(os.path.join(assets, "scenes", scene + ".scn")).read())
+    root = refdriver.make_root(str(tmp_path), assets, host.scene_to_text(parsed), "upgraded.scn")
+    tables = host.load_tables(host.parse_config_text(host.make_config_text(width=w, height=h)), assets)
+    sc, cam = host.load_scene_file(assets, f"scenes/{scene}.scn", tables, w, h)
+    sc2, cam2 = host.load_scene_file(root, "scenes/upgraded.scn", tables, w, h, flags=0)
     assert bytes(sc) == bytes(sc2) and bytes(cam)[:160] == bytes(cam2)[:160]
+
+
+@needs_ref
+@pytest.mark.parametrize("scene", SCENES)
+def test_scene_and_camera_bit_exact(host, assets, tmp_path, scene):
+    ref, tables, (sc, cam) = _load_both(host, assets, tmp_path, scene)
 
     mine_cam = np.array(list(cam.forward) + list(cam.right) + list(cam.up) + list(cam.aperture_position)
                         + [cam.aperture_radius, cam.focal_depth, cam.focal_length] + list(cam.film_bottom_left)
@@ -67,9 +78,10 @@ def test_scene_and_camera_bit_exact(host, assets, tmp_path, scene):
         assert np.array_equal(mine, r["spds"]), (scene, r["name"])
 
 
+@needs_ref
 def test_spectral_helpers_bit_exact(host, assets, tmp_path):
     import ctypes as C
-    ref, tables, _, _ = _load_both(host, assets, tmp_path, "cornell_plane_light")
+    ref, tables, _ = _load_both(host, assets, tmp_path, "cornell_plane_light")
     L = host.lib()
     n = ref.n
     rng = np.random.default_rng(7)

@@ -1,6 +1,8 @@
 """oracle/drt_oracle.c (the CPU restatement the CUDA path is checked against) pinned BIT-FOR-BIT against the
 unmodified reference's sample_scene (oracle/_ref, per-path RNG streams) -- every shipped scene plus a stress
-scene that exercises all 7 lobes, all 6 samplers, plane/sphere/point lights, multi-light NEE and the thin lens."""
+scene that exercises all 7 lobes, all 6 samplers, plane/sphere/point lights, multi-light NEE and the thin lens.
+Where oracle/_ref is absent, test_golden.py makes the same bit-exact comparison (per path and film) for every scene here against
+stored reference tiles; those are rendered at other sizes, sample counts and seeds, and cover tiles rather than whole frames."""
 import os
 
 import numpy as np
