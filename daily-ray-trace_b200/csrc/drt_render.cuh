@@ -13,8 +13,8 @@
  *   phase 2 "shade"   one HALF WARP per path, wavelengths across its 16 lanes (5 slots per lane for N = 69), two paths per
  *                     warp at a time.  The record is a broadcast read, spectra are conflict-free shared-memory rows,
  *                     throughput / radiance live in registers,
- *                     and the pixel's film (sum, Welford mean and M2, daily_ray_trace.c:732-743) stays in registers
- *                     for ALL samples of the pixel: each film plane is written to HBM exactly once, coalesced (K6).
+ *                     and the pixel's film (sum, Welford mean and M2, daily_ray_trace.c:732-743) stays on chip for ALL
+ *                     samples of the pixel: each film plane is written to HBM exactly once, coalesced (K6).
  *
  * No path state goes to global memory (deep renders excepted, see DEEP); HBM traffic is the film write, so the kernel is bound by
  * FP32 issue, not by the 1.2 KB-per-bounce queue traffic of a global-memory wavefront (SURVEY.md 8d).
@@ -22,7 +22,8 @@
  * Template parameters: R = float (default) or double (branch-flip diagnostic) arithmetic of phase 1; NS = wavelength slots per
  * half-warp lane (2, 3, 5, 8); PAIRED = one pixel per task (spp >= 32) or 32/spp pixels; MODE, chosen at scene upload:
  *   1 plastic-only  every surface material is a bp_diffuse / bp_glossy plastic under ONE light that is the scene's only emitter:
- *                   compact 4-word bounce records, the replay carries u = throughput * E; 72 registers, 2 CTAs x 14 warps per SM
+ *                   compact 4-word bounce records replayed backwards in units of the light's emission E (replay_compact),
+ *                   the film updated once per batch (BatchStats); 72 registers, 2 CTAs x 14 warps per SM
  *   2 classed       the same records for plastics, single-basis specular materials (mirror, fs_conductor, glass R / T) and
  *                   ct_conductor (GeomT::mclass); its hot code exceeds the 32 KB instruction cache, so the warps of a CTA run their
  *                   phases in lockstep behind mbarrier gates (LOCKSTEP); 64 registers, 2 CTAs x 16 warps
@@ -1086,18 +1087,19 @@ static __device__ __noinline__ ShadeState<NS> shade_bounce_general(const float *
 }
 
 /* ------------------------------------------------------------------ classed kernel: specular and rough-conductor bounces */
-/* One bounce of class SPECULAR or ROUGH (record layout: RenderLaunch in drt_device.cuh) on the replay loop's packed state: u2 / u1 =
- * throughput * E and d2 / d1 = radiance over the slot pairs and the odd last slot.  Inline (the struct-passing call cost 4 %), the
- * Fresnel formulas themselves out of line. */
+/* One bounce of class SPECULAR or ROUGH (record layout: RenderLaunch in drt_device.cuh) on the backward replay's packed state r2 / r1
+ * (the slot pairs and the odd last slot; see replay_compact).  Inline (the struct-passing call cost 4 %), the Fresnel formulas
+ * themselves out of line. */
 template <int NS>
 __device__ __forceinline__ void shade_special(uint32_t hdr, float4 w, const float *pool_lane, const SpdIndex &ix,
-                                              unsigned long long (&u2)[NS / 2 > 0 ? NS / 2 : 1], unsigned long long (&d2)[NS / 2 > 0 ? NS / 2 : 1], float &u1, float &d1)
+                                              unsigned long long (&r2)[NS / 2 > 0 ? NS / 2 : 1], float &r1)
 {
     constexpr int NP = NS / 2;
     const int cls = (int)(hdr & 3u), inside = (int)((hdr >> 4) & 1u), mat = (int)((hdr >> 5) & 31u);
     if(cls == DRT_CLASS_SPECULAR)
     {
-        /* throughput *= (c0 + c1 X) / pdf, cast_ray :467-469; X = mirror spectrum, dielectric R(on_dot) or conductor F(on_dot) */
+        /* r = (c0 + c1 X) / pdf * r: the bounce emits nothing (cast_ray :467-469); X = mirror spectrum, dielectric R(on_dot) or
+         * conductor F(on_dot) */
         const uint32_t basis = (hdr >> 2) & 3u;
         const float *x0 = pool_lane + (basis == 0u ? ix.row[mat][DRT_SPD_MIRROR] : basis == 1u ? ix.fres[mat][inside][0] : ix.fres[mat][inside][1]);
         const float *x1 = pool_lane + ix.fres[mat][inside][2];
@@ -1108,14 +1110,14 @@ __device__ __forceinline__ void shade_special(uint32_t hdr, float4 w, const floa
             unsigned long long x = pk2(x0[(2 * k) * DRT_HALF], x0[(2 * k + 1) * DRT_HALF]);
             if(basis == 1u) x = fresnel_dielectric_rel2(x, w.z);
             else if(basis == 2u) x = fresnel_conductor_ab2(x, pk2(x1[(2 * k) * DRT_HALF], x1[(2 * k + 1) * DRT_HALF]), w.z);
-            mul2_by(u2[k], fma2(c1, x, c0));
+            mul2_by(r2[k], fma2(c1, x, c0));
         }
         if(NS & 1)
         {
             float x = x0[(NS - 1) * DRT_HALF];
             if(basis == 1u) x = fresnel_dielectric_rel(x, w.z);
             else if(basis == 2u) x = fresnel_conductor_ab(x, x1[(NS - 1) * DRT_HALF], w.z);
-            u1 *= fmaf(w.y, x, w.x);
+            r1 *= fmaf(w.y, x, w.x);
         }
     }
     else
@@ -1127,115 +1129,165 @@ __device__ __forceinline__ void shade_special(uint32_t hdr, float4 w, const floa
             a2 = pk2(ra[(2 * k) * DRT_HALF], ra[(2 * k + 1) * DRT_HALF]); b2 = pk2(rb[(2 * k) * DRT_HALF], rb[(2 * k + 1) * DRT_HALF]);
         };
         const float a1 = (NS & 1) ? ra[(NS - 1) * DRT_HALF] : 0.f, b1 = (NS & 1) ? rb[(NS - 1) * DRT_HALF] : 0.f;
-        if(w.x != 0.f)   /* the light is visible: radiance += u * (w k F(cos_n)), :458-462 */
+        /* r = w / pdf F(cos_s) r + w k F(cos_n), cast_ray :458-469; the second term only when the light is visible */
+        const unsigned long long ws = pk2(w.z, w.z);
+#pragma unroll
+        for(int k = 0; k < NP; k += 1) { unsigned long long a2, b2; rows2(k, a2, b2); mul2_by(r2[k], mul2(ws, fresnel_conductor_ab2(a2, b2, w.w))); }
+        if(NS & 1) r1 *= w.z * fresnel_conductor_ab(a1, b1, w.w);
+        if(w.x != 0.f)
         {
             const unsigned long long wn = pk2(w.x, w.x);
 #pragma unroll
-            for(int k = 0; k < NP; k += 1) { unsigned long long a2, b2; rows2(k, a2, b2); fma2_acc(d2[k], u2[k], mul2(wn, fresnel_conductor_ab2(a2, b2, w.y))); }
-            if(NS & 1) d1 = fmaf(u1, w.x * fresnel_conductor_ab(a1, b1, w.y), d1);
+            for(int k = 0; k < NP; k += 1) { unsigned long long a2, b2; rows2(k, a2, b2); fma2_acc(r2[k], wn, fresnel_conductor_ab2(a2, b2, w.y)); }
+            if(NS & 1) r1 = fmaf(w.x, fresnel_conductor_ab(a1, b1, w.y), r1);
         }
-        const unsigned long long ws = pk2(w.z, w.z);
-#pragma unroll
-        for(int k = 0; k < NP; k += 1) { unsigned long long a2, b2; rows2(k, a2, b2); mul2_by(u2[k], mul2(ws, fresnel_conductor_ab2(a2, b2, w.w))); }
-        if(NS & 1) u1 *= w.z * fresnel_conductor_ab(a1, b1, w.w);
     }
 }
 
-/* cast_ray's spectral arithmetic (daily_ray_trace.c:446-473) replayed from the record `col` (nb >= 1 bounces);
+/* One 16-bit bounce header of a compact record, zero-extended into a 32-bit register.  A plain 16-bit load keeps the loop-carried
+ * header as a 16-bit value, which costs two more instructions per bounce to merge and widen.  Deep renders keep the generic load:
+ * their headers may lie in the global overflow row. */
+template <bool DEEP> __device__ __forceinline__ uint32_t load_hdr16(const uint16_t *p)
+{
+    if constexpr(DEEP) return *p;
+    uint32_t v;
+    asm volatile("ld.shared.u16 %0, [%1];" : "=r"(v) : "r"((uint32_t)__cvta_generic_to_shared(p)));
+    return v;
+}
+
+/* Compact records (modes 1 and 2; RenderLaunch in drt_device.cuh: header halves from word 2, four weights per bounce).  The light is
+ * the scene's only emitter, so every term of cast_ray's radiance (daily_ray_trace.c:446-473) is E times the light-free factors, and
+ * the path's contribution is E * r with, for a plastic bounce b (NEE weights n_b, sampled-direction weights s_b),
+ *     n_b = wd_n k D + wg_n k G    (NEE: bdsf * k, :322-327; the weights are 0 when the light is hidden)
+ *     s_b = wd_s/pdf D + wg_s/pdf G (:467-469)
+ *     r   = n_0 + s_0 (n_1 + s_1 (... (n_last + s_last e)))       e = 1 if the path ends on the light (:453-457), else 0.
+ * This evaluates r from the last bounce back to the first (Horner form), four f32x2 operations per slot pair and bounce:
+ *     r = D (wd_n + wd_s r) + G (wg_n + wg_s r)
+ * and two for the last bounce, whose r = e is a constant.  The vignette factor (:612-615) rides in bounce 0's weights (trace_path);
+ * a path that meets the light without a shaded bounce has r = vignette.  r is returned as f32x2 register pairs for wavelength slots
+ * (0,1), (2,3), ... (r2) plus one scalar for an odd last slot (r1); E is applied once per batch (PixelFilm::add_batch). */
+template <int NS, int MODE, bool DEEP>
+__device__ __forceinline__ void replay_compact(const float *col, const float *deep, uint32_t nb, const SpdIndex &ix, const float *pool, const float *pool_lane,
+                                               uint32_t lane16, const RenderLaunch &L, unsigned long long (&r2)[NS / 2 > 0 ? NS / 2 : 1], float &r1)
+{
+    constexpr bool CLASSED = MODE == 2;
+    constexpr int NP = NS / 2;
+    const uint32_t nshade = nb & 0xffffu;
+    if(nshade == 0u)   /* the camera ray met the light */
+    {
+        const float v = col[REC_VIG];
+#pragma unroll
+        for(int k = 0; k < NP; k += 1) r2[k] = pk2(v, v);
+        r1 = v;
+        return;
+    }
+    /* The bounces come in at most two spans: the first L.smem_depth in the slot's shared-memory record, the rest (deep renders only)
+     * in the slot's global overflow row, which is walked first.  b counts down through the current span; `rest` bounces of the
+     * shared-memory span are left when the overflow row is done. */
+    int b = (int)nshade - 1;
+    int rest = 0;
+    const uint16_t *hp = reinterpret_cast<const uint16_t *>(col + REC_HDR16) + b;   /* this bounce's header and weights */
+    const float4 *wp = reinterpret_cast<const float4 *>(col + L.head_words) + b;
+    if(DEEP && nshade > L.smem_depth)
+    {
+        rest = (int)L.smem_depth;
+        b = (int)(nshade - L.smem_depth) - 1;
+        hp = reinterpret_cast<const uint16_t *>(deep + L.deep_hdr_off) + b;
+        wp = reinterpret_cast<const float4 *>(deep) + b;
+    }
+    /* The previous bounce's header is in flight while this one is shaded (the D, G block address depends on it; the weights are
+     * loaded together with the block and need no head start).  Before the first bounce of the shared-memory span this reads (and
+     * never uses) the record's head words; in deep renders the step back stops at the span's first bounce, since the word before an
+     * overflow row may lie outside the allocation. */
+    auto step_back = [&]() { const int s = (!DEEP || b > 0) ? 1 : 0; hp -= s; wp -= s; };
+    uint32_t hdr = load_hdr16<DEEP>(hp);
+    const float e = (nb >> 16) ? 1.f : 0.f;
+    if(!CLASSED || (hdr & 3u) == 0u)
+    {
+        /* the last bounce, a plastic: r = (wd_n + wd_s e) D + (wg_n + wg_s e) G */
+        const float4 w = *wp;   /* wd_n k, wg_n k, wd_s / pdf, wg_s / pdf */
+        const float4 *blk = reinterpret_cast<const float4 *>(pool + hdr) + lane16;
+        const float wd = fmaf(w.z, e, w.x), wg = fmaf(w.w, e, w.y);
+        const unsigned long long wd2 = pk2(wd, wd), wg2 = pk2(wg, wg);
+        step_back();
+        hdr = load_hdr16<DEEP>(hp);
+        b -= 1;
+#pragma unroll
+        for(int k = 0; k < NP; k += 1)
+        {
+            const float4 dg = blk[k * DRT_HALF];
+            r2[k] = fma2(wg2, pk2(dg.z, dg.w), mul2(wd2, pk2(dg.x, dg.y)));
+        }
+        if(NS & 1)
+        {
+            const float2 q = *reinterpret_cast<const float2 *>(blk + NP * DRT_HALF);   /* D, G of the last slot */
+            r1 = fmaf(wg, q.y, wd * q.x);
+        }
+    }
+    else
+    {
+#pragma unroll
+        for(int k = 0; k < NP; k += 1) r2[k] = pk2(e, e);
+        r1 = e;
+    }
+#pragma unroll 1
+    for(;;)
+    {
+#pragma unroll 1
+        for(; b >= 0; b -= 1)
+        {
+            const float4 w = *wp;
+            if constexpr(CLASSED)
+            {
+                if(hdr & 3u)   /* a specular or rough-conductor bounce */
+                {
+                    shade_special<NS>(hdr, w, pool_lane, ix, r2, r1);
+                    step_back();
+                    hdr = load_hdr16<DEEP>(hp);
+                    continue;
+                }
+            }
+            const float4 *blk = reinterpret_cast<const float4 *>(pool + hdr) + lane16;
+            const unsigned long long wdn = pk2(w.x, w.x), wgn = pk2(w.y, w.y), wds = pk2(w.z, w.z), wgs = pk2(w.w, w.w);
+            step_back();
+            hdr = load_hdr16<DEEP>(hp);
+#pragma unroll
+            for(int k = 0; k < NP; k += 1)
+            {
+                const float4 dg = blk[k * DRT_HALF];
+                r2[k] = fma2(pk2(dg.z, dg.w), fma2(wgs, r2[k], wgn), mul2(pk2(dg.x, dg.y), fma2(wds, r2[k], wdn)));
+            }
+            if(NS & 1)
+            {
+                const float2 q = *reinterpret_cast<const float2 *>(blk + NP * DRT_HALF);
+                r1 = fmaf(q.y, fmaf(w.w, r1, w.y), q.x * fmaf(w.z, r1, w.x));
+            }
+        }
+        if(!DEEP || rest == 0) break;
+        b = rest - 1;
+        rest = 0;
+        hp = reinterpret_cast<const uint16_t *>(col + REC_HDR16) + b;
+        wp = reinterpret_cast<const float4 *>(col + L.head_words) + b;
+        hdr = load_hdr16<DEEP>(hp);
+    }
+}
+
+/* cast_ray's spectral arithmetic (daily_ray_trace.c:446-473) replayed forward from a general record `col` (nb >= 1 bounces);
  * returns the path contribution already multiplied by the vignette factor (:612-615).
  * Throughput and radiance are held as f32x2 register pairs for wavelength slots (0,1), (2,3), ... plus one scalar for an
  * odd last slot.  The hot bounce (two-lobe plastic under the scene's only light) is
  *     radiance   += throughput * (wd_n k * DE + wg_n k * GE)        (NEE: bdsf * emission * k, :322-327; weights are 0 when shadowed)
  *     throughput *= wd_s/pdf * D + wg_s/pdf * G                      (:467-469)
  * with D, G, DE = D*E, GE = G*E fetched from the material's interleaved plastic block by 16-byte loads. */
-template <int NS, int MODE, bool DEEP, typename G>
+template <int NS, bool DEEP, typename G>
 __device__ __forceinline__ void replay_path(const float *col, const float *deep, uint32_t nb, const G &g, const SpdIndex &ix, const float *pool, const float *pool_lane,
                                             uint32_t lane16, const RenderLaunch &L, float (&c)[NS])
 {
-    constexpr bool ALLFAST = MODE != 0, CLASSED = MODE == 2;
     constexpr int NP = NS / 2;
     unsigned long long thr2[NP > 0 ? NP : 1], dst2[NP > 0 ? NP : 1];
     float thr1 = 1.f, dst1 = 0.f;
 #pragma unroll
     for(int k = 0; k < NP; k += 1) { thr2[k] = pk2(1.f, 1.f); dst2[k] = pk2(0.f, 0.f); }
-    if constexpr(ALLFAST)
-    {
-        /* compact records (RenderLaunch in drt_device.cuh): header halves from word 2, four weights per bounce.
-         * Every term of the path is throughput * E * (...): the light is the scene's only emitter, so the replay carries
-         * u = throughput * E (thr2 / thr1 below) and needs only the D and G rows:
-         *     radiance += u * (wd_n k * D + wg_n k * G)      u *= wd_s/pdf * D + wg_s/pdf * G      closing emitter: radiance += u */
-        const uint16_t *hp = reinterpret_cast<const uint16_t *>(col + REC_HDR16);
-        const float4 *wp = reinterpret_cast<const float4 *>(col + L.head_words);
-        const uint32_t nshade = nb & 0xffffu;
-        {
-            /* every path starts with u = throughput * E = E (SpdIndex::light_pairs).  Loading E once per batch instead of once per
-             * path was measured: 5 more live registers spill in the 72-register kernel, -1.4 % */
-            const unsigned long long *ep = reinterpret_cast<const unsigned long long *>(pool + ix.light_pairs) + lane16;
-#pragma unroll
-            for(int k = 0; k < NP; k += 1) thr2[k] = ep[k * DRT_HALF];
-            if(NS & 1) thr1 = reinterpret_cast<const float *>(ep + NP * DRT_HALF)[0];
-        }
-        /* The bounces come in at most two spans: the first L.smem_depth in the slot's shared-memory record, the rest (deep renders
-         * only) in the slot's global overflow row. */
-        uint32_t left = nshade, span = DEEP ? min(nshade, L.smem_depth) : nshade;
-#pragma unroll 1
-        for(;;)
-        {
-        uint32_t hdr = hp[0];
-        float4 w = wp[0];   /* wd_n k, wg_n k, wd_s / pdf, wg_s / pdf */
-#pragma unroll 1
-        for(uint32_t b = 0; b < span; b += 1)
-        {
-            if constexpr(CLASSED)
-            {
-                if(hdr & 3u)   /* a specular or rough-conductor bounce */
-                {
-                    shade_special<NS>(hdr, w, pool_lane, ix, thr2, dst2, thr1, dst1);
-                    hdr = hp[b + 1];
-                    w = wp[b + 1];
-                    continue;
-                }
-            }
-            const float4 *blk = reinterpret_cast<const float4 *>(pool + hdr) + lane16;
-            const unsigned long long wdn = pk2(w.x, w.x), wgn = pk2(w.y, w.y), wds = pk2(w.z, w.z), wgs = pk2(w.w, w.w);
-            const float w1x = w.x, w1y = w.y, w1z = w.z, w1w = w.w;
-            /* the next bounce's header and weights are in flight while this one is shaded; after the last bounce this reads (and
-             * never uses) up to 16 bytes past the record, which is the next slot or the film parking area, both inside the CTA's
-             * shared memory */
-            hdr = hp[b + 1];
-            w = wp[b + 1];
-#pragma unroll
-            for(int k = 0; k < NP; k += 1)
-            {
-                const float4 dg = blk[k * DRT_HALF];
-                const unsigned long long d2 = pk2(dg.x, dg.y), g2 = pk2(dg.z, dg.w);
-                unsigned long long f = fma2(wgn, g2, mul2(wdn, d2));
-                fma2_acc(dst2[k], thr2[k], f);
-                unsigned long long t = fma2(wgs, g2, mul2(wds, d2));
-                mul2_by(thr2[k], t);
-            }
-            if(NS & 1)
-            {
-                const float2 q = *reinterpret_cast<const float2 *>(blk + NP * DRT_HALF);   /* D, G of the last slot */
-                dst1 = fmaf(thr1, fmaf(w1y, q.y, w1x * q.x), dst1);
-                thr1 *= fmaf(w1w, q.y, w1z * q.x);
-            }
-        }
-        left -= span;
-        if(!DEEP || left == 0u) break;
-        hp = reinterpret_cast<const uint16_t *>(deep + L.deep_hdr_off);
-        wp = reinterpret_cast<const float4 *>(deep);
-        span = left;
-        }
-        if(nb >> 16)   /* the path ran into the light, cast_ray :453-457: radiance += throughput * E = u */
-        {
-#pragma unroll
-            for(int k = 0; k < NP; k += 1) add2_acc(dst2[k], thr2[k]);
-            if(NS & 1) dst1 += thr1;
-        }
-    }
-    else
-    {
     const uint32_t bw = L.bounce_words, ew = L.eval_words;
     const float *p = (!DEEP || L.smem_depth) ? col + REC_HEAD : deep;
     float4 a_next = *reinterpret_cast<const float4 *>(p);
@@ -1276,33 +1328,64 @@ __device__ __forceinline__ void replay_path(const float *col, const float *deep,
             if(NS & 1) dst1 = fmaf(thr1, row[(NS - 1) * DRT_HALF], dst1);
             break;
         }
-        if constexpr(!ALLFAST)
-        {
-            ShadeState<NS> st;
+        ShadeState<NS> st;
 #pragma unroll
-            for(int k = 0; k < NP; k += 1) { upk2(thr2[k], st.thr.v[2 * k], st.thr.v[2 * k + 1]); upk2(dst2[k], st.dst.v[2 * k], st.dst.v[2 * k + 1]); }
-            if(NS & 1) { st.thr.v[NS - 1] = thr1; st.dst.v[NS - 1] = dst1; }
-            st = shade_bounce_general<NS, G>(pc, 0u, hdr, g, ix, pool_lane, ew, L.nlights, st);
+        for(int k = 0; k < NP; k += 1) { upk2(thr2[k], st.thr.v[2 * k], st.thr.v[2 * k + 1]); upk2(dst2[k], st.dst.v[2 * k], st.dst.v[2 * k + 1]); }
+        if(NS & 1) { st.thr.v[NS - 1] = thr1; st.dst.v[NS - 1] = dst1; }
+        st = shade_bounce_general<NS, G>(pc, 0u, hdr, g, ix, pool_lane, ew, L.nlights, st);
 #pragma unroll
-            for(int k = 0; k < NP; k += 1) { thr2[k] = pk2(st.thr.v[2 * k], st.thr.v[2 * k + 1]); dst2[k] = pk2(st.dst.v[2 * k], st.dst.v[2 * k + 1]); }
-            if(NS & 1) { thr1 = st.thr.v[NS - 1]; dst1 = st.dst.v[NS - 1]; }
-        }
+        for(int k = 0; k < NP; k += 1) { thr2[k] = pk2(st.thr.v[2 * k], st.thr.v[2 * k + 1]); dst2[k] = pk2(st.dst.v[2 * k], st.dst.v[2 * k + 1]); }
+        if(NS & 1) { thr1 = st.thr.v[NS - 1]; dst1 = st.dst.v[NS - 1]; }
     }
-    }
-    /* the vignette factor: compact records carry it in the first bounce's weights (trace_path) */
-    const float vig = (ALLFAST && (nb & 0xffffu) != 0u) ? 1.f : col[REC_VIG];
-    if(ALLFAST && (nb & 0xffffu) != 0u)
-    {
-#pragma unroll
-        for(int k = 0; k < NP; k += 1) upk2(dst2[k], c[2 * k], c[2 * k + 1]);
-        if(NS & 1) c[NS - 1] = dst1;
-        return;
-    }
+    const float vig = col[REC_VIG];
     const unsigned long long vig2 = pk2(vig, vig);
 #pragma unroll
     for(int k = 0; k < NP; k += 1) upk2(mul2(dst2[k], vig2), c[2 * k], c[2 * k + 1]);
     if(NS & 1) c[NS - 1] = dst1 * vig;
 }
+
+/* The replayed samples of one pixel in one batch that a half warp shaded, in units of the light's emission (replay_compact: sample
+ * = E * r): count, S = sum of r and the shifted sum of squares Q = sum of (r - K)^2 about the half's first sample K, which keeps the
+ * M2 of a pixel whose samples barely differ from cancelling (PixelFilm::add_batch).  Three f32x2 operations per slot pair and
+ * sample, against the five of a per-sample Welford update and the E multiply. */
+template <int NS> struct BatchStats
+{
+    static constexpr int NP = NS / 2, NP1 = NP > 0 ? NP : 1;
+    unsigned long long s2[NP1], q2[NP1], k2[NP1];
+    float s1, q1, k1;
+    uint32_t cnt;
+    __device__ __forceinline__ void clear()
+    {
+        cnt = 0u; s1 = 0.f; q1 = 0.f; k1 = 0.f;
+#pragma unroll
+        for(int k = 0; k < NP; k += 1) { s2[k] = pk2(0.f, 0.f); q2[k] = pk2(0.f, 0.f); k2[k] = pk2(0.f, 0.f); }
+    }
+    /* `first`: this is the half's first sample of the batch, which becomes the shift K */
+    __device__ __forceinline__ void add(const unsigned long long (&r2)[NP1], float r1, bool first)
+    {
+        const unsigned long long m1 = pk2(-1.f, -1.f);
+        if(first)
+        {
+#pragma unroll
+            for(int k = 0; k < NP; k += 1) k2[k] = r2[k];
+            k1 = r1;
+        }
+        cnt += 1u;
+#pragma unroll
+        for(int k = 0; k < NP; k += 1)
+        {
+            add2_acc(s2[k], r2[k]);
+            const unsigned long long d = fma2(k2[k], m1, r2[k]);
+            q2[k] = fma2(d, d, q2[k]);
+        }
+        if(NS & 1)
+        {
+            s1 += r1;
+            const float d = r1 - k1;
+            q1 = fmaf(d, d, q1);
+        }
+    }
+};
 
 /* film of one pixel held by a half warp: lane l16 owns wavelengths l16, l16+16, ...; when both halves work on the same
  * pixel each holds the partial film of its samples and merge_halves() combines them (Chan et al.) before the store */
@@ -1357,6 +1440,36 @@ template <int NS> struct PixelFilm
         {
             m2[j] = fmaf(mean[j] * mean[j], s, m2[j]);
             mean[j] = fmaf(-mean[j], w, mean[j]);
+        }
+    }
+    /* nz paths that contributed nothing and the samples E * r of `bs`, in one pairwise update (Chan et al.): the batch has count
+     * n = nz + bs.cnt, sum E S, mean E S / n and M2 = E^2 (Q + nz K^2 - n (S / n - K)^2) (the zeros are samples r = 0).  `e` = this
+     * lane's E in the SpdIndex::light_pairs layout.  Without replayed samples this is add_zeros(nz). */
+    __device__ __forceinline__ void add_batch(uint32_t nz, const BatchStats<NS> &bs, const float *e, uint32_t lane16)
+    {
+        if(bs.cnt == 0u) { add_zeros(nz); return; }
+        const float nb = (float)(bs.cnt + nz), n0 = cnt, zf = (float)nz;
+        cnt += nb; lit = true;
+        const float inv_nb = r_rcp_fast(nb);
+        const float w = nb * r_rcp_fast(cnt);   /* n / (n0 + n) */
+        const float s = n0 * w;
+#pragma unroll
+        for(int j = 0; j < NS; j += 1)
+        {
+            float S, Q, K, t;
+            if(j + 1 < NS || !(NS & 1))
+            {
+                if(j & 1) { upk2(bs.s2[j >> 1], t, S); upk2(bs.q2[j >> 1], t, Q); upk2(bs.k2[j >> 1], t, K); }
+                else      { upk2(bs.s2[j >> 1], S, t); upk2(bs.q2[j >> 1], Q, t); upk2(bs.k2[j >> 1], K, t); }
+            }
+            else { S = bs.s1; Q = bs.q1; K = bs.k1; }
+            const float E = e[2 * ((j >> 1) * DRT_HALF + lane16) + (j & 1)];
+            const float m = S * inv_nb, dk = m - K;
+            const float m2b = fmaxf(fmaf(-nb * dk, dk, fmaf(zf * K, K, Q)), 0.f);   /* the batch's M2 over r */
+            const float delta = fmaf(E, m, -mean[j]);
+            sum[j] = fmaf(E, S, sum[j]);
+            m2[j] = fmaf(delta * delta, s, fmaf(E * E, m2b, m2[j]));
+            mean[j] = fmaf(delta, w, mean[j]);
         }
     }
     /* this half <- this half (+) the other half: count, mean, M2 by the pairwise update, sums added */
@@ -1420,10 +1533,11 @@ static __device__ __noinline__ void film_store(FilmPtrs film, uint32_t gpix, uin
 /* ------------------------------------------------------------------ the kernel */
 
 /* Diagnostics (drt_cuda_sample_paths / drt_cuda_debug_records): per-path spectrum and raw record to global memory, by the 16
- * lanes of a half warp.  Out of line: never on the path of a film render. */
+ * lanes of a half warp.  Out of line: never on the path of a film render.  `e` (compact records, whose replay leaves out the light's
+ * emission): the SpdIndex::light_pairs row the spectrum c is multiplied by, else null. */
 template <int NS>
 static __device__ __noinline__ void dump_path(float *record_dump, float *path_dump, uint32_t path_words, const float *rec_slot, const float *c,
-                                       size_t path_index, uint32_t n, uint32_t lane16)
+                                       const float *e, size_t path_index, uint32_t n, uint32_t lane16)
 {
     if(record_dump)
         for(uint32_t wd = lane16; wd < path_words; wd += DRT_HALF) record_dump[path_index * path_words + wd] = rec_slot[wd];
@@ -1432,7 +1546,8 @@ static __device__ __noinline__ void dump_path(float *record_dump, float *path_du
         for(int k = 0; k < NS; k += 1)
         {
             uint32_t wl = lane16 + k * DRT_HALF;
-            if(wl < n) path_dump[path_index * n + wl] = c ? c[k] : 0.f;
+            const float ek = e ? e[2 * ((k >> 1) * DRT_HALF + lane16) + (k & 1)] : 1.f;
+            if(wl < n) path_dump[path_index * n + wl] = c ? ek * c[k] : 0.f;
         }
 }
 
@@ -1624,7 +1739,8 @@ __global__ void __launch_bounds__((MODE == 1 ? DRT_FAST_WARPS : MODE == 2 ? DRT_
             }
             __syncwarp();
             gate();
-            if((ALLFAST || DRT_PARK_GENERAL) && paired) film.unpark(park);
+            /* compact records: the film stays parked through the replay, which accumulates BatchStats instead */
+            if(!ALLFAST && DRT_PARK_GENERAL && paired) film.unpark(park);
             {
                 /* termination histogram: one shared-memory atomic per distinct bin of the batch (bin 9 = idle lane) */
                 const uint32_t peers = __match_any_sync(0xffffffffu, bin);
@@ -1636,6 +1752,7 @@ __global__ void __launch_bounds__((MODE == 1 ? DRT_FAST_WARPS : MODE == 2 ? DRT_
             if(paired && !dumping && !__any_sync(0xffffffffu, lane < count && my_nb != 0u))
             {
                 /* no path of the batch has a bounce record (every sample left the scene): nothing to replay */
+                if(ALLFAST) film.unpark(park);
                 if(half == 0) film.add_zeros(count);
                 __syncwarp();
                 continue;
@@ -1662,22 +1779,29 @@ __global__ void __launch_bounds__((MODE == 1 ? DRT_FAST_WARPS : MODE == 2 ? DRT_
             {
                 const uint32_t lp = p_begin + px;
                 uint32_t gpix = 0;
-                if(!paired)
+                /* compact records: the film of a pixel is loaded (or cleared) after the replay, so it takes no registers during it */
+                auto start_film = [&]()
                 {
-                    gpix = (L.y0 + lp / rw) * L.width + L.x0 + lp % rw;
-                    film.clear();
-                    if(L.accumulate && have_film) film = film_load<NS>(L.film, gpix, n, lane);
-                }
+                    if(!paired)
+                    {
+                        gpix = (L.y0 + lp / rw) * L.width + L.x0 + lp % rw;
+                        film.clear();
+                        if(L.accumulate && have_film) film = film_load<NS>(L.film, gpix, n, lane);
+                    }
+                };
+                if(!ALLFAST) start_film();
                 const uint32_t lo = px * per_px;
                 const uint32_t nzero = __popc(__ballot_sync(0xffffffffu, lane < count && my_px == px && my_nb == 0u));
-                if(half == 0) film.add_zeros(nzero);   /* paths that contributed nothing */
+                if(!ALLFAST && half == 0) film.add_zeros(nzero);   /* paths that contributed nothing */
                 if(dumping)
                     for(uint32_t i = lo; i < lo + nzero; i += 1)
                     {
                         const uint32_t slot = __shfl_sync(0xffffffffu, v, i) & 31u;
                         const uint32_t s_in = paired ? q0 + slot : slot - px * spp;
-                        if(half == 0) dump_path<NS>(L.record_dump, L.path_dump, L.path_words, rec + slot * stride, nullptr, (size_t)lp * spp + s_in, n, lane16);
+                        if(half == 0) dump_path<NS>(L.record_dump, L.path_dump, L.path_words, rec + slot * stride, nullptr, nullptr, (size_t)lp * spp + s_in, n, lane16);
                     }
+                BatchStats<NS> bs;
+                if(ALLFAST) bs.clear();
                 for(uint32_t i = lo + nzero; i < lo + per_px; i += 2)
                 {
                     const uint32_t pos = i + half;
@@ -1686,16 +1810,39 @@ __global__ void __launch_bounds__((MODE == 1 ? DRT_FAST_WARPS : MODE == 2 ? DRT_
                     if(pos < lo + per_px)
                     {
                         float c[NS];
-                        replay_path<NS, MODE, DEEP>(rec + slot * stride, deep_w + (size_t)slot * L.deep_stride, nb, g, ix, spool, pool_lane, lane16, L, c);
-                        film.add(c);
+                        if constexpr(ALLFAST)
+                        {
+                            unsigned long long r2[BatchStats<NS>::NP1];
+                            float r1;
+                            replay_compact<NS, MODE, DEEP>(rec + slot * stride, deep_w + (size_t)slot * L.deep_stride, nb, ix, spool, pool_lane, lane16, L, r2, r1);
+                            bs.add(r2, r1, i == lo + nzero);
+                            if(dumping)
+                            {
+#pragma unroll
+                                for(int k = 0; k < NS / 2; k += 1) upk2(r2[k], c[2 * k], c[2 * k + 1]);
+                                if(NS & 1) c[NS - 1] = r1;
+                            }
+                        }
+                        else
+                        {
+                            replay_path<NS, DEEP>(rec + slot * stride, deep_w + (size_t)slot * L.deep_stride, nb, g, ix, spool, pool_lane, lane16, L, c);
+                            film.add(c);
+                        }
                         if(dumping)
                         {
                             float cc[NS];   /* a copy whose address is taken only here: c itself stays in registers */
 #pragma unroll
                             for(int k = 0; k < NS; k += 1) cc[k] = c[k];
-                            dump_path<NS>(L.record_dump, L.path_dump, L.path_words, rec + slot * stride, cc, (size_t)lp * spp + (paired ? q0 + slot : slot - px * spp), n, lane16);
+                            dump_path<NS>(L.record_dump, L.path_dump, L.path_words, rec + slot * stride, cc, ALLFAST ? spool + ix.light_pairs : nullptr,
+                                          (size_t)lp * spp + (paired ? q0 + slot : slot - px * spp), n, lane16);
                         }
                     }
+                }
+                if constexpr(ALLFAST)
+                {
+                    if(paired) film.unpark(park);
+                    else start_film();
+                    film.add_batch(half == 0 ? nzero : 0u, bs, spool + ix.light_pairs, lane16);
                 }
                 if(!paired)
                 {
