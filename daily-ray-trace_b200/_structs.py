@@ -48,6 +48,10 @@ class RenderParams(C.Structure):
                 ("max_depth", C.c_uint32), ("pixel_scheme", C.c_int32), ("seed", C.c_uint64)]
 
 
+class Adaptive(C.Structure):
+    _fields_ = [("rel_error", C.c_float), ("min_samples", C.c_uint32)]
+
+
 class Config(C.Structure):
     _paths = ["input_scene", "output_spd", "average_spd", "variance_spd", "output_bmp", "average_bmp", "variance_bmp",
               "white_spd", "cmf_x", "cmf_y", "cmf_z", "red_spd", "green_spd", "blue_spd", "cyan_spd", "magenta_spd",

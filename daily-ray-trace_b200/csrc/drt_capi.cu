@@ -733,7 +733,7 @@ extern "C" int drt_cuda_render_kernel_info(drt_cuda_context *ctx, const drt_rend
 static int launch(drt_cuda_context *ctx, const drt_render_params *p, uint32_t x0, uint32_t y0, uint32_t x1, uint32_t y1,
                   FilmPtrs film, float *dump, int accumulate, cudaStream_t stream, float *record_dump = nullptr, uint32_t *path_words_out = nullptr,
                   const drt_film *scatter = nullptr, int scatter_count = 0, int scatter_rank = 0, uint64_t scatter_slice = 0, bool keep_stats = false,
-                  uint64_t band_begin = 0, uint64_t band_end = 0)
+                  uint64_t band_begin = 0, uint64_t band_end = 0, const drt_adaptive *adaptive = nullptr)
 {
     if(!ctx->have_scene) return fail(DRT_CUDA_E_STATE, "upload a scene first");
     if(p->width == 0 || p->height == 0 || x1 > p->width || y1 > p->height || x0 >= x1 || y0 >= y1) return fail(DRT_CUDA_E_ARG, "bad image rectangle");
@@ -775,6 +775,11 @@ static int launch(drt_cuda_context *ctx, const drt_render_params *p, uint32_t x0
     /* max_cast_depth 0 casts no ray at all (cast_ray's loop, daily_ray_trace.c:446): nothing to cull, and the culled pixels' "one closest-hit ray" must not be counted */
     hit_rect(ctx->hit_bound && p->max_depth > 0, ctx->hit_u0, ctx->hit_u1, ctx->hit_v0, ctx->hit_v1, p->width, p->height, rect);
     L.hit_x0 = rect[0]; L.hit_y0 = rect[1]; L.hit_x1 = rect[2]; L.hit_y1 = rect[3];
+    if(adaptive)   /* checked by adaptive_args: f32 geometry, >= 32 samples (one pixel per task), no scatter */
+    {
+        L.adaptive = 1; L.rel_error = adaptive->rel_error; L.min_samples = adaptive->min_samples;
+        L.luminance_w = reinterpret_cast<const float *>(static_cast<const unsigned char *>(ctx->d_rgb_tables) + drt_rgb_tables_yw_offset());
+    }
     /* record dumps (diagnostics) want the whole record in shared memory; renders keep full occupancy and let deep bounces overflow */
     const bool whole = record_dump != nullptr || (path_words_out != nullptr && !dump && !film.sum);
     int warps, ctas_per_sm;
@@ -864,7 +869,34 @@ int drt_ensure_buffer(float **buf, size_t *have, size_t need)
     return DRT_CUDA_OK;
 }
 
-extern "C" int drt_cuda_render_host(drt_cuda_context *ctx, const drt_render_params *params, const drt_film *out)
+/* argument checks of the adaptive entry points (drt_cuda.h) */
+static int adaptive_args(const drt_cuda_context *ctx, const drt_render_params *p, const drt_adaptive *a)
+{
+    if(!ctx->have_scene) return fail(DRT_CUDA_E_STATE, "upload a scene first");
+    if(p->sample_end < p->sample_begin) return fail(DRT_CUDA_E_ARG, "bad sample range [%u,%u)", p->sample_begin, p->sample_end);
+    const uint32_t range = p->sample_end - p->sample_begin;
+    if(!(a->rel_error > 0.f) || !isfinite(a->rel_error))
+        return fail(DRT_CUDA_E_ARG, "adaptive sampling: rel_error must be a finite number > 0 (got %g)", (double)a->rel_error);
+    if(a->min_samples < 32u || a->min_samples > range)
+        return fail(DRT_CUDA_E_ARG, "adaptive sampling: min_samples must lie in [32, %u], the call's sample range [%u,%u) (got %u); "
+                    "a pixel is checked after each batch of 32 samples, so the range needs at least 32", range, p->sample_begin, p->sample_end, a->min_samples);
+    if(ctx->f64_geometry)
+        return fail(DRT_CUDA_E_UNSUPPORTED, "adaptive sampling runs with f32 geometry only: f64 geometry is the branch-flip diagnostic and has no adaptive kernel");
+    return DRT_CUDA_OK;
+}
+
+extern "C" int drt_cuda_render_device_adaptive(drt_cuda_context *ctx, const drt_render_params *params, const drt_adaptive *adaptive,
+                                               const drt_film *film, int accumulate, void *stream)
+{
+    if(!ctx || !params || !adaptive || !film || !film->sum || !film->filter || !film->mean || !film->m2) return fail(DRT_CUDA_E_ARG, "NULL argument");
+    int rc = adaptive_args(ctx, params, adaptive);
+    if(rc != DRT_CUDA_OK) return rc;
+    FilmPtrs f = { film->sum, film->filter, film->mean, film->m2 };
+    return launch(ctx, params, 0, 0, params->width, params->height, f, nullptr, accumulate, (cudaStream_t)stream, nullptr, nullptr, nullptr, 0, 0, 0, false, 0, 0, adaptive);
+}
+
+/* render_host and render_host_adaptive (adaptive != NULL) */
+static int render_host(drt_cuda_context *ctx, const drt_render_params *params, const drt_adaptive *adaptive, const drt_film *out)
 {
     if(!ctx || !params || !out || !out->sum || !out->filter || !out->mean || !out->m2) return fail(DRT_CUDA_E_ARG, "NULL argument");
     if(!ctx->have_scene) return fail(DRT_CUDA_E_STATE, "upload a scene first");
@@ -894,7 +926,7 @@ extern "C" int drt_cuda_render_host(drt_cuda_context *ctx, const drt_render_para
     {
         const uint32_t y0 = bands > 1 ? (uint32_t)((uint64_t)params->height * cut[b] / 16) : 0u;
         const uint32_t y1 = bands > 1 ? (uint32_t)((uint64_t)params->height * cut[b + 1] / 16) : params->height;
-        rc = launch(ctx, params, 0, y0, params->width, y1, f, nullptr, 0, sr, nullptr, nullptr, nullptr, 0, 0, 0, b > 0);
+        rc = launch(ctx, params, 0, y0, params->width, y1, f, nullptr, 0, sr, nullptr, nullptr, nullptr, 0, 0, 0, b > 0, 0, 0, adaptive);
         if(rc != DRT_CUDA_OK) return rc;
         if(bands > 1) { CU(cudaEventRecord(ctx->band_done[b], sr)); CU(cudaStreamWaitEvent(sc, ctx->band_done[b], 0)); }
         const size_t at = (size_t)y0 * w * n, cnt = (size_t)(y1 - y0) * w * n * 4;
@@ -907,6 +939,19 @@ extern "C" int drt_cuda_render_host(drt_cuda_context *ctx, const drt_render_para
     if(bands > 1) { CU(cudaStreamSynchronize(sr)); CU(cudaStreamSynchronize(sc)); }
     CU(cudaStreamSynchronize(0));
     return DRT_CUDA_OK;
+}
+
+extern "C" int drt_cuda_render_host(drt_cuda_context *ctx, const drt_render_params *params, const drt_film *out)
+{
+    return render_host(ctx, params, nullptr, out);
+}
+
+extern "C" int drt_cuda_render_host_adaptive(drt_cuda_context *ctx, const drt_render_params *params, const drt_adaptive *adaptive, const drt_film *out)
+{
+    if(!ctx || !params || !adaptive) return fail(DRT_CUDA_E_ARG, "NULL argument");
+    int rc = adaptive_args(ctx, params, adaptive);
+    if(rc != DRT_CUDA_OK) return rc;
+    return render_host(ctx, params, adaptive, out);
 }
 
 extern "C" int drt_cuda_get_stats(drt_cuda_context *ctx, drt_cuda_stats *out)

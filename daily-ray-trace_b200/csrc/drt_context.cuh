@@ -21,6 +21,7 @@ void        drt_launch_fma_peak(int packed, float *out, int iters, int grid, cud
 void        drt_launch_film_gather_merge(const void *tables, int count, const FilmPtrs *films, FilmPtrs dst, uint32_t pixel_begin, uint32_t pixel_end, uint32_t src_base, uint32_t dst_base,
                                          uint32_t *bgra_sum, uint32_t *bgra_mean, uint32_t *bgra_var, int grid, cudaStream_t stream);
 size_t      drt_rgb_tables_bytes(void);
+size_t      drt_rgb_tables_yw_offset(void);   /* byte offset of the luminance weights cmf_y * ref_white (adaptive sampling) */
 void        drt_fill_rgb_tables(void *dst_host, const drt_tables *t);
 
 int drt_fail(int code, const char *fmt, ...);   /* records the message drt_cuda_last_error() returns (thread-local), returns code */

@@ -230,4 +230,12 @@ struct RenderLaunch
     uint32_t task_rotate;          /* tasks are walked from this index (mod the task count): with scatter_rank * slice every rank starts in its own
                                     * slice, so at any moment each owner receives from one peer instead of from all of them */
     FilmPtrs scatter[DRT_MAX_PEERS];
+    /* Adaptive sampling (drt_cuda_render_*_adaptive, render_kernel_adaptive): a pixel stops at the end of a batch once its count is
+     * >= min_samples and the bound on the standard error of its luminance is <= rel_error times the luminance (pixel_converged in
+     * drt_render.cuh).  luminance_w: the per-wavelength weights cmf_y * ref_white of the film-to-RGB tables, in device memory.
+     * adaptive = 0: every pixel takes all samples [sample_begin, sample_end). */
+    const float *luminance_w;
+    float    rel_error;
+    uint32_t min_samples;
+    uint32_t adaptive;
 };

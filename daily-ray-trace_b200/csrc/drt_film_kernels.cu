@@ -303,6 +303,7 @@ void drt_launch_film_gather_merge(const void *tables, int count, const FilmPtrs 
 }
 
 size_t drt_rgb_tables_bytes(void) { return sizeof(drt::RgbTables); }
+size_t drt_rgb_tables_yw_offset(void) { return offsetof(drt::RgbTables, yw); }
 
 void drt_fill_rgb_tables(void *dst_host, const drt_tables *t)
 {

@@ -8,7 +8,7 @@ import os
 import numpy as np
 
 from . import PACKAGE_DIR
-from ._structs import Camera, RenderParams, Scene, Tables
+from ._structs import Adaptive, Camera, RenderParams, Scene, Tables
 
 GEOMETRY_F32, GEOMETRY_F64 = 0, 1
 
@@ -19,7 +19,8 @@ EXPORTS = ["drt_cuda_last_error", "drt_cuda_device_count", "drt_cuda_create", "d
            "drt_cuda_film_ipc_open", "drt_cuda_film_ipc_close", "drt_cuda_film_merge_many", "drt_cuda_film_merge_slices", "drt_cuda_render_device_scatter", "drt_cuda_debug_records", "drt_cuda_buffer_alloc", "drt_cuda_buffer_free",
            "drt_cuda_buffer_ipc_export", "drt_cuda_buffer_ipc_open", "drt_cuda_buffer_ipc_close",
            "drt_cuda_film_merge_slices_local", "drt_cuda_film_read_slice", "drt_cuda_flags_signal", "drt_cuda_flags_wait", "drt_cuda_flags_timeouts",
-           "drt_cuda_host_alloc", "drt_cuda_host_free", "drt_cuda_render_host_multi_images", "drt_cuda_render_device_scatter_band", "drt_cuda_plan_scene"]
+           "drt_cuda_host_alloc", "drt_cuda_host_free", "drt_cuda_render_host_multi_images", "drt_cuda_render_device_scatter_band", "drt_cuda_plan_scene",
+           "drt_cuda_render_device_adaptive", "drt_cuda_render_host_adaptive"]
 
 
 class Film(C.Structure):
@@ -72,6 +73,8 @@ def lib():
         L.drt_cuda_film_merge_slices.argtypes = [C.c_void_p, C.POINTER(Film), C.POINTER(Film), C.c_int, C.c_uint64, C.c_uint32, C.c_uint32,
                                                  C.c_uint64, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         L.drt_cuda_render_host.argtypes = [C.c_void_p, C.POINTER(RenderParams), C.POINTER(Film)]
+        L.drt_cuda_render_device_adaptive.argtypes = [C.c_void_p, C.POINTER(RenderParams), C.POINTER(Adaptive), C.POINTER(Film), C.c_int, C.c_void_p]
+        L.drt_cuda_render_host_adaptive.argtypes = [C.c_void_p, C.POINTER(RenderParams), C.POINTER(Adaptive), C.POINTER(Film)]
         L.drt_cuda_film_merge_slices_local.argtypes = [C.c_void_p, C.POINTER(Film), C.POINTER(Film), C.c_int, C.c_uint64, C.c_uint32, C.c_uint32,
                                                        C.c_uint64, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         L.drt_cuda_film_read_slice.argtypes = [C.c_void_p, C.POINTER(Film), C.c_uint64, C.c_uint64, C.c_uint64, C.POINTER(Film), C.c_void_p]
@@ -161,6 +164,21 @@ class Context:
         film = Film(out["sum"].ctypes.data, out["filter"].ctypes.data, out["mean"].ctypes.data, out["m2"].ctypes.data)
         _check(lib().drt_cuda_render_host(self._h, C.byref(params), C.byref(film)))
         return out
+
+    def render_host_adaptive(self, params, rel_error, min_samples):
+        """render_host with adaptive sampling (drt_cuda_render_host_adaptive): every pixel stops once the error bound of its luminance
+        is <= rel_error times the luminance and it has >= min_samples samples; filter holds each pixel's count."""
+        npix = max(params.width * params.height, 1)
+        n = self.n or 1
+        out = {"sum": np.empty((npix, n), np.float32), "filter": np.empty(npix, np.float32),
+               "mean": np.empty((npix, n), np.float32), "m2": np.empty((npix, n), np.float32)}
+        film = Film(out["sum"].ctypes.data, out["filter"].ctypes.data, out["mean"].ctypes.data, out["m2"].ctypes.data)
+        _check(lib().drt_cuda_render_host_adaptive(self._h, C.byref(params), C.byref(Adaptive(rel_error, min_samples)), C.byref(film)))
+        return out
+
+    def render_device_adaptive(self, params, rel_error, min_samples, film, accumulate=False, stream=None):
+        _check(lib().drt_cuda_render_device_adaptive(self._h, C.byref(params), C.byref(Adaptive(rel_error, min_samples)), C.byref(film),
+                                                     int(accumulate), stream))
 
     def render_host_into(self, params, film):
         _check(lib().drt_cuda_render_host(self._h, C.byref(params), C.byref(film)))

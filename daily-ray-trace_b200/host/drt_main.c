@@ -6,11 +6,14 @@
  * (win32_main.c:129-152).  The render itself goes through the C ABI of include/drt_cuda.h; the timed region is the
  * reference's render_timer scope (sampling + film accumulation, daily_ray_trace.c:709-752; file I/O excluded).
  *
- *   drt_raytrace [config.cfg] [--device N] [--gpus G] [--seed S] [--strict] [--f64-geometry] [--cpu-images]
+ *   drt_raytrace [config.cfg] [--device N] [--gpus G] [--seed S] [--strict] [--f64-geometry] [--cpu-images] [--adaptive REL [--min-spp M]]
  * --gpus G renders on devices N .. N+G-1: the samples of every pixel are split over them (drt_cuda_render_host_multi_images).
  * The three .bmp images come from the devices with the film (converted from the merged film there, fused into the multi-GPU merge
  * kernel); --cpu-images converts them the reference's way instead: by reading the .spd files back (spd_file_to_rgb_f64_pixels,
  * daily_ray_trace.c:1-28, in f64 -- bytes may differ by 1 from the device's f32 conversion).
+ * --adaptive REL samples adaptively (drt_cuda_render_host_adaptive): a pixel stops once the error bound of its luminance is at most REL
+ * times the luminance and it has at least M samples (--min-spp, default 64, at most num_pixel_samples); num_pixel_samples is the cap.
+ * One device only, and the .bmp images are converted from the .spd files as with --cpu-images.
  */
 #include <stdio.h>
 #include <stdlib.h>
@@ -42,8 +45,9 @@ static int spd_to_bmp(const char *spd, const char *bmp, const drt_tables *t)
 int main(int argc, char **argv)
 {
     const char *config_path = "config.cfg";
-    int device = 0, gpus = 1, flags = DRT_PARSE_LEGACY_COMPAT, precision = DRT_GEOMETRY_F32, cpu_images = 0;
+    int device = 0, gpus = 1, flags = DRT_PARSE_LEGACY_COMPAT, precision = DRT_GEOMETRY_F32, cpu_images = 0, adaptive = 0;
     unsigned long long seed = 0;
+    drt_adaptive ad = { 0.f, 64u };
     for(int i = 1; i < argc; i += 1)
     {
         if(strcmp(argv[i], "--device") == 0 && i + 1 < argc) device = atoi(argv[++i]);
@@ -52,8 +56,17 @@ int main(int argc, char **argv)
         else if(strcmp(argv[i], "--strict") == 0) flags = DRT_PARSE_STRICT;
         else if(strcmp(argv[i], "--f64-geometry") == 0) precision = DRT_GEOMETRY_F64;
         else if(strcmp(argv[i], "--cpu-images") == 0) cpu_images = 1;
+        else if(strcmp(argv[i], "--adaptive") == 0 && i + 1 < argc) { adaptive = 1; ad.rel_error = strtof(argv[++i], NULL); }
+        else if(strcmp(argv[i], "--min-spp") == 0 && i + 1 < argc) ad.min_samples = (uint32_t)strtoul(argv[++i], NULL, 0);
         else config_path = argv[i];
     }
+    if(adaptive && gpus != 1)
+    {
+        /* with the samples of a pixel split over devices no device sees the merged film the stopping rule needs */
+        fprintf(stderr, "ERROR: --adaptive renders on one GPU: it cannot be combined with --gpus %d\n", gpus);
+        return 1;
+    }
+    if(adaptive) cpu_images = 1;
 
     drt_config cfg;
     if(drt_parse_config_file(config_path, &cfg) != DRT_OK) return die_host("config");
@@ -98,9 +111,12 @@ int main(int argc, char **argv)
     prm.sample_begin = 0; prm.sample_end = cfg.num_pixel_samples;
     prm.max_depth = cfg.max_cast_depth; prm.pixel_scheme = cfg.pixel_scheme; prm.seed = seed;
 
+    if(adaptive && ad.min_samples > cfg.num_pixel_samples) ad.min_samples = cfg.num_pixel_samples;
+
     printf("Starting render...\n");
     double t0 = now_ms();
-    int rrc = cpu_images ? drt_cuda_render_host_multi(ctxs, gpus, &prm, &film)
+    int rrc = adaptive   ? drt_cuda_render_host_adaptive(ctxs[0], &prm, &ad, &film)
+            : cpu_images ? drt_cuda_render_host_multi(ctxs, gpus, &prm, &film)
                          : drt_cuda_render_host_multi_images(ctxs, gpus, &prm, &film, images[0], images[1], images[2]);
     if(rrc != DRT_CUDA_OK) return die_cuda("render");
     double ms = now_ms() - t0;
@@ -116,6 +132,9 @@ int main(int argc, char **argv)
     printf("Total render time: %fms\n", ms);
     printf("Camera paths: %llu (%.3f Mpaths/s), rays: %llu (%.3f Mrays/s)\n", (unsigned long long)st.paths, (double)st.paths / ms * 1e-3,
            (unsigned long long)(st.closest_rays + st.shadow_rays), (double)(st.closest_rays + st.shadow_rays) / ms * 1e-3);
+    if(adaptive)
+        printf("Adaptive sampling: rel_error %g, min %u, cap %u samples per pixel; mean %.2f samples per pixel\n", (double)ad.rel_error,
+               ad.min_samples, cfg.num_pixel_samples, npix ? (double)st.paths / (double)npix : 0.0);
     printf("Render complete.\n");
 
     if(drt_write_spd_sum(cfg.output_spd, &tables, prm.width, prm.height, film.sum, film.filter) != DRT_OK) return die_host("output spd");

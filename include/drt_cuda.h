@@ -102,6 +102,30 @@ int  drt_cuda_render_device_scatter(drt_cuda_context *ctx, const drt_render_para
  * `film_host` (pinned or pageable) and waits.  This is the end-to-end call the Linux main uses. */
 int  drt_cuda_render_host(drt_cuda_context *ctx, const drt_render_params *params, const drt_film *film_host);
 
+/* Adaptive sampling: every pixel takes samples from sample_begin on in batches of 32 and stops at the end of the first batch after which
+ * its film (count n, including samples an accumulate=1 call loaded) satisfies
+ *     n >= min_samples  and  err <= rel_error * Y,   Y = sum_l w_l mean_l,   err = sum_l w_l sqrt(M2_l / (n (n - 1)))
+ * with w_l the luminance weights cmf_y * ref_white of the .bmp conversion (err bounds the standard error of Y from above: the sd of a
+ * sum is at most the sum of the sds), or when the samples of [sample_begin, sample_end) run out.  Sample s of a pixel is the same path
+ * as in a uniform render, so a pixel that stops after k samples holds the film of [sample_begin, sample_begin + k): k is a multiple of
+ * 32, or the whole range.  The filter plane holds each pixel's count, so sum / filter stays the mean; M2 (and the variance image) is a
+ * sum over a count that varies from pixel to pixel.  Pixels whose samples are all zero (also those the screen-space culling counts
+ * instead of tracing) and pixels without variance stop at the first batch end at or past min_samples; pixels with Y = 0 but noise, and
+ * pixels whose film holds a NaN, run to the end of the range.  drt_cuda_get_stats reports the paths actually taken.
+ * rel_error: finite, > 0; min_samples: 32 ..  sample_end - sample_begin (so the range holds at least 32 samples); else DRT_CUDA_E_ARG.
+ * f64 geometry (a diagnostic) has no adaptive kernel: DRT_CUDA_E_UNSUPPORTED.  There is no multi-GPU form: with the samples of a
+ * pixel split over devices, no device sees the merged film the rule needs. */
+typedef struct
+{
+    float    rel_error;
+    uint32_t min_samples;
+} drt_adaptive;
+
+int  drt_cuda_render_device_adaptive(drt_cuda_context *ctx, const drt_render_params *params, const drt_adaptive *adaptive,
+                                     const drt_film *film_device, int accumulate, void *stream);
+int  drt_cuda_render_host_adaptive(drt_cuda_context *ctx, const drt_render_params *params, const drt_adaptive *adaptive,
+                                   const drt_film *film_host);
+
 /* render_host on several devices of ONE process (what `drt_raytrace --gpus G` calls): contexts[g] live on distinct devices and hold
  * the same scene; the samples [sample_begin, sample_end) are split evenly over them.  With peer access every device renders its share
  * of every pixel with drt_cuda_render_device_scatter, announces it with device-side flags (drt_cuda_flags_signal / _wait, no host
