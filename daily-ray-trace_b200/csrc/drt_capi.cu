@@ -970,6 +970,21 @@ extern "C" int drt_cuda_get_stats(drt_cuda_context *ctx, drt_cuda_stats *out)
     return DRT_CUDA_OK;
 }
 
+#ifdef DRT_PHASE_CLOCKS
+/* Diagnostic builds only (tools/phase_split.py): the warp cycles of the last render call by part of a batch -- trace, batch
+ * bookkeeping, replay, other (DRT_PHASE_* in drt_render.cuh).  Not part of include/drt_cuda.h. */
+extern "C" int drt_cuda_phase_clocks(drt_cuda_context *ctx, uint64_t out[4])
+{
+    if(!ctx || !out) return fail(DRT_CUDA_E_ARG, "NULL argument");
+    CU(cudaSetDevice(ctx->device));
+    CU(cudaDeviceSynchronize());
+    DeviceStats s;
+    CU(cudaMemcpy(&s, ctx->d_stats, sizeof(s), cudaMemcpyDeviceToHost));
+    for(int i = 0; i < 4; i += 1) out[i] = s.phase_clocks[i];
+    return DRT_CUDA_OK;
+}
+#endif
+
 extern "C" int drt_cuda_sample_paths(drt_cuda_context *ctx, const drt_render_params *params,
                                      uint32_t x0, uint32_t y0, uint32_t x1, uint32_t y1, float *out_host)
 {

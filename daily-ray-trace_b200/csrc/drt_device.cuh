@@ -155,6 +155,10 @@ struct DeviceStats
     unsigned long long paths, closest_rays, shadow_rays, shaded_bounces, rng_draws;
     unsigned long long terminated_at_depth[8];
     unsigned long long reached_depth_cap;
+#ifdef DRT_PHASE_CLOCKS
+    /* diagnostic builds only: SM-clock cycles the warps spent in each part of a batch (DRT_PHASE_* in drt_render.cuh) */
+    unsigned long long phase_clocks[4];
+#endif
 };
 
 /* Path record in shared memory, one row per path slot (word w of slot s at rec[s*path_stride + w]; path_stride is 4 times an

@@ -503,17 +503,41 @@ template <typename T> __device__ __forceinline__ T fresnel_dielectric(T ir, T tr
 
 /* ------------------------------------------------------------------ K4: the six direction samplers, bdsf.c:191-292 */
 
+/* sin(pi u) and cos(pi u) for |u| <= 1/4, inline and without range reduction: minimax polynomials in v = u^2 whose float32
+ * coefficients come from tools/fit_sincospi_quarter.py (numpy, float64 fit).  Under 1 ulp from float64 sin / cos on a dense grid and
+ * on the float32 values next to 0 and +-1/4 (tests/test_trace_trim.py models this evaluation order). */
+__device__ __forceinline__ void sincospi_quarter(float u, float &s, float &c)
+{
+    const float v = u * u;
+    const float ps = fmaf(fmaf(-0x1.330cc6p-1f, v, 0x1.46805cp+1f), v, -0x1.4abc24p+2f);
+    s = fmaf(u, 0x1.921fb6p+1f, (u * v) * ps);
+    const float pc = fmaf(fmaf(fmaf(0x1.d9f7bcp-3f, v, -0x1.55c664p+0f), v, 0x1.03c1dep+2f), v, -0x1.3bd3ccp+2f);
+    c = fmaf(v, pc, 1.f);
+}
+
+/* sin and cos of the concentric map's angle: pi/4 q, or pi/2 - pi/4 q for the `steep` octants (q = the smaller coordinate over the
+ * larger, in [-1, 1]).  f32: sin(pi/2 - x) = cos(x), so both come from sincospi_quarter(q / 4) with s and c swapped; f64 (the branch-
+ * flip diagnostic) keeps the library's sincos. */
+__device__ __forceinline__ void disc_sincos(float q, bool steep, float &s, float &c)
+{
+    float a, b;
+    sincospi_quarter(0.25f * q, a, b);
+    s = steep ? b : a; c = steep ? a : b;
+}
+__device__ __forceinline__ void disc_sincos(double q, bool steep, double &s, double &c) { r_sincospi(steep ? 0.5 - 0.25 * q : 0.25 * q, &s, &c); }
+
 template <typename R> __device__ __forceinline__ V3<R> sample_disc(Rng &rng)   /* uniform_sample_disc, rng.c:25-51 */
 {
     R rx = rng.unit<R>();
     R ry = rng.unit<R>();
     R ox = R(2) * rx - R(1), oy = R(2) * ry - R(1);
     if(ox == R(0) && oy == R(0)) return mk<R>(R(0), R(0), R(0));
-    R r, t;   /* t in units of pi */
-    if(r_abs(ox) > r_abs(oy)) { r = ox; t = R(0.25) * r_div(oy, ox); }
-    else                      { r = oy; t = R(0.5) - R(0.25) * r_div(ox, oy); }
+    R r, q;
+    const bool steep = !(r_abs(ox) > r_abs(oy));
+    if(!steep) { r = ox; q = r_div(oy, ox); }
+    else       { r = oy; q = r_div(ox, oy); }
     R s, c;
-    r_sincospi(t, &s, &c);
+    disc_sincos(q, steep, s, c);
     return mk<R>(r * c, r * s, R(0));
 }
 
@@ -781,11 +805,23 @@ __device__ __forceinline__ uint32_t trace_path(const GeomT<R> &g, const SpdIndex
         }
         /* K4: sample the next direction and evaluate the BSDF for it, cast_ray :464-472 */
         V3<R> in; R inv_pdf; int match;
-        sample_direction<R>(g, h, rng, in, inv_pdf, match);
         const uint32_t es = 2 + (ew + 1) * (uint32_t)nlights;
         float wd_s = 0.f, wg_s = 0.f;
-        if(plastic) plastic_weights<R>(g, sm, h.nrm, h.out, in, (float)inv_pdf, wd_s, wg_s);
-        else if(!CLASSED) eval_weights_general<R>(g, sm, h.nrm, h.out, h.on_dot, in, match, (float)inv_pdf, rb, es);
+        if(ALLFAST && plastic && depth + 1 == L.max_depth && g.dirf[sm] == DRT_DIR_COS_WEIGHTED_HEMISPHERE)
+        {
+            /* The last bounce's sampled direction is never cast, and the compact replay multiplies its weights by e = 0 (replay_compact):
+             * it is not sampled, and its weights are 0.  The cosine sampler's two draws are still counted.  No draw follows them in
+             * this path (the next path has a stream of its own), so only the draw counter sees them; it differs from the reference's
+             * only when the disc sample would have been rejected (|q| rounds to 1, Q16). */
+            rng.draws += 2;
+            in = h.nrm;
+        }
+        else
+        {
+            sample_direction<R>(g, h, rng, in, inv_pdf, match);
+            if(plastic) plastic_weights<R>(g, sm, h.nrm, h.out, in, (float)inv_pdf, wd_s, wg_s);
+            else if(!CLASSED) eval_weights_general<R>(g, sm, h.nrm, h.out, h.on_dot, in, match, (float)inv_pdf, rb, es);
+        }
         if(ALLFAST)
         {
             uint32_t hdr16;
@@ -1594,6 +1630,22 @@ static __device__ __noinline__ void dump_path(float *record_dump, float *path_du
  * contains neither the general lobe evaluators nor the general shader. */
 #ifndef DRT_PARK_GENERAL
 #define DRT_PARK_GENERAL 0   /* park the film of the general kernel too (pays off only if that buys resident warps) */
+#endif
+/* Phase clocks, diagnostic builds only (tools/build_variant.sh NAME -DDRT_PHASE_CLOCKS; tools/phase_split.py reads them through
+ * drt_cuda_phase_clocks).  Each warp's timeline after the scene staging is cut at the boundaries of a batch, and the SM-clock cycles
+ * since the previous cut go to the part that just ended: TRACE = phase 1 (film parking, the gate in front of it, trace_path), BOOK =
+ * the batch bookkeeping (histogram, sort, zero counts, film unpark, add_batch, the phase-2 gate), REPLAY = phase 2 (the replay of the
+ * records and BatchStats::add), OTHER = task fetch, film load / store, culled pixels.  Lane 0 adds each piece to a shared-memory
+ * counter.  Without the flag the macro is empty and the kernels compile to the same code. */
+#define DRT_PHASE_TRACE  0
+#define DRT_PHASE_BOOK   1
+#define DRT_PHASE_REPLAY 2
+#define DRT_PHASE_OTHER  3
+#ifdef DRT_PHASE_CLOCKS
+#define DRT_PHASE_CUT(k) do { uint32_t t_; asm volatile("mov.u32 %0, %%clock;" : "=r"(t_) :: "memory"); \
+                              if(lane == 0) atomicAdd(&s_phase[k], (unsigned long long)(t_ - phase_t)); phase_t = t_; } while(0)
+#else
+#define DRT_PHASE_CUT(k) do {} while(0)
 #endif
 /* PAIRED: one pixel per task with all its samples (spp >= 32) against 32/spp whole pixels per task; see the task loop. */
 #define DRT_RENDER_BOUNDS(MODE) __launch_bounds__((MODE == 1 ? DRT_FAST_WARPS : MODE == 2 ? DRT_CLASSED_WARPS : DRT_CTA_WARPS) * DRT_WARP, \

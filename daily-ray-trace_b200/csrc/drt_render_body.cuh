@@ -14,6 +14,11 @@
     constexpr bool LOCKSTEP = MODE == 2 ? ((DRT_LOCKSTEP & 2) != 0) : MODE == 0 ? ((DRT_LOCKSTEP & 1) != 0) : ((DRT_LOCKSTEP & 4) != 0);
     __shared__ unsigned long long phase_bar;
     __shared__ uint32_t gates_off;
+#ifdef DRT_PHASE_CLOCKS
+    __shared__ unsigned long long s_phase[4];
+    uint32_t phase_t = 0;
+    if(threadIdx.x < 4) s_phase[threadIdx.x] = 0ull;
+#endif
     const uint32_t bar_addr = (uint32_t)__cvta_generic_to_shared(&phase_bar);
     if(LOCKSTEP && threadIdx.x == 0)
     {
@@ -53,6 +58,9 @@
 
     const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
     const uint32_t lane16 = lane & (DRT_HALF - 1), half = lane >> 4;
+#ifdef DRT_PHASE_CLOCKS
+    asm volatile("mov.u32 %0, %%clock;" : "=r"(phase_t) :: "memory");
+#endif
     float *rec = srec + (size_t)warp * L.path_stride * DRT_WARP;   /* word w of slot s at rec[s * path_stride + w] */
     const uint32_t stride = L.path_stride;
     float *park = spark + (size_t)warp * (3 * NS + 2) * DRT_WARP + lane;
@@ -170,6 +178,7 @@
         for(uint32_t q0 = 0; q0 < total; q0 += DRT_WARP)
         {
             /* ---- phase 1: lane = path ---- */
+            DRT_PHASE_CUT(DRT_PHASE_OTHER);
             gate();
             if((ALLFAST || DRT_PARK_GENERAL) && paired) film.park(park);
             const uint32_t q = q0 + lane;
@@ -195,6 +204,7 @@
                 }
             }
             __syncwarp();
+            DRT_PHASE_CUT(DRT_PHASE_TRACE);
             gate();
             /* compact records: the film stays parked through the replay, which accumulates BatchStats instead */
             if(!ALLFAST && DRT_PARK_GENERAL && paired) film.unpark(park);
@@ -212,6 +222,7 @@
                 if(ALLFAST) film.unpark(park);
                 if(half == 0) film.add_zeros(count);
                 __syncwarp();
+                DRT_PHASE_CUT(DRT_PHASE_BOOK);
                 if constexpr(ADAPTIVE)
                     if(pixel_converged<NS>(film, L, n, lane16)) { traced -= total - (q0 + count); break; }
                 continue;
@@ -261,6 +272,7 @@
                     }
                 BatchStats<NS> bs;
                 if(ALLFAST) bs.clear();
+                DRT_PHASE_CUT(DRT_PHASE_BOOK);
                 for(uint32_t i = lo + nzero; i < lo + per_px; i += 2)
                 {
                     const uint32_t pos = i + half;
@@ -297,6 +309,7 @@
                         }
                     }
                 }
+                DRT_PHASE_CUT(DRT_PHASE_REPLAY);
                 if constexpr(ALLFAST)
                 {
                     if(paired) film.unpark(park);
@@ -310,6 +323,7 @@
                 }
             }
             __syncwarp();
+            DRT_PHASE_CUT(DRT_PHASE_BOOK);
             /* A warp that ends its pixel here has passed both gates of this batch, like one that ends it with its last batch: the
              * phase gates of the classed kernel see no difference. */
             if constexpr(ADAPTIVE)
@@ -322,6 +336,7 @@
         }
     }
 
+    DRT_PHASE_CUT(DRT_PHASE_OTHER);
     /* work counters: one shared-memory atomic per warp per counter, then one global atomic per CTA per counter */
 #pragma unroll
     for(int k = 0; k < 4; k += 1)
@@ -335,3 +350,6 @@
     __syncthreads();
     if(threadIdx.x < 14 && s_stats[threadIdx.x])
         atomicAdd(reinterpret_cast<unsigned long long *>(L.stats) + threadIdx.x, s_stats[threadIdx.x]);
+#ifdef DRT_PHASE_CLOCKS
+    if(threadIdx.x < 4) atomicAdd(&L.stats->phase_clocks[threadIdx.x], s_phase[threadIdx.x]);
+#endif
