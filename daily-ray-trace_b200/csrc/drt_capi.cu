@@ -1207,6 +1207,9 @@ extern "C" int drt_cuda_film_merge_slices(drt_cuda_context *ctx, const drt_film 
     for(int g = 0; g < count; g += 1)   /* rank g's partial film of this slice: staging pixels [g * slice, (g + 1) * slice) */
         films[g] = FilmPtrs{ staging->sum + (size_t)g * slice_pixels * n, staging->filter + (size_t)g * slice_pixels,
                              staging->mean + (size_t)g * slice_pixels * n, staging->m2 + (size_t)g * slice_pixels * n };
+    /* staging is indexed from the first pixel of the owner's slice; [pixel_begin, pixel_end) may be a part (a band) of it */
+    const uint64_t slice_begin = slice_pixels ? (pixel_begin / slice_pixels) * slice_pixels : 0;
+    if(pixel_end > pixel_begin && pixel_end - slice_begin > slice_pixels) return fail(DRT_CUDA_E_ARG, "pixel range crosses a slice boundary");
     if(pixel_end > pixel_begin)
     {
         /* merged planes of the slice go to a local scratch film first and travel to dst_device (the root's film: usually peer
@@ -1217,7 +1220,7 @@ extern "C" int drt_cuda_film_merge_slices(drt_cuda_context *ctx, const drt_film 
         if(rc != DRT_CUDA_OK) return rc;
         float *base = ctx->d_slice;
         FilmPtrs d = { base, base + 3 * (plane / 4), base + plane / 4, base + 2 * (plane / 4) };
-        drt_launch_film_gather_merge(ctx->d_rgb_tables, count, films, d, (uint32_t)pixel_begin, (uint32_t)pixel_end, (uint32_t)pixel_begin,
+        drt_launch_film_gather_merge(ctx->d_rgb_tables, count, films, d, (uint32_t)pixel_begin, (uint32_t)pixel_end, (uint32_t)slice_begin,
                                      (uint32_t)pixel_begin, bgra_sum, bgra_mean, bgra_var, ctx->num_sms * 8, (cudaStream_t)stream);
         CU(cudaGetLastError());
         const size_t at = (size_t)pixel_begin * n;

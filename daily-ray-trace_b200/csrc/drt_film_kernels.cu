@@ -108,7 +108,8 @@ __global__ void __launch_bounds__(256) film_merge_kernel(FilmPtrs dst, FilmPtrs 
         float nab = na + nb;
         float ma = dst.mean[i], mb = src.mean[i];
         float delta = mb - ma;
-        float wb = (nab > 0.f) ? nb / nab : 0.f;
+        /* correctly rounded: the build's -prec-div=false division can give nb / nb != 1, and merging into an empty film must be exact */
+        float wb = (nab > 0.f) ? __fdiv_rn(nb, nab) : 0.f;
         dst.mean[i] = fmaf(delta, wb, ma);
         dst.m2[i] = dst.m2[i] + src.m2[i] + delta * delta * na * wb;
         dst.sum[i] = dst.sum[i] + src.sum[i];
@@ -168,7 +169,7 @@ __global__ void __launch_bounds__(256) film_gather_merge_kernel(const RgbTables 
             for(int c = 0; c < CHUNK; c += 1)
             {
                 float nab = cnt + nb[c];
-                float wb = (nab > 0.f) ? nb[c] / nab : 0.f;
+                float wb = (nab > 0.f) ? __fdiv_rn(nb[c], nab) : 0.f;   /* exact 1 for the first non-empty film (see film_merge_kernel) */
 #pragma unroll
                 for(int k = 0; k < DRT_MAX_SLOTS; k += 1)
                 {

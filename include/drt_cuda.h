@@ -217,7 +217,9 @@ int  drt_cuda_film_merge_many(drt_cuda_context *ctx, const drt_film *dst_device,
 /* The merge half of the scattered exchange, ONE kernel per rank on LOCAL data: merges the `count` partial films of this rank's
  * slice [pixel_begin, pixel_end) held in staging_device (layout of drt_cuda_render_device_scatter) into a library-owned
  * local scratch film, writes the three images like drt_cuda_film_merge_many, then copies the merged planes to dst_device at
- * the global pixel positions (may be peer memory, e.g. the root's film) as four contiguous stream-ordered copies. */
+ * the global pixel positions (may be peer memory, e.g. the root's film) as four contiguous stream-ordered copies.
+ * [pixel_begin, pixel_end) may be a part (a band) of the slice: staging stays indexed from the slice's first pixel.  A range that
+ * crosses a slice boundary is DRT_CUDA_E_ARG. */
 int  drt_cuda_film_merge_slices(drt_cuda_context *ctx, const drt_film *dst_device, const drt_film *staging_device, int count, uint64_t slice_pixels,
                                 uint32_t width, uint32_t height, uint64_t pixel_begin, uint64_t pixel_end,
                                 uint32_t *bgra_sum, uint32_t *bgra_mean, uint32_t *bgra_var, void *stream);
