@@ -222,7 +222,9 @@ static int classify_material(const drt_scene *s, int m, int *nd_out, int *ng_out
     return DRT_CLASS_GENERAL;
 }
 
-/* Which render kernel a scene gets (drt_render.cuh): 1 plastic-only, 2 classed, 0 general. */
+/* Which render kernel a scene gets (drt_render.cuh): 1 plastic-only, 2 classed, 0 general.  The compact-record kernels (1, 2) carry
+ * throughput * E(light): the only emitter a path can run into must then be that light, so an emissive escape material (a sky, Q19) or
+ * a second light sends the scene to the general kernel. */
 static int scene_kernel_mode(const drt_scene *scene)
 {
     int nlights = 0;
@@ -451,6 +453,15 @@ extern "C" int drt_cuda_validate_scene(const drt_scene *scene)
     return DRT_CUDA_OK;
 }
 
+/* The compact records address the D, G blocks with 16-bit word offsets.  The pool of a scene that passes drt_cuda_validate_scene, with
+ * rows of npad <= DRT_MAX_HALF_SLOTS * 16 words, holds at most row 0 and one row per material SPD, a D, G block per material and the
+ * light's emission in slot pairs (each 16-byte aligned), and three Fresnel rows per orientation of every material but the base one. */
+static_assert((1 + DRT_MAX_MATERIALS * DRT_SPD_COUNT) * DRT_MAX_HALF_SLOTS * DRT_HALF
+                  + DRT_MAX_MATERIALS * ((DRT_MAX_HALF_SLOTS + 1) / 2 * 4 * DRT_HALF + 3)
+                  + ((DRT_MAX_HALF_SLOTS + 1) / 2 * 2 * DRT_HALF + 3)
+                  + (DRT_MAX_MATERIALS - 1) * 2 * 3 * DRT_MAX_HALF_SLOTS * DRT_HALF <= 65535,
+              "the spectrum pool can outgrow the 16-bit offsets of the compact records");
+
 extern "C" int drt_cuda_upload_scene(drt_cuda_context *ctx, const drt_scene *scene, const drt_camera *camera, const drt_tables *tables)
 {
     if(!ctx || !scene || !camera || !tables) return fail(DRT_CUDA_E_ARG, "NULL argument");
@@ -458,8 +469,6 @@ extern "C" int drt_cuda_upload_scene(drt_cuda_context *ctx, const drt_scene *sce
     if(vrc != DRT_CUDA_OK) return vrc;
     CU(cudaSetDevice(ctx->device));
     const int n = scene->num_wavelengths;
-    const uint32_t i0 = (uint32_t)((DRT_TRANS_WL - scene->min_wl) / scene->wl_interval);
-    (void)i0;
 
     GeomT<float> *g32 = new GeomT<float>();
     GeomT<double> *g64 = new GeomT<double>();
@@ -488,48 +497,10 @@ extern "C" int drt_cuda_upload_scene(drt_cuda_context *ctx, const drt_scene *sce
             for(int i = 0; i < n; i += 1) pool[at + (size_t)i] = (float)scene->materials[m].spd[k][i];
         }
     index.nrows = rows;
-    /* interleaved plastic blocks (SpdIndex::plastic) for the two-lobe Blinn-Phong materials when the scene has one light */
     if(g32->nlights == 1)
     {
-        const double *emission = scene->materials[scene->surfaces[g32->light_surf[0]].material].spd[DRT_SPD_EMISSION];
-        const bool have_e = (scene->materials[scene->surfaces[g32->light_surf[0]].material].spd_mask & (1 << DRT_SPD_EMISSION)) != 0;
-        for(int m = 0; m < scene->num_materials; m += 1)
-        {
-            const drt_material *mm = &scene->materials[m];
-            if(mm->is_black_body || mm->num_lobes != 2 || g32->bmask[m] != ((1 << BK_DIFFUSE) | (1 << BK_GLOSSY))) continue;
-            size_t at = (pool.size() + 3) & ~(size_t)3;
-            pool.resize(at + (size_t)half_slots * 64, 0.f);
-            index.plastic[m] = (int)at;
-            auto val = [&](int k, int slot, int lane) -> float {
-                int wl = lane + slot * 16;
-                return (wl < n && (mm->spd_mask & (1 << k))) ? (float)mm->spd[k][wl] : 0.f;
-            };
-            auto emi = [&](int slot, int lane) -> float {
-                int wl = lane + slot * 16;
-                return (wl < n && have_e) ? (float)emission[wl] : 0.f;
-            };
-            const int np = half_slots / 2;
-            for(int lane = 0; lane < 16; lane += 1)
-            {
-                for(int pr = 0; pr < np; pr += 1)
-                    for(int j = 0; j < 2; j += 1)
-                    {
-                        int slot = 2 * pr + j;
-                        float d = val(DRT_SPD_DIFFUSE, slot, lane), gl = val(DRT_SPD_GLOSSY, slot, lane), e = emi(slot, lane);
-                        float *c0 = &pool[at + ((size_t)(2 * pr) * 16 + lane) * 4], *c1 = &pool[at + ((size_t)(2 * pr + 1) * 16 + lane) * 4];
-                        c0[j] = d; c0[2 + j] = gl; c1[j] = d * e; c1[2 + j] = gl * e;
-                    }
-                if(half_slots & 1)
-                {
-                    int slot = half_slots - 1;
-                    float d = val(DRT_SPD_DIFFUSE, slot, lane), gl = val(DRT_SPD_GLOSSY, slot, lane), e = emi(slot, lane);
-                    float *c = &pool[at + ((size_t)(half_slots - 1) * 16 + lane) * 4];
-                    c[0] = d; c[1] = gl; c[2] = d * e; c[3] = gl * e;
-                }
-            }
-        }
-        /* the D, G blocks of the compact-record kernels (SpdIndex::plastic2): every material whose lobes are all bp_diffuse /
-         * bp_glossy; a lobe listed k times counts k times (bdsf() sums the lobes, daily_ray_trace.c:215-229) */
+        /* the D, G blocks of the plastic bounces (SpdIndex::plastic2): every material whose lobes are all bp_diffuse / bp_glossy;
+         * a lobe listed k times counts k times (bdsf() sums the lobes, daily_ray_trace.c:215-229) */
         for(int m = 0; m < scene->num_materials; m += 1)
         {
             const drt_material *mm = &scene->materials[m];
@@ -556,6 +527,8 @@ extern "C" int drt_cuda_upload_scene(drt_cuda_context *ctx, const drt_scene *sce
                 }
         }
         /* the light's emission in slot pairs (SpdIndex::light_pairs) */
+        const double *emission = scene->materials[scene->surfaces[g32->light_surf[0]].material].spd[DRT_SPD_EMISSION];
+        const bool have_e = (scene->materials[scene->surfaces[g32->light_surf[0]].material].spd_mask & (1 << DRT_SPD_EMISSION)) != 0;
         const int nchunks = (half_slots + 1) / 2;
         size_t ate = (pool.size() + 3) & ~(size_t)3;
         pool.resize(ate + (size_t)nchunks * 32, 0.f);
@@ -621,16 +594,10 @@ extern "C" int drt_cuda_upload_scene(drt_cuda_context *ctx, const drt_scene *sce
     if(e == cudaSuccess) e = cudaMemcpy(ctx->d_pool, pool.data(), pool.size() * 4, cudaMemcpyHostToDevice);
     if(e == cudaSuccess) e = cudaMemcpy(ctx->d_rgb_tables, rgbt.data(), rgbt.size(), cudaMemcpyHostToDevice);
     int nlights = g32->nlights;
-    /* The compact-record kernels carry throughput * E(light): the only emitter a path can run into must then be that light, so an
-     * emissive escape material (a sky, Q19) or a second light sends the scene to the general kernel.  all_fast: every surface
-     * material is a plastic (kernel mode 1); classed: plastics, single-basis specular materials and ct_conductor (mode 2). */
-    int mode = scene_kernel_mode(scene);
-    bool all_fast = mode == 1, classed = mode != 0;
-    if(pool.size() > 65535) all_fast = classed = false;   /* compact records address the blocks with 16-bit word offsets */
     int eval_words = g32->eval_words > 0 ? g32->eval_words : 1;
     delete g32; delete g64;
     if(e != cudaSuccess) return fail(DRT_CUDA_E_CUDA, "scene upload: %s", cudaGetErrorString(e));
-    ctx->n = n; ctx->nslots = index.nslots; ctx->nlights = nlights; ctx->eval_words = eval_words; ctx->all_fast = all_fast; ctx->classed = classed && !all_fast; ctx->pool_words = (uint32_t)pool.size();
+    ctx->n = n; ctx->nslots = index.nslots; ctx->nlights = nlights; ctx->eval_words = eval_words; ctx->scene_mode = scene_kernel_mode(scene); ctx->pool_words = (uint32_t)pool.size();
     ctx->upload_bytes = sizeof(GeomT<float>) + sizeof(GeomT<double>) + sizeof(SpdIndex) + pool.size() * 4 + rgbt.size();
     ctx->have_scene = true;
     return DRT_CUDA_OK;
@@ -660,7 +627,7 @@ extern "C" int drt_cuda_film_sizes(const drt_cuda_context *ctx, uint32_t width, 
 
 /* which instantiation of the render kernel serves the uploaded scene: 0 general (any lobe list, any number of lights; always for the
  * f64-geometry diagnostic), 1 plastic-only, 2 classed (drt_render.cuh) */
-static int kernel_mode(const drt_cuda_context *ctx) { return ctx->f64_geometry ? 0 : ctx->all_fast ? 1 : ctx->classed ? 2 : 0; }
+static int kernel_mode(const drt_cuda_context *ctx) { return ctx->f64_geometry ? 0 : ctx->scene_mode; }
 
 /* record layout of a render with `max_depth` bounces (RenderLaunch in drt_device.cuh) */
 static void record_layout(const drt_cuda_context *ctx, uint32_t max_depth, uint32_t smem_depth, RenderLaunch &L)

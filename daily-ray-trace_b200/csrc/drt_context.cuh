@@ -41,8 +41,7 @@ struct drt_cuda_context
     int    n = 0, nslots = 0, nlights = 0, eval_words = 1;
     bool   hit_bound = false;      /* hit_u/v: film-plane bound (in pixel units of the uploaded camera) of everything a camera ray can hit */
     double hit_u0 = 0, hit_u1 = 0, hit_v0 = 0, hit_v1 = 0;
-    bool   classed = false;       /* plastics + specular / rough-conductor materials under one light: the classed compact-record kernel */
-    bool   all_fast = false;      /* every surface material has a plastic block (SpdIndex::plastic): the specialised kernel applies */
+    int    scene_mode = 0;        /* the render kernel the uploaded scene gets (scene_kernel_mode in drt_capi.cu) */
     void  *d_geom32 = nullptr, *d_geom64 = nullptr;
     SpdIndex *d_index = nullptr;
     float *d_pool = nullptr;

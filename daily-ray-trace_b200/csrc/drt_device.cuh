@@ -126,17 +126,12 @@ struct SpdIndex
 {
     int n, nslots, npad, nrows;
     int row[DRT_MAX_MATERIALS][DRT_SPD_COUNT];
-    /* word offset (multiple of 4) of the material's interleaved "plastic block", 0 if it has none: the diffuse and glossy
-     * rows D, G and their products DE, GE with the emission of light 0, laid out so that a half-warp lane fetches all it
-     * needs for one bounce with 16-byte loads that land in f32x2 register pairs.  For wavelength slots (2p, 2p+1) of lane l:
-     *   chunk 2p   = { D[2p], D[2p+1], G[2p], G[2p+1] }      chunk 2p+1 = { DE[2p], DE[2p+1], GE[2p], GE[2p+1] }
-     * and for an odd last slot s the last chunk (index nslots - 1) = { D[s], G[s], DE[s], GE[s] }; chunk c of lane l is the
-     * float4 at index c*16 + l of the block (nslots*64 words in all). */
-    int plastic[DRT_MAX_MATERIALS];
-    /* The ALLFAST kernel carries u = throughput * E (E = emission of the scene's only light) instead of the throughput, so its
-     * blocks hold D and G only: chunk p (a float4 at index p*16 + l) = { D[2p], D[2p+1], G[2p], G[2p+1] }, and for an odd last slot s
-     * the last chunk = { D[s], G[s], 0, 0 }: ceil(nslots / 2) * 64 words.  light_pairs = word offset of E in the same pairing:
-     * float2 { E[2p], E[2p+1] } at index p*16 + l, { E[s], 0 } for an odd last slot. */
+    /* Plastic bounces under a scene's only light (every kernel mode): word offset (multiple of 4) of the material's D, G block, 0 if
+     * it has none -- the diffuse and glossy rows D, G, each times its lobe's multiplicity, laid out so that a half-warp lane fetches a
+     * slot pair with one 16-byte load that lands in f32x2 register pairs.  For lane l, chunk p (a float4 at index p*16 + l) =
+     * { D[2p], D[2p+1], G[2p], G[2p+1] }, and for an odd last slot s the last chunk = { D[s], G[s], 0, 0 }: ceil(nslots / 2) * 64
+     * words.  light_pairs = word offset of the light's emission E in the same pairing: float2 { E[2p], E[2p+1] } at index p*16 + l,
+     * { E[s], 0 } for an odd last slot. */
     int plastic2[DRT_MAX_MATERIALS];
     int light_pairs, pad[3];
     /* Fresnel inputs per wavelength, precomputed in f64 at upload for the two orientations a surface can be met in (0: from the
@@ -171,7 +166,7 @@ struct DeviceStats
  *                         nlights x { eval weights (eval_words), light scale k }      next-event estimation
  *                         eval weights (eval_words)                                   sampled direction, x 1/pdf
  *   per bounce, fast      two-lobe plastic under the scene's only light:
- *                         [0] header: kind(2) | 1<<2 | plastic block float4 index<<4
+ *                         [0] header: kind(2) | 1<<2 | D, G block word offset (SpdIndex::plastic2, a multiple of 4)<<2
  *                         [1] w_diffuse * k  [2] w_glossy * k   (next-event estimation, 0 when the light is hidden)
  *                         [4] w_diffuse / pdf [5] w_glossy / pdf (sampled direction)
  *   bounce_words is a multiple of 4 and at least 8.

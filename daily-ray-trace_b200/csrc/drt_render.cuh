@@ -663,7 +663,7 @@ __device__ __forceinline__ void sample_direction(const GeomT<R> &g, const Hit<R>
 #define KIND_SHADE 1u
 #define KIND_EMIT  2u
 /* bounce header word (record layout: RenderLaunch in drt_device.cuh):
- *   fast (two-lobe plastic, one light):  kind(2) | 1<<2 | plastic block float4 index<<4
+ *   fast (two-lobe plastic, one light):  kind(2) | 1<<2 | D, G block word offset (SpdIndex::plastic2)<<2
  *   general:                             kind(2) | 0<<2 | surface material(5)<<3 | media swapped<<8 | light visibility mask(16)<<16
  * so the hot replay needs two 16-byte record reads per bounce and no material-table lookups. */
 #define HDR_FAST 4u
@@ -742,7 +742,7 @@ __device__ __forceinline__ uint32_t trace_path(const GeomT<R> &g, const SpdIndex
         const int sm = h.surf_mat;
         const int cls = CLASSED ? g.mclass[sm] : DRT_CLASS_PLASTIC;
         const bool plastic = ALLFAST ? (cls == DRT_CLASS_PLASTIC) : (g.bmask[sm] == BMASK_PLASTIC && g.nlobes[sm] == 2);
-        const bool fast = ALLFAST || (plastic && ix.plastic[sm] != 0);
+        const bool fast = ALLFAST || (plastic && ix.plastic2[sm] != 0);
         const int nlights = ALLFAST ? 1 : g.nlights;
         float *recw = in_smem ? rec + L.head_words + 4u * nb : deep + 4u * (nb - L.smem_depth);   /* this bounce's four words in a compact record */
         if(CLASSED && cls == DRT_CLASS_ROUGH) { recw[0] = 0.f; recw[1] = 1.f; }   /* the light may turn out hidden */
@@ -870,7 +870,7 @@ __device__ __forceinline__ uint32_t trace_path(const GeomT<R> &g, const SpdIndex
         else if(fast)
         {
             float4 *r4 = reinterpret_cast<float4 *>(rb);
-            r4[0] = make_float4(__uint_as_float(KIND_SHADE | HDR_FAST | ((uint32_t)ix.plastic[sm] << 2)), wd_n, wg_n, 0.f);
+            r4[0] = make_float4(__uint_as_float(KIND_SHADE | HDR_FAST | ((uint32_t)ix.plastic2[sm] << 2)), wd_n, wg_n, 0.f);
             r4[1] = make_float4(wd_s, wg_s, 0.f, 0.f);
         }
         else
@@ -1314,7 +1314,8 @@ __device__ __forceinline__ void replay_compact(const float *col, const float *de
  * odd last slot.  The hot bounce (two-lobe plastic under the scene's only light) is
  *     radiance   += throughput * (wd_n k * DE + wg_n k * GE)        (NEE: bdsf * emission * k, :322-327; weights are 0 when shadowed)
  *     throughput *= wd_s/pdf * D + wg_s/pdf * G                      (:467-469)
- * with D, G, DE = D*E, GE = G*E fetched from the material's interleaved plastic block by 16-byte loads. */
+ * with D, G from the material's D, G block (16-byte loads) and E from the light's slot pairs (SpdIndex::plastic2, light_pairs);
+ * DE = D*E and GE = G*E are formed here. */
 template <int NS, bool DEEP, typename G>
 __device__ __forceinline__ void replay_path(const float *col, const float *deep, uint32_t nb, const G &g, const SpdIndex &ix, const float *pool, const float *pool_lane,
                                             uint32_t lane16, const RenderLaunch &L, float (&c)[NS])
@@ -1338,20 +1339,24 @@ __device__ __forceinline__ void replay_path(const float *col, const float *deep,
         {
             const float4 s4 = *reinterpret_cast<const float4 *>(pc + 4);
             const float4 *blk = reinterpret_cast<const float4 *>(pool) + (hdr >> 4) + lane16;
+            const float2 *ep = reinterpret_cast<const float2 *>(pool + ix.light_pairs) + lane16;
             const unsigned long long wdn = pk2(a.y, a.y), wgn = pk2(a.z, a.z), wds = pk2(s4.x, s4.x), wgs = pk2(s4.y, s4.y);
 #pragma unroll
             for(int k = 0; k < NP; k += 1)
             {
-                const float4 dg = blk[(2 * k) * DRT_HALF], ee = blk[(2 * k + 1) * DRT_HALF];
-                unsigned long long f = fma2(wgn, pk2(ee.z, ee.w), mul2(wdn, pk2(ee.x, ee.y)));
+                const float4 dg = blk[k * DRT_HALF];
+                const float2 e = ep[k * DRT_HALF];
+                const unsigned long long d2 = pk2(dg.x, dg.y), g2 = pk2(dg.z, dg.w), e2 = pk2(e.x, e.y);
+                unsigned long long f = fma2(wgn, mul2(g2, e2), mul2(wdn, mul2(d2, e2)));
                 dst2[k] = fma2(thr2[k], f, dst2[k]);
-                unsigned long long t = fma2(wgs, pk2(dg.z, dg.w), mul2(wds, pk2(dg.x, dg.y)));
+                unsigned long long t = fma2(wgs, g2, mul2(wds, d2));
                 thr2[k] = mul2(thr2[k], t);
             }
             if(NS & 1)
             {
-                const float4 q = blk[(NS - 1) * DRT_HALF];   /* D, G, DE, GE of the last slot */
-                dst1 = fmaf(thr1, fmaf(a.z, q.w, a.y * q.z), dst1);
+                const float2 q = *reinterpret_cast<const float2 *>(blk + NP * DRT_HALF);   /* D, G of the last slot */
+                const float e = ep[NP * DRT_HALF].x;
+                dst1 = fmaf(thr1, fmaf(a.z, q.y * e, a.y * (q.x * e)), dst1);
                 thr1 *= fmaf(s4.y, q.y, s4.x * q.x);
             }
             continue;
