@@ -700,12 +700,22 @@ extern "C" int drt_cuda_render_kernel_info(drt_cuda_context *ctx, const drt_rend
 static int launch(drt_cuda_context *ctx, const drt_render_params *p, uint32_t x0, uint32_t y0, uint32_t x1, uint32_t y1,
                   FilmPtrs film, float *dump, int accumulate, cudaStream_t stream, float *record_dump = nullptr, uint32_t *path_words_out = nullptr,
                   const drt_film *scatter = nullptr, int scatter_count = 0, int scatter_rank = 0, uint64_t scatter_slice = 0, bool keep_stats = false,
-                  uint64_t band_begin = 0, uint64_t band_end = 0, const drt_adaptive *adaptive = nullptr)
+                  uint64_t band_begin = 0, uint64_t band_end = 0, const drt_adaptive *adaptive = nullptr, int rows_count = 0, int rows_rank = 0)
 {
     if(!ctx->have_scene) return fail(DRT_CUDA_E_STATE, "upload a scene first");
     if(p->width == 0 || p->height == 0 || x1 > p->width || y1 > p->height || x0 >= x1 || y0 >= y1) return fail(DRT_CUDA_E_ARG, "bad image rectangle");
     if(p->sample_end < p->sample_begin) return fail(DRT_CUDA_E_ARG, "bad sample range [%u,%u)", p->sample_begin, p->sample_end);
     CU(cudaSetDevice(ctx->device));
+    /* a row shard (adaptive only) of a rank without rows: no launch (a grid of 0 is an error), and the call's counters read zero */
+    uint32_t shard_rows = 0;
+    if(rows_count && (uint32_t)rows_rank < p->height) shard_rows = (p->height - (uint32_t)rows_rank + (uint32_t)rows_count - 1) / (uint32_t)rows_count;
+    if(rows_count && shard_rows == 0)
+    {
+        ctx->d_stats = ctx->d_stats_ring + (ctx->stats_calls++ % DRT_RING);
+        CU(cudaMemsetAsync(ctx->d_stats, 0, sizeof(DeviceStats), stream));
+        ctx->last_launches = 0;
+        return DRT_CUDA_OK;
+    }
     if(p->sample_end == p->sample_begin)
     {
         /* num_pixel_samples 0: render_image's sample loop does not run (daily_ray_trace.c:710) and the films stay as allocated, all zero */
@@ -763,7 +773,12 @@ static int launch(drt_cuda_context *ctx, const drt_render_params *p, uint32_t x0
             return fail(DRT_CUDA_E_ARG, "a band needs a scattered whole-frame render with at least 32 samples per pixel");
         L.band_chunk = (uint32_t)(band_end - band_begin); L.band_period = (uint32_t)scatter_slice; L.band_base = (uint32_t)band_begin;
     }
-    uint64_t ntasks = band ? (uint64_t)L.band_chunk * scatter_count : (npix + L.pixels_per_task - 1) / L.pixels_per_task;
+    if(rows_count)   /* checked by drt_cuda_render_device_adaptive_rows: an adaptive whole-frame render, no scatter, no band */
+    {
+        L.band_chunk = p->width; L.band_period = (uint32_t)rows_count * p->width; L.band_base = (uint32_t)rows_rank * p->width;
+        L.row_tasks = p->width * shard_rows;
+    }
+    uint64_t ntasks = band ? (uint64_t)L.band_chunk * scatter_count : rows_count ? (uint64_t)L.row_tasks : (npix + L.pixels_per_task - 1) / L.pixels_per_task;
     if(scatter_count > 1)
         L.task_rotate = band ? (uint32_t)(((uint64_t)scatter_rank * L.band_chunk) % ntasks)
                              : (uint32_t)((((uint64_t)scatter_rank * scatter_slice) / L.pixels_per_task) % ntasks);
@@ -862,6 +877,28 @@ extern "C" int drt_cuda_render_device_adaptive(drt_cuda_context *ctx, const drt_
     return launch(ctx, params, 0, 0, params->width, params->height, f, nullptr, accumulate, (cudaStream_t)stream, nullptr, nullptr, nullptr, 0, 0, 0, false, 0, 0, adaptive);
 }
 
+extern "C" int drt_cuda_render_device_adaptive_rows(drt_cuda_context *ctx, const drt_render_params *params, const drt_adaptive *adaptive,
+                                                    const drt_film *film, int accumulate, int count, int rank, void *stream)
+{
+    if(!ctx || !params || !adaptive || !film || !film->sum || !film->filter || !film->mean || !film->m2) return fail(DRT_CUDA_E_ARG, "NULL argument");
+    if(count < 1 || count > DRT_MAX_PEERS || rank < 0 || rank >= count) return fail(DRT_CUDA_E_ARG, "bad row shard: rank %d of %d (1..%d ranks)", rank, count, DRT_MAX_PEERS);
+    int rc = adaptive_args(ctx, params, adaptive);
+    if(rc != DRT_CUDA_OK) return rc;
+    FilmPtrs f = { film->sum, film->filter, film->mean, film->m2 };
+    return launch(ctx, params, 0, 0, params->width, params->height, f, nullptr, accumulate, (cudaStream_t)stream, nullptr, nullptr, nullptr, 0, 0, 0, false, 0, 0,
+                  adaptive, count, rank);
+}
+
+/* the non-blocking streams (and events) of render_host's banded read-back, created on first use */
+static int band_streams(drt_cuda_context *ctx)
+{
+    if(ctx->band_render) return DRT_CUDA_OK;
+    CU(cudaStreamCreateWithFlags(&ctx->band_render, cudaStreamNonBlocking));
+    CU(cudaStreamCreateWithFlags(&ctx->band_copy, cudaStreamNonBlocking));
+    for(int i = 0; i < 16; i += 1) CU(cudaEventCreateWithFlags(&ctx->band_done[i], cudaEventDisableTiming));
+    return DRT_CUDA_OK;
+}
+
 /* render_host and render_host_adaptive (adaptive != NULL) */
 static int render_host(drt_cuda_context *ctx, const drt_render_params *params, const drt_adaptive *adaptive, const drt_film *out)
 {
@@ -880,11 +917,10 @@ static int render_host(drt_cuda_context *ctx, const drt_render_params *params, c
      * after the last render is 1/16 of the film */
     static const int cut[] = { 0, 4, 8, 12, 14, 15, 16 };
     int bands = (paths >= (1ull << 26) && params->height >= 64) ? 6 : 1;
-    if(bands > 1 && !ctx->band_render)
+    if(bands > 1)
     {
-        CU(cudaStreamCreateWithFlags(&ctx->band_render, cudaStreamNonBlocking));
-        CU(cudaStreamCreateWithFlags(&ctx->band_copy, cudaStreamNonBlocking));
-        for(int i = 0; i < 16; i += 1) CU(cudaEventCreateWithFlags(&ctx->band_done[i], cudaEventDisableTiming));
+        rc = band_streams(ctx);
+        if(rc != DRT_CUDA_OK) return rc;
     }
     cudaStream_t sr = bands > 1 ? ctx->band_render : 0, sc = bands > 1 ? ctx->band_copy : 0;
     if(bands > 1) CU(cudaDeviceSynchronize());   /* the band streams do not synchronise with the legacy stream */
@@ -919,6 +955,62 @@ extern "C" int drt_cuda_render_host_adaptive(drt_cuda_context *ctx, const drt_re
     int rc = adaptive_args(ctx, params, adaptive);
     if(rc != DRT_CUDA_OK) return rc;
     return render_host(ctx, params, adaptive, out);
+}
+
+/* Every pixel's samples stay on the device that renders its row, so its stopping rule sees its whole film and nothing is merged:
+ * device g renders rows y = g (mod count) into its own full-frame film and copies them to out on the same stream.  All renders are
+ * queued before any copy. */
+extern "C" int drt_cuda_render_host_multi_adaptive(drt_cuda_context **ctxs, int count, const drt_render_params *params, const drt_adaptive *adaptive,
+                                                   const drt_film *out)
+{
+    if(!ctxs || count < 1 || count > DRT_MAX_PEERS || !params || !adaptive || !out || !out->sum || !out->filter || !out->mean || !out->m2)
+        return fail(DRT_CUDA_E_ARG, "bad argument (1..%d contexts)", DRT_MAX_PEERS);
+    for(int g = 0; g < count; g += 1)
+    {
+        if(!ctxs[g]) return fail(DRT_CUDA_E_ARG, "context %d is NULL", g);
+        int rc = adaptive_args(ctxs[g], params, adaptive);
+        if(rc != DRT_CUDA_OK) return rc;
+        if(ctxs[g]->n != ctxs[0]->n) return fail(DRT_CUDA_E_ARG, "context %d holds another scene", g);
+        for(int h = 0; h < g; h += 1) if(ctxs[h]->device == ctxs[g]->device) return fail(DRT_CUDA_E_ARG, "contexts %d and %d share device %d", h, g, ctxs[g]->device);
+    }
+    const size_t npix = (size_t)params->width * params->height, plane = npix * (size_t)ctxs[0]->n * 4;
+    if(npix == 0) return fail(DRT_CUDA_E_ARG, "bad image rectangle");
+    int rc = DRT_CUDA_OK;
+    for(int g = 0; g < count && rc == DRT_CUDA_OK; g += 1)
+    {
+        drt_cuda_context *ctx = ctxs[g];
+        if((uint32_t)g >= params->height)
+        {
+            /* a surplus device: no rows, no launch; its counters read zero */
+            FilmPtrs none = { nullptr, nullptr, nullptr, nullptr };
+            rc = launch(ctx, params, 0, 0, params->width, params->height, none, nullptr, 0, 0, nullptr, nullptr, nullptr, 0, 0, 0, false, 0, 0, adaptive, count, g);
+            continue;
+        }
+        if(cudaSetDevice(ctx->device) != cudaSuccess) { rc = fail(DRT_CUDA_E_CUDA, "cudaSetDevice(%d)", ctx->device); break; }
+        rc = drt_ensure_buffer(&ctx->d_film, &ctx->film_bytes, 3 * plane + npix * 4);
+        if(rc == DRT_CUDA_OK) rc = band_streams(ctx);
+        /* the non-blocking stream does not wait for work of this context on the legacy stream */
+        if(rc == DRT_CUDA_OK && cudaDeviceSynchronize() != cudaSuccess) rc = fail(DRT_CUDA_E_CUDA, "device %d: %s", ctx->device, cudaGetErrorString(cudaGetLastError()));
+        if(rc != DRT_CUDA_OK) break;
+        float *base = ctx->d_film;
+        const drt_film f = { base, base + 3 * (plane / 4), base + plane / 4, base + 2 * (plane / 4) };
+        rc = drt_cuda_render_device_adaptive_rows(ctx, params, adaptive, &f, 0, count, g, ctx->band_render);
+    }
+    /* The read-backs are queued only once every device renders: a copy into pageable host memory returns when it has finished, so
+     * queued right after its own render it would hold the host, and the renders of the devices after it, until that render ends. */
+    for(int g = 0; g < count && (uint32_t)g < params->height && rc == DRT_CUDA_OK; g += 1)
+    {
+        float *base = ctxs[g]->d_film;
+        const drt_film f = { base, base + 3 * (plane / 4), base + plane / 4, base + 2 * (plane / 4) };
+        rc = drt_cuda_film_read_rows(ctxs[g], &f, params->width, params->height, count, g, out, ctxs[g]->band_render);
+    }
+    for(int g = 0; g < count && (uint32_t)g < params->height; g += 1)
+    {
+        if(!ctxs[g]->band_render || cudaSetDevice(ctxs[g]->device) != cudaSuccess) continue;
+        if(cudaStreamSynchronize(ctxs[g]->band_render) != cudaSuccess && rc == DRT_CUDA_OK)
+            rc = fail(DRT_CUDA_E_CUDA, "device %d: %s", ctxs[g]->device, cudaGetErrorString(cudaGetLastError()));
+    }
+    return rc;
 }
 
 extern "C" int drt_cuda_get_stats(drt_cuda_context *ctx, drt_cuda_stats *out)

@@ -237,4 +237,9 @@ struct RenderLaunch
     float    rel_error;
     uint32_t min_samples;
     uint32_t adaptive;
+    /* Row shard of an adaptive render (drt_cuda_render_device_adaptive_rows; read by render_kernel_adaptive only): the launch covers the
+     * rows y = rank (mod count) of the frame with the band walk above, band_chunk = width, band_period = count * width, band_base =
+     * rank * width, and row_tasks = width * ceil((height - rank) / count) tasks, every one a pixel.  Finished pixels go to their global
+     * positions in `film` (scatter_count = 0).  An adaptive launch without a band covers its rectangle. */
+    uint32_t row_tasks;
 };

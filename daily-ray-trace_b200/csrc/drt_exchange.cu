@@ -157,6 +157,26 @@ extern "C" int drt_cuda_film_read_slice(drt_cuda_context *ctx, const drt_film *s
     return DRT_CUDA_OK;
 }
 
+extern "C" int drt_cuda_film_read_rows(drt_cuda_context *ctx, const drt_film *film_device, uint32_t width, uint32_t height, int count, int rank,
+                                       const drt_film *film_host, void *stream)
+{
+    if(!ctx || !film_device || !film_device->sum || !film_device->filter || !film_device->mean || !film_device->m2 ||
+       !film_host || !film_host->sum || !film_host->filter || !film_host->mean || !film_host->m2) return fail(DRT_CUDA_E_ARG, "NULL argument");
+    if(count < 1 || count > DRT_MAX_PEERS || rank < 0 || rank >= count) return fail(DRT_CUDA_E_ARG, "bad row shard: rank %d of %d (1..%d ranks)", rank, count, DRT_MAX_PEERS);
+    if(!ctx->have_scene) return fail(DRT_CUDA_E_STATE, "upload a scene first");
+    CU(cudaSetDevice(ctx->device));
+    if(width == 0 || (uint32_t)rank >= height) return DRT_CUDA_OK;
+    /* rows rank, rank + count, ...: one strided copy per plane, row pitch count rows in both films */
+    const size_t rows = (height - (uint32_t)rank + (uint32_t)count - 1) / (uint32_t)count, n = (size_t)ctx->n;
+    const size_t row = (size_t)width * n * 4, at = (size_t)rank * width * n, frow = (size_t)width * 4, fat = (size_t)rank * width;
+    cudaStream_t s = (cudaStream_t)stream;
+    CU(cudaMemcpy2DAsync(film_host->sum + at, row * count, film_device->sum + at, row * count, row, rows, cudaMemcpyDeviceToHost, s));
+    CU(cudaMemcpy2DAsync(film_host->mean + at, row * count, film_device->mean + at, row * count, row, rows, cudaMemcpyDeviceToHost, s));
+    CU(cudaMemcpy2DAsync(film_host->m2 + at, row * count, film_device->m2 + at, row * count, row, rows, cudaMemcpyDeviceToHost, s));
+    CU(cudaMemcpy2DAsync(film_host->filter + fat, frow * count, film_device->filter + fat, frow * count, frow, rows, cudaMemcpyDeviceToHost, s));
+    return DRT_CUDA_OK;
+}
+
 extern "C" int drt_cuda_host_alloc(size_t bytes, void **out)
 {
     if(!out || bytes == 0) return fail(DRT_CUDA_E_ARG, "bad argument");

@@ -70,7 +70,9 @@
     const uint32_t rw = L.x1 - L.x0, npix = rw * (L.y1 - L.y0);
     const uint32_t spp = L.sample_end - L.sample_begin;
     const uint32_t n = (uint32_t)ix.n;
-    const uint32_t ntasks = (PAIRED && L.band_chunk) ? L.band_chunk * L.scatter_count : (npix + L.pixels_per_task - 1) / L.pixels_per_task;
+    /* a band of an adaptive launch is a row shard (RenderLaunch::row_tasks): one row per chunk, no scatter */
+    const uint32_t ntasks = (PAIRED && L.band_chunk) ? (ADAPTIVE ? L.row_tasks : L.band_chunk * L.scatter_count)
+                                                     : (npix + L.pixels_per_task - 1) / L.pixels_per_task;
     const bool have_film = L.film.sum != nullptr;
     /* A task is one pixel with all its samples (spp >= 32: `paired`, the film stays in registers across the pixel's batches of
      * 32 paths) or 32/spp whole pixels traced as ONE batch.  Either way phase 2 walks the batch pixel by pixel, both half
@@ -135,7 +137,7 @@
         task += L.task_rotate;
         if(task >= ntasks) task -= ntasks;
         uint32_t p_begin = task * L.pixels_per_task;
-        if(paired && L.band_chunk)   /* a band of a scattered render: the same part of every owner's slice */
+        if(paired && L.band_chunk)   /* a band of a scattered render: the same part of every owner's slice (or an adaptive row shard) */
         {
             p_begin = (p_begin / L.band_chunk) * L.band_period + L.band_base + p_begin % L.band_chunk;
             if(p_begin >= L.width * L.height) continue;

@@ -20,7 +20,8 @@ EXPORTS = ["drt_cuda_last_error", "drt_cuda_device_count", "drt_cuda_create", "d
            "drt_cuda_buffer_ipc_export", "drt_cuda_buffer_ipc_open", "drt_cuda_buffer_ipc_close",
            "drt_cuda_film_merge_slices_local", "drt_cuda_film_read_slice", "drt_cuda_flags_signal", "drt_cuda_flags_wait", "drt_cuda_flags_timeouts",
            "drt_cuda_host_alloc", "drt_cuda_host_free", "drt_cuda_render_host_multi_images", "drt_cuda_render_device_scatter_band", "drt_cuda_plan_scene",
-           "drt_cuda_render_device_adaptive", "drt_cuda_render_host_adaptive"]
+           "drt_cuda_render_device_adaptive", "drt_cuda_render_host_adaptive", "drt_cuda_render_device_adaptive_rows", "drt_cuda_film_read_rows",
+           "drt_cuda_render_host_multi_adaptive"]
 
 
 class Film(C.Structure):
@@ -75,6 +76,10 @@ def lib():
         L.drt_cuda_render_host.argtypes = [C.c_void_p, C.POINTER(RenderParams), C.POINTER(Film)]
         L.drt_cuda_render_device_adaptive.argtypes = [C.c_void_p, C.POINTER(RenderParams), C.POINTER(Adaptive), C.POINTER(Film), C.c_int, C.c_void_p]
         L.drt_cuda_render_host_adaptive.argtypes = [C.c_void_p, C.POINTER(RenderParams), C.POINTER(Adaptive), C.POINTER(Film)]
+        L.drt_cuda_render_device_adaptive_rows.argtypes = [C.c_void_p, C.POINTER(RenderParams), C.POINTER(Adaptive), C.POINTER(Film), C.c_int,
+                                                           C.c_int, C.c_int, C.c_void_p]
+        L.drt_cuda_film_read_rows.argtypes = [C.c_void_p, C.POINTER(Film), C.c_uint32, C.c_uint32, C.c_int, C.c_int, C.POINTER(Film), C.c_void_p]
+        L.drt_cuda_render_host_multi_adaptive.argtypes = [C.POINTER(C.c_void_p), C.c_int, C.POINTER(RenderParams), C.POINTER(Adaptive), C.POINTER(Film)]
         L.drt_cuda_film_merge_slices_local.argtypes = [C.c_void_p, C.POINTER(Film), C.POINTER(Film), C.c_int, C.c_uint64, C.c_uint32, C.c_uint32,
                                                        C.c_uint64, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
         L.drt_cuda_film_read_slice.argtypes = [C.c_void_p, C.POINTER(Film), C.c_uint64, C.c_uint64, C.c_uint64, C.POINTER(Film), C.c_void_p]
@@ -179,6 +184,15 @@ class Context:
     def render_device_adaptive(self, params, rel_error, min_samples, film, accumulate=False, stream=None):
         _check(lib().drt_cuda_render_device_adaptive(self._h, C.byref(params), C.byref(Adaptive(rel_error, min_samples)), C.byref(film),
                                                      int(accumulate), stream))
+
+    def render_device_adaptive_rows(self, params, rel_error, min_samples, film, count, rank, accumulate=False, stream=None):
+        """render_device_adaptive of the rows y = rank (mod count) only, into the full-frame device film `film` (other rows untouched)."""
+        _check(lib().drt_cuda_render_device_adaptive_rows(self._h, C.byref(params), C.byref(Adaptive(rel_error, min_samples)), C.byref(film),
+                                                          int(accumulate), count, rank, stream))
+
+    def film_read_rows(self, film, width, height, count, rank, host_film, stream=None):
+        """Stream-ordered copy of the rows y = rank (mod count) of a full-frame device film into a whole host film (drt_film of host pointers)."""
+        _check(lib().drt_cuda_film_read_rows(self._h, C.byref(film), width, height, count, rank, C.byref(host_film), stream))
 
     def render_host_into(self, params, film):
         _check(lib().drt_cuda_render_host(self._h, C.byref(params), C.byref(film)))
@@ -309,6 +323,23 @@ def render_host_multi(contexts, params):
     film = Film(out["sum"].ctypes.data, out["filter"].ctypes.data, out["mean"].ctypes.data, out["m2"].ctypes.data)
     handles = (C.c_void_p * len(contexts))(*[c._h for c in contexts])
     _check(lib().drt_cuda_render_host_multi(handles, len(contexts), C.byref(params), C.byref(film)))
+    return out
+
+
+def render_host_multi_adaptive(contexts, params, rel_error, min_samples, film=None):
+    """render_host_adaptive over several Context objects on distinct devices of this process, device g rendering the rows y = g (mod G):
+    dict of numpy f32 arrays like Context.render_host_adaptive.  The devices render at once; the read-backs into these pageable arrays run
+    one after another.  `film` (optional): a Film of caller-owned host planes to fill instead (pinned ones let the read-backs overlap);
+    then None is returned."""
+    out = None
+    if film is None:
+        npix, n = params.width * params.height, contexts[0].n or 1
+        out = {"sum": np.empty((npix, n), np.float32), "filter": np.empty(npix, np.float32),
+               "mean": np.empty((npix, n), np.float32), "m2": np.empty((npix, n), np.float32)}
+        film = Film(out["sum"].ctypes.data, out["filter"].ctypes.data, out["mean"].ctypes.data, out["m2"].ctypes.data)
+    handles = (C.c_void_p * len(contexts))(*[c._h for c in contexts])
+    _check(lib().drt_cuda_render_host_multi_adaptive(handles, len(contexts), C.byref(params), C.byref(Adaptive(rel_error, min_samples)),
+                                                      C.byref(film)))
     return out
 
 

@@ -113,8 +113,10 @@ int  drt_cuda_render_host(drt_cuda_context *ctx, const drt_render_params *params
  * instead of tracing) and pixels without variance stop at the first batch end at or past min_samples; pixels with Y = 0 but noise, and
  * pixels whose film holds a NaN, run to the end of the range.  drt_cuda_get_stats reports the paths actually taken.
  * rel_error: finite, > 0; min_samples: 32 ..  sample_end - sample_begin (so the range holds at least 32 samples); else DRT_CUDA_E_ARG.
- * f64 geometry (a diagnostic) has no adaptive kernel: DRT_CUDA_E_UNSUPPORTED.  There is no multi-GPU form: with the samples of a
- * pixel split over devices, no device sees the merged film the rule needs. */
+ * f64 geometry (a diagnostic) has no adaptive kernel: DRT_CUDA_E_UNSUPPORTED.  The multi-GPU form shards by ROWS, not by samples (with
+ * the samples of a pixel split over devices, no device would see the merged film the rule needs): a device renders every sample of the
+ * pixels of its rows, so each pixel's rule sees its whole film, nothing is merged, and the shards together are the one-device film bit
+ * for bit (a pixel's paths and their order within a batch do not depend on the device or warp that takes it). */
 typedef struct
 {
     float    rel_error;
@@ -125,6 +127,24 @@ int  drt_cuda_render_device_adaptive(drt_cuda_context *ctx, const drt_render_par
                                      const drt_film *film_device, int accumulate, void *stream);
 int  drt_cuda_render_host_adaptive(drt_cuda_context *ctx, const drt_render_params *params, const drt_adaptive *adaptive,
                                    const drt_film *film_host);
+
+/* Adaptive sampling of the rows y = rank (mod count) of the frame into a full-frame device film (other rows untouched): pixels are
+ * stored, and with accumulate = 1 loaded, at their global positions.  count: 1 .. 16, rank: 0 .. count - 1, else DRT_CUDA_E_ARG; the other
+ * checks are those of drt_cuda_render_device_adaptive.  A rank without rows (rank >= height) launches nothing, and drt_cuda_get_stats
+ * then reports zeros.  Multi-process callers: rank r of `count` calls this with (count, r), then drt_cuda_film_read_rows. */
+int  drt_cuda_render_device_adaptive_rows(drt_cuda_context *ctx, const drt_render_params *params, const drt_adaptive *adaptive,
+                                          const drt_film *film_device, int accumulate, int count, int rank, void *stream);
+/* Stream-ordered copy of those rows of a full-frame device film into a WHOLE host film (pinned for the copy to run asynchronously): one
+ * cudaMemcpy2DAsync per plane; the host film's other rows are untouched. */
+int  drt_cuda_film_read_rows(drt_cuda_context *ctx, const drt_film *film_device, uint32_t width, uint32_t height,
+                             int count, int rank, const drt_film *film_host, void *stream);
+/* Adaptive sampling on several devices of ONE process: contexts[g] live on distinct devices and hold the same scene; device g renders
+ * rows y = g (mod count) into its library-owned full-frame film and copies them to film_host over its own PCIe link, then the call
+ * waits.  The devices render at once; the copies overlap each other and the slower renders when film_host is pinned
+ * (drt_cuda_host_alloc), and run one after another when it is pageable.  No peer access, no exchange.  With count > height the surplus devices stay idle.  Each context's
+ * drt_cuda_get_stats reports the paths its device took.  count = 1 gives the film of drt_cuda_render_host_adaptive. */
+int  drt_cuda_render_host_multi_adaptive(drt_cuda_context **contexts, int count, const drt_render_params *params,
+                                         const drt_adaptive *adaptive, const drt_film *film_host);
 
 /* render_host on several devices of ONE process (what `drt_raytrace --gpus G` calls): contexts[g] live on distinct devices and hold
  * the same scene; the samples [sample_begin, sample_end) are split evenly over them.  With peer access every device renders its share
