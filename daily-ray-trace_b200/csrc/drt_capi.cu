@@ -9,7 +9,6 @@
 #include <math.h>
 #include <stdarg.h>
 #include <stdio.h>
-#include <stdlib.h>
 #include <string.h>
 #include <vector>
 #include "drt_context.cuh"
@@ -238,7 +237,6 @@ static int scene_kernel_mode(const drt_scene *scene)
         if(cls != DRT_CLASS_PLASTIC) all_fast = false;
         if(cls == DRT_CLASS_GENERAL) classed = false;
     }
-    if(getenv("DRT_NO_CLASSED")) classed = all_fast;   /* A/B switch: mixed scenes on the general kernel */
     return all_fast ? 1 : classed ? 2 : 0;
 }
 
@@ -651,11 +649,12 @@ static void record_layout(const drt_cuda_context *ctx, uint32_t max_depth, uint3
 /* Path records live in shared memory.  A record holds as many bounces as fit with the kernel's full number of warps and CTAs per SM
  * (smem_depth); deeper bounces overflow to global memory, so neither max_cast_depth nor the number of lights limits a render
  * (cast_ray loops `depth < max_depth` without a bound, daily_ray_trace.c:446).  whole = true (record dumps): the whole record must
- * sit in shared memory, with fewer warps per CTA if need be. */
+ * sit in shared memory, with fewer warps per CTA if need be.  Fills in L's pool size and record layout (path_words and the rest). */
 static bool launch_shape(const drt_cuda_context *ctx, uint32_t max_depth, bool whole, RenderLaunch &L, int *warps_out, int *ctas_out, size_t *smem_out)
 {
-    const int mode = kernel_mode(ctx);
-    const int full_warps = drt_render_cta_warps(ctx->f64_geometry, mode), want_ctas = drt_render_min_ctas(ctx->f64_geometry, mode);
+    const RenderShape &shape = DRT_RENDER_SHAPE[kernel_mode(ctx)];
+    const int full_warps = shape.warps, want_ctas = shape.min_ctas;
+    L.pool_words = ctx->pool_words;
     auto bytes = [&](uint32_t depth, int warps) { record_layout(ctx, max_depth, depth, L); return drt_render_smem_bytes(L, ctx->f64_geometry, warps, ctx->nslots); };
     int warps = full_warps;
     uint32_t depth = max_depth;
@@ -685,7 +684,6 @@ extern "C" int drt_cuda_render_kernel_info(drt_cuda_context *ctx, const drt_rend
     if(!ctx->have_scene) return fail(DRT_CUDA_E_STATE, "upload a scene first");
     RenderLaunch L;
     memset(&L, 0, sizeof(L));
-    L.pool_words = ctx->pool_words;
     int warps = 0, ctas = 0;
     size_t smem = 0;
     if(!launch_shape(ctx, max_depth, false, L, &warps, &ctas, &smem)) return fail(DRT_CUDA_E_UNSUPPORTED, "one bounce record of this scene does not fit in shared memory");
@@ -697,8 +695,16 @@ extern "C" int drt_cuda_render_kernel_info(drt_cuda_context *ctx, const drt_rend
     return DRT_CUDA_OK;
 }
 
+/* starts the work counters of a public call: the next block of the ring, zeroed on `stream` (drt_cuda_get_stats reads the latest) */
+static int begin_call(drt_cuda_context *ctx, cudaStream_t stream)
+{
+    ctx->d_stats = ctx->d_stats_ring + (ctx->stats_calls++ % DRT_RING);
+    CU(cudaMemsetAsync(ctx->d_stats, 0, sizeof(DeviceStats), stream));
+    return DRT_CUDA_OK;
+}
+
 static int launch(drt_cuda_context *ctx, const drt_render_params *p, uint32_t x0, uint32_t y0, uint32_t x1, uint32_t y1,
-                  FilmPtrs film, float *dump, int accumulate, cudaStream_t stream, float *record_dump = nullptr, uint32_t *path_words_out = nullptr,
+                  FilmPtrs film, float *dump, int accumulate, cudaStream_t stream, float *record_dump = nullptr,
                   const drt_film *scatter = nullptr, int scatter_count = 0, int scatter_rank = 0, uint64_t scatter_slice = 0, bool keep_stats = false,
                   uint64_t band_begin = 0, uint64_t band_end = 0, const drt_adaptive *adaptive = nullptr, int rows_count = 0, int rows_rank = 0)
 {
@@ -711,20 +717,16 @@ static int launch(drt_cuda_context *ctx, const drt_render_params *p, uint32_t x0
     if(rows_count && (uint32_t)rows_rank < p->height) shard_rows = (p->height - (uint32_t)rows_rank + (uint32_t)rows_count - 1) / (uint32_t)rows_count;
     if(rows_count && shard_rows == 0)
     {
-        ctx->d_stats = ctx->d_stats_ring + (ctx->stats_calls++ % DRT_RING);
-        CU(cudaMemsetAsync(ctx->d_stats, 0, sizeof(DeviceStats), stream));
+        int rc = begin_call(ctx, stream);
+        if(rc != DRT_CUDA_OK) return rc;
         ctx->last_launches = 0;
         return DRT_CUDA_OK;
     }
     if(p->sample_end == p->sample_begin)
     {
         /* num_pixel_samples 0: render_image's sample loop does not run (daily_ray_trace.c:710) and the films stay as allocated, all zero */
-        if(path_words_out) *path_words_out = 0;
-        if(!keep_stats)
-        {
-            ctx->d_stats = ctx->d_stats_ring + (ctx->stats_calls++ % DRT_RING);
-            CU(cudaMemsetAsync(ctx->d_stats, 0, sizeof(DeviceStats), stream));
-        }
+        int rc = keep_stats ? DRT_CUDA_OK : begin_call(ctx, stream);
+        if(rc != DRT_CUDA_OK) return rc;
         ctx->last_launches = 0;
         if(film.sum && !accumulate && scatter_count == 0)
         {
@@ -739,14 +741,14 @@ static int launch(drt_cuda_context *ctx, const drt_render_params *p, uint32_t x0
     RenderLaunch L;
     memset(&L, 0, sizeof(L));
     L.geom = ctx->f64_geometry ? ctx->d_geom64 : ctx->d_geom32;
-    L.spd_index = ctx->d_index; L.pool = ctx->d_pool; L.pool_words = ctx->pool_words;
+    L.spd_index = ctx->d_index; L.pool = ctx->d_pool;
     L.film = film; L.path_dump = dump; L.record_dump = record_dump;
     L.width = p->width; L.height = p->height; L.x0 = x0; L.y0 = y0; L.x1 = x1; L.y1 = y1;
     L.sample_begin = p->sample_begin; L.sample_end = p->sample_end; L.max_depth = p->max_depth;
     L.pixel_scheme = p->pixel_scheme; L.seed = p->seed; L.accumulate = accumulate; L.nlights = ctx->nlights;
     uint32_t spp = p->sample_end - p->sample_begin;
     L.pixels_per_task = spp >= 32 ? 1 : 32 / spp;
-    for(int i = 0; i < scatter_count; i += 1) L.scatter[i] = FilmPtrs{ scatter[i].sum, scatter[i].filter, scatter[i].mean, scatter[i].m2 };
+    for(int i = 0; i < scatter_count; i += 1) L.scatter[i] = film_ptrs(scatter[i]);
     L.scatter_count = (uint32_t)scatter_count; L.scatter_rank = (uint32_t)scatter_rank; L.scatter_slice = (uint32_t)scatter_slice;
     uint32_t rect[4];
     /* max_cast_depth 0 casts no ray at all (cast_ray's loop, daily_ray_trace.c:446): nothing to cull, and the culled pixels' "one closest-hit ray" must not be counted */
@@ -758,13 +760,12 @@ static int launch(drt_cuda_context *ctx, const drt_render_params *p, uint32_t x0
         L.luminance_w = reinterpret_cast<const float *>(static_cast<const unsigned char *>(ctx->d_rgb_tables) + drt_rgb_tables_yw_offset());
     }
     /* record dumps (diagnostics) want the whole record in shared memory; renders keep full occupancy and let deep bounces overflow */
-    const bool whole = record_dump != nullptr || (path_words_out != nullptr && !dump && !film.sum);
+    const bool whole = record_dump != nullptr;
     int warps, ctas_per_sm;
     size_t smem;
     if(!launch_shape(ctx, p->max_depth, whole, L, &warps, &ctas_per_sm, &smem))
         return fail(DRT_CUDA_E_UNSUPPORTED, "%s: max_cast_depth %u with %d lights needs %zu bytes of shared memory per warp (limit %zu)",
                     whole ? "record dump" : "render", p->max_depth, ctx->nlights, smem, ctx->smem_optin);
-    if(path_words_out) { *path_words_out = L.path_words; if(!record_dump && !dump && !film.sum) return DRT_CUDA_OK; }
     uint64_t npix = (uint64_t)(x1 - x0) * (y1 - y0);
     const bool band = band_end > band_begin;
     if(band)
@@ -794,11 +795,8 @@ static int launch(drt_cuda_context *ctx, const drt_render_params *p, uint32_t x0
         if(rc != DRT_CUDA_OK) return rc;
         L.deep = ctx->d_deep;
     }
-    if(!keep_stats)
-    {
-        ctx->d_stats = ctx->d_stats_ring + (ctx->stats_calls++ % DRT_RING);
-        CU(cudaMemsetAsync(ctx->d_stats, 0, sizeof(DeviceStats), stream));
-    }
+    int rc = keep_stats ? DRT_CUDA_OK : begin_call(ctx, stream);
+    if(rc != DRT_CUDA_OK) return rc;
     L.stats = ctx->d_stats;
     L.task_counter = ctx->d_counter_ring + (ctx->counter_launches++ % DRT_RING);
     CU(cudaMemsetAsync(L.task_counter, 0, sizeof(unsigned int), stream));
@@ -811,9 +809,8 @@ static int launch(drt_cuda_context *ctx, const drt_render_params *p, uint32_t x0
 
 extern "C" int drt_cuda_render_device(drt_cuda_context *ctx, const drt_render_params *params, const drt_film *film, int accumulate, void *stream)
 {
-    if(!ctx || !params || !film || !film->sum || !film->filter || !film->mean || !film->m2) return fail(DRT_CUDA_E_ARG, "NULL argument");
-    FilmPtrs f = { film->sum, film->filter, film->mean, film->m2 };
-    return launch(ctx, params, 0, 0, params->width, params->height, f, nullptr, accumulate, (cudaStream_t)stream);
+    if(!ctx || !params || !film_complete(film)) return fail(DRT_CUDA_E_ARG, "NULL argument");
+    return launch(ctx, params, 0, 0, params->width, params->height, film_ptrs(*film), nullptr, accumulate, (cudaStream_t)stream);
 }
 
 extern "C" int drt_cuda_render_device_scatter(drt_cuda_context *ctx, const drt_render_params *params, const drt_film *staging, int count, int rank,
@@ -823,9 +820,8 @@ extern "C" int drt_cuda_render_device_scatter(drt_cuda_context *ctx, const drt_r
     uint64_t npix = (uint64_t)params->width * params->height;
     if(slice_pixels == 0 || slice_pixels * (uint64_t)count < npix || slice_pixels > 0xffffffffull) return fail(DRT_CUDA_E_ARG, "slices of %llu pixels do not cover the image", (unsigned long long)slice_pixels);
     for(int i = 0; i < count; i += 1)
-        if(!staging[i].sum || !staging[i].filter || !staging[i].mean || !staging[i].m2) return fail(DRT_CUDA_E_ARG, "NULL staging film %d", i);
-    FilmPtrs f = { staging[0].sum, staging[0].filter, staging[0].mean, staging[0].m2 };
-    return launch(ctx, params, 0, 0, params->width, params->height, f, nullptr, 0, (cudaStream_t)stream, nullptr, nullptr, staging, count, rank, slice_pixels);
+        if(!film_complete(&staging[i])) return fail(DRT_CUDA_E_ARG, "NULL staging film %d", i);
+    return launch(ctx, params, 0, 0, params->width, params->height, film_ptrs(staging[0]), nullptr, 0, (cudaStream_t)stream, nullptr, staging, count, rank, slice_pixels);
 }
 
 extern "C" int drt_cuda_render_device_scatter_band(drt_cuda_context *ctx, const drt_render_params *params, const drt_film *staging, int count, int rank,
@@ -836,9 +832,8 @@ extern "C" int drt_cuda_render_device_scatter_band(drt_cuda_context *ctx, const 
     if(slice_pixels == 0 || slice_pixels * (uint64_t)count < npix || slice_pixels > 0xffffffffull) return fail(DRT_CUDA_E_ARG, "slices of %llu pixels do not cover the image", (unsigned long long)slice_pixels);
     if(band_begin >= band_end || band_end > slice_pixels) return fail(DRT_CUDA_E_ARG, "bad band [%llu, %llu) of a slice of %llu pixels", (unsigned long long)band_begin, (unsigned long long)band_end, (unsigned long long)slice_pixels);
     for(int i = 0; i < count; i += 1)
-        if(!staging[i].sum || !staging[i].filter || !staging[i].mean || !staging[i].m2) return fail(DRT_CUDA_E_ARG, "NULL staging film %d", i);
-    FilmPtrs f = { staging[0].sum, staging[0].filter, staging[0].mean, staging[0].m2 };
-    return launch(ctx, params, 0, 0, params->width, params->height, f, nullptr, 0, (cudaStream_t)stream, nullptr, nullptr, staging, count, rank, slice_pixels,
+        if(!film_complete(&staging[i])) return fail(DRT_CUDA_E_ARG, "NULL staging film %d", i);
+    return launch(ctx, params, 0, 0, params->width, params->height, film_ptrs(staging[0]), nullptr, 0, (cudaStream_t)stream, nullptr, staging, count, rank, slice_pixels,
                   keep_stats != 0, band_begin, band_end);
 }
 
@@ -848,6 +843,14 @@ int drt_ensure_buffer(float **buf, size_t *have, size_t need)
     cudaFree(*buf); *buf = nullptr; *have = 0;
     CU(cudaMalloc(buf, need));
     *have = need;
+    return DRT_CUDA_OK;
+}
+
+int drt_library_film(const drt_cuda_context *ctx, float **buf, size_t *have, size_t npix, drt_film *out)
+{
+    int rc = drt_ensure_buffer(buf, have, (3 * npix * (size_t)ctx->n + npix) * 4);
+    if(rc != DRT_CUDA_OK) return rc;
+    *out = film_planes(*buf, npix, ctx->n);
     return DRT_CUDA_OK;
 }
 
@@ -870,22 +873,20 @@ static int adaptive_args(const drt_cuda_context *ctx, const drt_render_params *p
 extern "C" int drt_cuda_render_device_adaptive(drt_cuda_context *ctx, const drt_render_params *params, const drt_adaptive *adaptive,
                                                const drt_film *film, int accumulate, void *stream)
 {
-    if(!ctx || !params || !adaptive || !film || !film->sum || !film->filter || !film->mean || !film->m2) return fail(DRT_CUDA_E_ARG, "NULL argument");
+    if(!ctx || !params || !adaptive || !film_complete(film)) return fail(DRT_CUDA_E_ARG, "NULL argument");
     int rc = adaptive_args(ctx, params, adaptive);
     if(rc != DRT_CUDA_OK) return rc;
-    FilmPtrs f = { film->sum, film->filter, film->mean, film->m2 };
-    return launch(ctx, params, 0, 0, params->width, params->height, f, nullptr, accumulate, (cudaStream_t)stream, nullptr, nullptr, nullptr, 0, 0, 0, false, 0, 0, adaptive);
+    return launch(ctx, params, 0, 0, params->width, params->height, film_ptrs(*film), nullptr, accumulate, (cudaStream_t)stream, nullptr, nullptr, 0, 0, 0, false, 0, 0, adaptive);
 }
 
 extern "C" int drt_cuda_render_device_adaptive_rows(drt_cuda_context *ctx, const drt_render_params *params, const drt_adaptive *adaptive,
                                                     const drt_film *film, int accumulate, int count, int rank, void *stream)
 {
-    if(!ctx || !params || !adaptive || !film || !film->sum || !film->filter || !film->mean || !film->m2) return fail(DRT_CUDA_E_ARG, "NULL argument");
+    if(!ctx || !params || !adaptive || !film_complete(film)) return fail(DRT_CUDA_E_ARG, "NULL argument");
     if(count < 1 || count > DRT_MAX_PEERS || rank < 0 || rank >= count) return fail(DRT_CUDA_E_ARG, "bad row shard: rank %d of %d (1..%d ranks)", rank, count, DRT_MAX_PEERS);
     int rc = adaptive_args(ctx, params, adaptive);
     if(rc != DRT_CUDA_OK) return rc;
-    FilmPtrs f = { film->sum, film->filter, film->mean, film->m2 };
-    return launch(ctx, params, 0, 0, params->width, params->height, f, nullptr, accumulate, (cudaStream_t)stream, nullptr, nullptr, nullptr, 0, 0, 0, false, 0, 0,
+    return launch(ctx, params, 0, 0, params->width, params->height, film_ptrs(*film), nullptr, accumulate, (cudaStream_t)stream, nullptr, nullptr, 0, 0, 0, false, 0, 0,
                   adaptive, count, rank);
 }
 
@@ -902,14 +903,13 @@ static int band_streams(drt_cuda_context *ctx)
 /* render_host and render_host_adaptive (adaptive != NULL) */
 static int render_host(drt_cuda_context *ctx, const drt_render_params *params, const drt_adaptive *adaptive, const drt_film *out)
 {
-    if(!ctx || !params || !out || !out->sum || !out->filter || !out->mean || !out->m2) return fail(DRT_CUDA_E_ARG, "NULL argument");
+    if(!ctx || !params || !film_complete(out)) return fail(DRT_CUDA_E_ARG, "NULL argument");
     if(!ctx->have_scene) return fail(DRT_CUDA_E_STATE, "upload a scene first");
     CU(cudaSetDevice(ctx->device));
-    size_t npix = (size_t)params->width * params->height, plane = npix * (size_t)ctx->n * 4, fplane = npix * 4;
-    int rc = drt_ensure_buffer(&ctx->d_film, &ctx->film_bytes, 3 * plane + fplane);
+    size_t npix = (size_t)params->width * params->height;
+    drt_film f;
+    int rc = drt_library_film(ctx, &ctx->d_film, &ctx->film_bytes, npix, &f);
     if(rc != DRT_CUDA_OK) return rc;
-    float *base = ctx->d_film;
-    FilmPtrs f = { base, base + 3 * (plane / 4), base + plane / 4, base + 2 * (plane / 4) };
     /* Large frames are rendered in row bands so that the read-back of a finished band (PCIe) runs under the render of the
      * next one: with pinned host buffers only the last (small) band's copy is exposed.  Rows are contiguous in every plane. */
     const uint64_t paths = (uint64_t)npix * (params->sample_end - params->sample_begin);
@@ -929,7 +929,7 @@ static int render_host(drt_cuda_context *ctx, const drt_render_params *params, c
     {
         const uint32_t y0 = bands > 1 ? (uint32_t)((uint64_t)params->height * cut[b] / 16) : 0u;
         const uint32_t y1 = bands > 1 ? (uint32_t)((uint64_t)params->height * cut[b + 1] / 16) : params->height;
-        rc = launch(ctx, params, 0, y0, params->width, y1, f, nullptr, 0, sr, nullptr, nullptr, nullptr, 0, 0, 0, b > 0, 0, 0, adaptive);
+        rc = launch(ctx, params, 0, y0, params->width, y1, film_ptrs(f), nullptr, 0, sr, nullptr, nullptr, 0, 0, 0, b > 0, 0, 0, adaptive);
         if(rc != DRT_CUDA_OK) return rc;
         if(bands > 1) { CU(cudaEventRecord(ctx->band_done[b], sr)); CU(cudaStreamWaitEvent(sc, ctx->band_done[b], 0)); }
         const size_t at = (size_t)y0 * w * n, cnt = (size_t)(y1 - y0) * w * n * 4;
@@ -963,7 +963,7 @@ extern "C" int drt_cuda_render_host_adaptive(drt_cuda_context *ctx, const drt_re
 extern "C" int drt_cuda_render_host_multi_adaptive(drt_cuda_context **ctxs, int count, const drt_render_params *params, const drt_adaptive *adaptive,
                                                    const drt_film *out)
 {
-    if(!ctxs || count < 1 || count > DRT_MAX_PEERS || !params || !adaptive || !out || !out->sum || !out->filter || !out->mean || !out->m2)
+    if(!ctxs || count < 1 || count > DRT_MAX_PEERS || !params || !adaptive || !film_complete(out))
         return fail(DRT_CUDA_E_ARG, "bad argument (1..%d contexts)", DRT_MAX_PEERS);
     for(int g = 0; g < count; g += 1)
     {
@@ -973,37 +973,31 @@ extern "C" int drt_cuda_render_host_multi_adaptive(drt_cuda_context **ctxs, int 
         if(ctxs[g]->n != ctxs[0]->n) return fail(DRT_CUDA_E_ARG, "context %d holds another scene", g);
         for(int h = 0; h < g; h += 1) if(ctxs[h]->device == ctxs[g]->device) return fail(DRT_CUDA_E_ARG, "contexts %d and %d share device %d", h, g, ctxs[g]->device);
     }
-    const size_t npix = (size_t)params->width * params->height, plane = npix * (size_t)ctxs[0]->n * 4;
+    const size_t npix = (size_t)params->width * params->height;
     if(npix == 0) return fail(DRT_CUDA_E_ARG, "bad image rectangle");
     int rc = DRT_CUDA_OK;
+    drt_film films[DRT_MAX_PEERS];   /* device g's full-frame film */
     for(int g = 0; g < count && rc == DRT_CUDA_OK; g += 1)
     {
         drt_cuda_context *ctx = ctxs[g];
         if((uint32_t)g >= params->height)
         {
             /* a surplus device: no rows, no launch; its counters read zero */
-            FilmPtrs none = { nullptr, nullptr, nullptr, nullptr };
-            rc = launch(ctx, params, 0, 0, params->width, params->height, none, nullptr, 0, 0, nullptr, nullptr, nullptr, 0, 0, 0, false, 0, 0, adaptive, count, g);
+            rc = launch(ctx, params, 0, 0, params->width, params->height, FilmPtrs{}, nullptr, 0, 0, nullptr, nullptr, 0, 0, 0, false, 0, 0, adaptive, count, g);
             continue;
         }
         if(cudaSetDevice(ctx->device) != cudaSuccess) { rc = fail(DRT_CUDA_E_CUDA, "cudaSetDevice(%d)", ctx->device); break; }
-        rc = drt_ensure_buffer(&ctx->d_film, &ctx->film_bytes, 3 * plane + npix * 4);
+        rc = drt_library_film(ctx, &ctx->d_film, &ctx->film_bytes, npix, &films[g]);
         if(rc == DRT_CUDA_OK) rc = band_streams(ctx);
         /* the non-blocking stream does not wait for work of this context on the legacy stream */
         if(rc == DRT_CUDA_OK && cudaDeviceSynchronize() != cudaSuccess) rc = fail(DRT_CUDA_E_CUDA, "device %d: %s", ctx->device, cudaGetErrorString(cudaGetLastError()));
         if(rc != DRT_CUDA_OK) break;
-        float *base = ctx->d_film;
-        const drt_film f = { base, base + 3 * (plane / 4), base + plane / 4, base + 2 * (plane / 4) };
-        rc = drt_cuda_render_device_adaptive_rows(ctx, params, adaptive, &f, 0, count, g, ctx->band_render);
+        rc = drt_cuda_render_device_adaptive_rows(ctx, params, adaptive, &films[g], 0, count, g, ctx->band_render);
     }
     /* The read-backs are queued only once every device renders: a copy into pageable host memory returns when it has finished, so
      * queued right after its own render it would hold the host, and the renders of the devices after it, until that render ends. */
     for(int g = 0; g < count && (uint32_t)g < params->height && rc == DRT_CUDA_OK; g += 1)
-    {
-        float *base = ctxs[g]->d_film;
-        const drt_film f = { base, base + 3 * (plane / 4), base + plane / 4, base + 2 * (plane / 4) };
-        rc = drt_cuda_film_read_rows(ctxs[g], &f, params->width, params->height, count, g, out, ctxs[g]->band_render);
-    }
+        rc = drt_cuda_film_read_rows(ctxs[g], &films[g], params->width, params->height, count, g, out, ctxs[g]->band_render);
     for(int g = 0; g < count && (uint32_t)g < params->height; g += 1)
     {
         if(!ctxs[g]->band_render || cudaSetDevice(ctxs[g]->device) != cudaSuccess) continue;
@@ -1054,8 +1048,7 @@ extern "C" int drt_cuda_sample_paths(drt_cuda_context *ctx, const drt_render_par
     size_t bytes = (size_t)(x1 - x0) * (y1 - y0) * (params->sample_end - params->sample_begin) * (size_t)ctx->n * 4;
     int rc = drt_ensure_buffer(&ctx->d_dump, &ctx->dump_bytes, bytes);
     if(rc != DRT_CUDA_OK) return rc;
-    FilmPtrs none = { nullptr, nullptr, nullptr, nullptr };
-    rc = launch(ctx, params, x0, y0, x1, y1, none, ctx->d_dump, 0, 0);
+    rc = launch(ctx, params, x0, y0, x1, y1, FilmPtrs{}, ctx->d_dump, 0, 0);
     if(rc != DRT_CUDA_OK) return rc;
     CU(cudaMemcpy(out_host, ctx->d_dump, bytes, cudaMemcpyDeviceToHost));
     return DRT_CUDA_OK;
@@ -1068,14 +1061,21 @@ extern "C" int drt_cuda_debug_records(drt_cuda_context *ctx, const drt_render_pa
     if(!ctx->have_scene) return fail(DRT_CUDA_E_STATE, "upload a scene first");
     if(x1 <= x0 || y1 <= y0 || params->sample_end <= params->sample_begin) return fail(DRT_CUDA_E_ARG, "empty rectangle or sample range");
     CU(cudaSetDevice(ctx->device));
-    FilmPtrs none = { nullptr, nullptr, nullptr, nullptr };
-    int rc = launch(ctx, params, x0, y0, x1, y1, none, nullptr, 0, 0, nullptr, words_per_path);   /* size query only */
-    if(rc != DRT_CUDA_OK || !out_host) return rc;
+    if(x1 > params->width || y1 > params->height) return fail(DRT_CUDA_E_ARG, "bad image rectangle");
+    RenderLaunch L;
+    memset(&L, 0, sizeof(L));
+    int warps, ctas;
+    size_t smem;
+    if(!launch_shape(ctx, params->max_depth, /*whole=*/true, L, &warps, &ctas, &smem))
+        return fail(DRT_CUDA_E_UNSUPPORTED, "record dump: max_cast_depth %u with %d lights needs %zu bytes of shared memory per warp (limit %zu)",
+                    params->max_depth, ctx->nlights, smem, ctx->smem_optin);
+    *words_per_path = L.path_words;
+    if(!out_host) return DRT_CUDA_OK;
     size_t words = (size_t)(x1 - x0) * (y1 - y0) * (params->sample_end - params->sample_begin) * (size_t)*words_per_path;
     if(words > out_capacity_words) return fail(DRT_CUDA_E_ARG, "record buffer too small: need %zu words", words);
-    rc = drt_ensure_buffer(&ctx->d_dump, &ctx->dump_bytes, words * 4);
+    int rc = drt_ensure_buffer(&ctx->d_dump, &ctx->dump_bytes, words * 4);
     if(rc != DRT_CUDA_OK) return rc;
-    rc = launch(ctx, params, x0, y0, x1, y1, none, nullptr, 0, 0, ctx->d_dump, nullptr);
+    rc = launch(ctx, params, x0, y0, x1, y1, FilmPtrs{}, nullptr, 0, 0, ctx->d_dump);
     if(rc != DRT_CUDA_OK) return rc;
     CU(cudaMemcpy(out_host, ctx->d_dump, words * 4, cudaMemcpyDeviceToHost));
     return DRT_CUDA_OK;
@@ -1105,8 +1105,7 @@ extern "C" int drt_cuda_film_merge(drt_cuda_context *ctx, const drt_film *dst, c
     if(!ctx || !dst || !src) return fail(DRT_CUDA_E_ARG, "NULL argument");
     if(!ctx->have_scene) return fail(DRT_CUDA_E_STATE, "upload a scene first");
     CU(cudaSetDevice(ctx->device));
-    FilmPtrs d = { dst->sum, dst->filter, dst->mean, dst->m2 }, s = { src->sum, src->filter, src->mean, src->m2 };
-    drt_launch_film_merge(d, s, (uint32_t)ctx->n, (size_t)width * height, ctx->num_sms * 8, (cudaStream_t)stream);
+    drt_launch_film_merge(film_ptrs(*dst), film_ptrs(*src), (uint32_t)ctx->n, (size_t)width * height, ctx->num_sms * 8, (cudaStream_t)stream);
     CU(cudaGetLastError());
     ctx->launches += 2;
     return DRT_CUDA_OK;
@@ -1239,11 +1238,10 @@ extern "C" int drt_cuda_film_merge_many(drt_cuda_context *ctx, const drt_film *d
     if((bgra_sum || bgra_mean || bgra_var) && !(bgra_sum && bgra_mean && bgra_var)) return fail(DRT_CUDA_E_ARG, "give all three image buffers or none");
     CU(cudaSetDevice(ctx->device));
     FilmPtrs films[16];
-    for(int i = 0; i < count; i += 1) films[i] = FilmPtrs{ srcs[i].sum, srcs[i].filter, srcs[i].mean, srcs[i].m2 };
-    FilmPtrs d = { dst->sum, dst->filter, dst->mean, dst->m2 };
+    for(int i = 0; i < count; i += 1) films[i] = film_ptrs(srcs[i]);
     if(pixel_end > pixel_begin)
     {
-        drt_launch_film_gather_merge(ctx->d_rgb_tables, count, films, d, (uint32_t)pixel_begin, (uint32_t)pixel_end, 0u, 0u, bgra_sum, bgra_mean, bgra_var,
+        drt_launch_film_gather_merge(ctx->d_rgb_tables, count, films, film_ptrs(*dst), (uint32_t)pixel_begin, (uint32_t)pixel_end, 0u, 0u, bgra_sum, bgra_mean, bgra_var,
                                      ctx->num_sms * 8, (cudaStream_t)stream);
         CU(cudaGetLastError());
         ctx->launches += 1;
@@ -1275,11 +1273,10 @@ extern "C" int drt_cuda_film_merge_slices(drt_cuda_context *ctx, const drt_film 
          * memory) as four contiguous copies: the copy engines move large blocks over NVLink about twice as fast as the
          * kernel's 4-byte-per-lane peer stores did (measured: 763 MB into the root in 2.2 ms from kernel stores) */
         const size_t spx = (size_t)(pixel_end - pixel_begin), plane = spx * n * 4;
-        int rc = drt_ensure_buffer(&ctx->d_slice, &ctx->slice_bytes, 3 * plane + spx * 4);
+        drt_film d;
+        int rc = drt_library_film(ctx, &ctx->d_slice, &ctx->slice_bytes, spx, &d);
         if(rc != DRT_CUDA_OK) return rc;
-        float *base = ctx->d_slice;
-        FilmPtrs d = { base, base + 3 * (plane / 4), base + plane / 4, base + 2 * (plane / 4) };
-        drt_launch_film_gather_merge(ctx->d_rgb_tables, count, films, d, (uint32_t)pixel_begin, (uint32_t)pixel_end, (uint32_t)slice_begin,
+        drt_launch_film_gather_merge(ctx->d_rgb_tables, count, films, film_ptrs(d), (uint32_t)pixel_begin, (uint32_t)pixel_end, (uint32_t)slice_begin,
                                      (uint32_t)pixel_begin, bgra_sum, bgra_mean, bgra_var, ctx->num_sms * 8, (cudaStream_t)stream);
         CU(cudaGetLastError());
         const size_t at = (size_t)pixel_begin * n;

@@ -11,8 +11,6 @@
 #include "drt_device.cuh"
 
 cudaError_t drt_launch_render(const RenderLaunch &L, bool f64_geometry, int mode, int nslots, int grid, int warps, size_t smem, cudaStream_t stream);
-int         drt_render_cta_warps(bool f64_geometry, int mode);
-int         drt_render_min_ctas(bool f64_geometry, int mode);
 size_t      drt_render_smem_bytes(const RenderLaunch &L, bool f64_geometry, int warps, int nslots);
 void        drt_launch_film_to_rgb(const void *tables, const float *plane, const float *filter, int normalise_by_max, uint32_t npix,
                                    float *rgb, uint32_t *bgra, int grid, cudaStream_t stream);
@@ -76,3 +74,14 @@ struct drt_cuda_context
 
 void drt_exchange_release(drt_cuda_context *ctx);   /* frees what drt_exchange.cu hung on the context */
 int drt_ensure_buffer(float **buf, size_t *have, size_t need);
+/* The library's layout of a device film of npix pixels and n wavelengths at base: the sum, mean, m2 and filter planes one after the other. */
+static inline drt_film film_planes(float *base, size_t npix, int n)
+{
+    const size_t plane = npix * (size_t)n;
+    return drt_film{ base, base + 3 * plane, base + plane, base + 2 * plane };
+}
+/* film_planes in one of the context's growing buffers (buf, have: d_film, film_bytes or d_slice, slice_bytes), grown first if need be */
+int drt_library_film(const drt_cuda_context *ctx, float **buf, size_t *have, size_t npix, drt_film *out);
+
+static inline bool film_complete(const drt_film *f) { return f && f->sum && f->filter && f->mean && f->m2; }
+static inline FilmPtrs film_ptrs(const drt_film &f) { return FilmPtrs{ f.sum, f.filter, f.mean, f.m2 }; }

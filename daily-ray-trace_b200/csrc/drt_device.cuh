@@ -16,42 +16,29 @@
 #define DRT_MAX_SLOTS 4            /* ceil(DRT_MAX_WAVELENGTHS / 32): full-warp wavelength layout of the film epilogue kernels */
 #define DRT_HALF 16                /* phase 2 of the render kernel: a path is shaded by a HALF warp, lane l16 holds wavelengths l16 + 16k */
 #define DRT_MAX_HALF_SLOTS 8       /* ceil(DRT_MAX_WAVELENGTHS / 16) */
-#ifndef DRT_CTA_WARPS
-#define DRT_CTA_WARPS 8      /* warps per CTA of the general kernel */
-#endif
-#ifndef DRT_FAST_WARPS
-#define DRT_FAST_WARPS 14     /* warps per CTA of the ALLFAST kernel: 2 CTAs x 14 warps x 72 registers per SM (measured: 8 warps 6.7, 12: 9.70, 14: 9.79, 16: 9.65 G paths/s) */
-#endif
-#ifndef DRT_CLASSED_WARPS
-#define DRT_CLASSED_WARPS 16   /* warps per CTA of the classed kernel: 2 CTAs x 16 warps x 64 registers (measured on cornell_plane_light, G paths/s at
-                                * 64 spp: 10 warps 3.96, 12: 4.09, 14: 4.34, 16: 4.53; with the phase gates 16 x 2: 5.04, 32 x 1: 4.97, 28 x 1: 4.79) */
-#endif
-#ifndef DRT_CLASSED_CTAS
-#define DRT_CLASSED_CTAS 2     /* resident CTAs per SM the classed / the general kernel is compiled for */
-#endif
-#ifndef DRT_GENERAL_CTAS
-#define DRT_GENERAL_CTAS 2
-#endif
-#ifndef DRT_LOCKSTEP
-#define DRT_LOCKSTEP 2         /* bit mask of kernel modes whose CTAs run their phases in lockstep (drt_render.cuh): bit 1 = the classed kernel
-                                * (measured +15 %: its hot code is 38 KB against a 32 KB instruction cache); bit 0 = the general kernel
-                                * (measured -26 % on stress_all: its phase-2 times differ too much between warps); bit 2 = the plastic-only kernel */
-#endif
-#ifndef DRT_GATE_PATIENCE_CYCLES
+
+/* Launch shape of each render kernel mode (0 general, 1 plastic-only, 2 classed; kernel_mode in drt_capi.cu): warps per CTA and resident
+ * CTAs per SM, which __launch_bounds__ (DRT_RENDER_BOUNDS) compiles for and launch_shape launches with, and whether the warps of a CTA
+ * run their phases in lockstep (LOCKSTEP in drt_render_body.cuh). */
+struct RenderShape { int warps, min_ctas; bool lockstep; };
+constexpr RenderShape DRT_RENDER_SHAPE[3] = {
+    /* general: 2 CTAs x 8 warps.  Lockstep measured -26 % on stress_all: its phase-2 times differ too much between warps. */
+    { 8, 2, false },
+    /* plastic-only: 2 CTAs x 14 warps x 72 registers per SM (measured: 8 warps 6.7, 12: 9.70, 14: 9.79, 16: 9.65 G paths/s).  Lockstep
+     * measured -9 % (DESIGN.md section 2). */
+    { 14, 2, false },
+    /* classed: 2 CTAs x 16 warps x 64 registers (measured on cornell_plane_light, G paths/s at 64 spp: 10 warps 3.96, 12: 4.09, 14: 4.34,
+     * 16: 4.53; with the phase gates 16 x 2: 5.04, 32 x 1: 4.97, 28 x 1: 4.79).  Lockstep measured +15 %: its hot code is 38 KB against
+     * a 32 KB instruction cache. */
+    { 16, 2, true },
+};
 /* A phase gate gives up after this many SM clock cycles (about 10 ms at 1.97 GHz; a phase takes 50 - 200 us) and switches the
  * CTA's gates off: lockstep is a performance aid, never a dependency.  Multi-GPU renders (scatter_count > 1) start with the gates
  * off: bench.py --scene cornell_plane_light --gpus 2/4/8 did not complete in the round's last GPU session (cause not found before
  * the GPU budget ran out; the same kernel passes every single-device and in-process two-device test), and an untested multi-rank
  * combination is not worth 13 % -- see DESIGN.md section 9. */
 #define DRT_GATE_PATIENCE_CYCLES 20000000ll
-#endif
-#ifndef DRT_GATE_SUSPEND_NS
 #define DRT_GATE_SUSPEND_NS 20000u   /* suspend-time hint of a phase gate's mbarrier.try_wait */
-#endif
-#define DRT_CTA_THREADS (DRT_CTA_WARPS * DRT_WARP)
-#ifndef DRT_MIN_CTAS
-#define DRT_MIN_CTAS 2        /* resident CTAs per SM the render kernels are compiled for (__launch_bounds__) */
-#endif
 
 /* Spectral basis a BSDF evaluation is expressed in (eval_weights in drt_kernels.cu).  A material's lobe list fixes
  * which of the seven can ever be non-zero (bmask); only those weights are stored in a path record, in this order,
@@ -141,6 +128,25 @@ struct SpdIndex
      *   [1] condA = (tr / ir)^2 - (te / ir)^2   [2] condB = 4 (tr / ir)^2 (te / ir)^2          conductor (fresnel_conductor_ab) */
     int fres[DRT_MAX_MATERIALS][2][3];
 };
+
+/* Shared memory of a render CTA, carved in this order: GeomT<R> (GEOM_BYTES), SpdIndex, the spectrum pool, 16 work-counter words, the
+ * warps' path records (PATH_STRIDE words per slot) and their film parking ((3 NS + 2) * 32 words per warp).  Written once and expanded
+ * in two places: the kernel body (drt_render_body.cuh) takes its section pointers from it, SECTION(type, name, byte offset) declaring
+ * each one, and drt_render_smem_bytes sizes a launch by the `off` it leaves behind (SECTION empty).  A macro rather than a function:
+ * the kernels' register allocation depends on the body seeing this arithmetic inline. */
+#define DRT_RENDER_SMEM_CARVE(SECTION, GEOM_BYTES, POOL_WORDS, WARPS, PATH_STRIDE, NS) \
+    size_t off = ((GEOM_BYTES) + 15) & ~size_t(15);                                 \
+    SECTION(SpdIndex, six, off)                                                     \
+    off += (sizeof(SpdIndex) + 15) & ~size_t(15);                                   \
+    SECTION(float, spool, off)                                                      \
+    off += (size_t)(POOL_WORDS) * 4;                                                \
+    SECTION(unsigned long long, s_stats, off)                                       \
+    off += 16 * 8;                                                                  \
+    off = (off + 15) & ~size_t(15);                                                 \
+    SECTION(float, srec, off)                                                       \
+    off += (size_t)(WARPS) * (PATH_STRIDE) * DRT_WARP * 4;                          \
+    SECTION(float, spark, off)                                                      \
+    off += (size_t)(WARPS) * (3 * (size_t)(NS) + 2) * DRT_WARP * 4;
 
 struct FilmPtrs { float *sum, *filter, *mean, *m2; };
 #define DRT_MAX_PEERS 16

@@ -116,8 +116,8 @@ extern "C" int drt_cuda_film_merge_slices_local(drt_cuda_context *ctx, const drt
                                                 uint32_t *bgra_sum, uint32_t *bgra_mean, uint32_t *bgra_var, void *stream)
 {
     if(!ctx || !slice_device || !staging || count < 1 || count > DRT_MAX_PEERS) return fail(DRT_CUDA_E_ARG, "bad argument (1..%d ranks)", DRT_MAX_PEERS);
-    if(!slice_device->sum || !slice_device->filter || !slice_device->mean || !slice_device->m2) return fail(DRT_CUDA_E_ARG, "NULL slice film");
-    if(!staging->sum || !staging->filter || !staging->mean || !staging->m2) return fail(DRT_CUDA_E_ARG, "NULL staging film");
+    if(!film_complete(slice_device)) return fail(DRT_CUDA_E_ARG, "NULL slice film");
+    if(!film_complete(staging)) return fail(DRT_CUDA_E_ARG, "NULL staging film");
     if(!ctx->have_scene) return fail(DRT_CUDA_E_STATE, "upload a scene first");
     const uint64_t npix = (uint64_t)width * height;
     if(pixel_begin > pixel_end || pixel_end > npix || pixel_end - pixel_begin > slice_pixels || npix > 0xffffffffull) return fail(DRT_CUDA_E_ARG, "bad pixel range");
@@ -129,11 +129,10 @@ extern "C" int drt_cuda_film_merge_slices_local(drt_cuda_context *ctx, const drt
     for(int g = 0; g < count; g += 1)   /* rank g's partial film of this slice: staging pixels [g * slice, (g + 1) * slice) */
         films[g] = FilmPtrs{ staging->sum + (size_t)g * slice_pixels * n, staging->filter + (size_t)g * slice_pixels,
                              staging->mean + (size_t)g * slice_pixels * n, staging->m2 + (size_t)g * slice_pixels * n };
-    FilmPtrs d = { slice_device->sum, slice_device->filter, slice_device->mean, slice_device->m2 };
     /* staging and slice film are indexed from the first pixel of the owner's slice; [pixel_begin, pixel_end) may be a part (a band) of it */
     const uint64_t slice_begin = (pixel_begin / slice_pixels) * slice_pixels;
     if(pixel_end - slice_begin > slice_pixels) return fail(DRT_CUDA_E_ARG, "pixel range crosses a slice boundary");
-    drt_launch_film_gather_merge(ctx->d_rgb_tables, count, films, d, (uint32_t)pixel_begin, (uint32_t)pixel_end, (uint32_t)slice_begin,
+    drt_launch_film_gather_merge(ctx->d_rgb_tables, count, films, film_ptrs(*slice_device), (uint32_t)pixel_begin, (uint32_t)pixel_end, (uint32_t)slice_begin,
                                  (uint32_t)slice_begin, bgra_sum, bgra_mean, bgra_var, ctx->num_sms * 8, (cudaStream_t)stream);
     CU(cudaGetLastError());
     ctx->launches += 1;
@@ -143,7 +142,7 @@ extern "C" int drt_cuda_film_merge_slices_local(drt_cuda_context *ctx, const drt
 extern "C" int drt_cuda_film_read_slice(drt_cuda_context *ctx, const drt_film *slice_device, uint64_t slice_begin, uint64_t pixel_begin, uint64_t pixel_end,
                                         const drt_film *film_host, void *stream)
 {
-    if(!ctx || !slice_device || !film_host || !film_host->sum || !film_host->filter || !film_host->mean || !film_host->m2) return fail(DRT_CUDA_E_ARG, "NULL argument");
+    if(!ctx || !slice_device || !film_complete(film_host)) return fail(DRT_CUDA_E_ARG, "NULL argument");
     if(!ctx->have_scene) return fail(DRT_CUDA_E_STATE, "upload a scene first");
     if(pixel_begin > pixel_end || slice_begin > pixel_begin) return fail(DRT_CUDA_E_ARG, "bad pixel range");
     CU(cudaSetDevice(ctx->device));
@@ -160,8 +159,7 @@ extern "C" int drt_cuda_film_read_slice(drt_cuda_context *ctx, const drt_film *s
 extern "C" int drt_cuda_film_read_rows(drt_cuda_context *ctx, const drt_film *film_device, uint32_t width, uint32_t height, int count, int rank,
                                        const drt_film *film_host, void *stream)
 {
-    if(!ctx || !film_device || !film_device->sum || !film_device->filter || !film_device->mean || !film_device->m2 ||
-       !film_host || !film_host->sum || !film_host->filter || !film_host->mean || !film_host->m2) return fail(DRT_CUDA_E_ARG, "NULL argument");
+    if(!ctx || !film_complete(film_device) || !film_complete(film_host)) return fail(DRT_CUDA_E_ARG, "NULL argument");
     if(count < 1 || count > DRT_MAX_PEERS || rank < 0 || rank >= count) return fail(DRT_CUDA_E_ARG, "bad row shard: rank %d of %d (1..%d ranks)", rank, count, DRT_MAX_PEERS);
     if(!ctx->have_scene) return fail(DRT_CUDA_E_STATE, "upload a scene first");
     CU(cudaSetDevice(ctx->device));
@@ -316,7 +314,7 @@ extern "C" int drt_cuda_render_host_multi_images(drt_cuda_context **ctxs, int co
     const bool want_images = bgra_sum_host || bgra_mean_host || bgra_var_host;
     if(want_images && !(bgra_sum_host && bgra_mean_host && bgra_var_host)) return fail(DRT_CUDA_E_ARG, "give all three image buffers or none");
     uint32_t *const host_images[3] = { bgra_sum_host, bgra_mean_host, bgra_var_host };
-    if(!ctxs || count < 1 || count > DRT_MAX_PEERS || !params || !out || !out->sum || !out->filter || !out->mean || !out->m2)
+    if(!ctxs || count < 1 || count > DRT_MAX_PEERS || !params || !film_complete(out))
         return fail(DRT_CUDA_E_ARG, "bad argument (1..%d contexts)", DRT_MAX_PEERS);
     for(int g = 0; g < count; g += 1)
     {
@@ -332,8 +330,8 @@ extern "C" int drt_cuda_render_host_multi_images(drt_cuda_context **ctxs, int co
         int rc1 = drt_cuda_render_host(ctxs[0], params, out);
         if(rc1 != DRT_CUDA_OK || !want_images) return rc1;
         /* the film render_host just produced is still in the library's device planes */
-        const size_t np1 = (size_t)params->width * params->height, plane = np1 * (size_t)ctxs[0]->n;
-        drt_film dev = { ctxs[0]->d_film, ctxs[0]->d_film + 3 * plane, ctxs[0]->d_film + plane, ctxs[0]->d_film + 2 * plane };
+        const size_t np1 = (size_t)params->width * params->height;
+        const drt_film dev = film_planes(ctxs[0]->d_film, np1, ctxs[0]->n);
         uint32_t *scratch = nullptr;
         CU(cudaSetDevice(ctxs[0]->device));
         CU(cudaMalloc(&scratch, 3 * np1 * 4));

@@ -1,6 +1,6 @@
 /*
- * csrc/drt_kernels.cu -- dispatch to the render kernel instantiations and the launch geometry they are compiled for.
- * The kernel itself is the template in drt_render.cuh.
+ * csrc/drt_kernels.cu -- dispatch to the render kernel instantiations and the shared memory a launch of them needs.
+ * The kernel itself is the template in drt_render.cuh, its launch shapes are DRT_RENDER_SHAPE in drt_device.cuh.
  */
 #include <cuda_runtime.h>
 #include "drt_device.cuh"
@@ -34,27 +34,11 @@ cudaError_t drt_launch_render(const RenderLaunch &L, bool f64_geometry, int mode
     return deep ? drt_launch_render_f32_general_deep(L, paired, nslots, grid, warps, smem, stream) : drt_launch_render_f32_general(L, paired, nslots, grid, warps, smem, stream);
 }
 
-int drt_render_cta_warps(bool f64_geometry, int mode)
-{
-    if(f64_geometry) return DRT_CTA_WARPS;
-    return mode == 1 ? DRT_FAST_WARPS : mode == 2 ? DRT_CLASSED_WARPS : DRT_CTA_WARPS;
-}
-
-int drt_render_min_ctas(bool f64_geometry, int mode)
-{
-    if(f64_geometry) return DRT_GENERAL_CTAS;
-    return mode == 1 ? DRT_MIN_CTAS : mode == 2 ? DRT_CLASSED_CTAS : DRT_GENERAL_CTAS;
-}
-
+/* the carve of the kernel body, without its pointers */
 size_t drt_render_smem_bytes(const RenderLaunch &L, bool f64_geometry, int warps, int nslots)
 {
-    size_t geom = f64_geometry ? sizeof(GeomT<double>) : sizeof(GeomT<float>);
-    size_t off = (geom + 15) & ~size_t(15);
-    off += (sizeof(SpdIndex) + 15) & ~size_t(15);
-    off += (size_t)L.pool_words * 4;
-    off += 16 * 8;
-    off = (off + 15) & ~size_t(15);
-    off += (size_t)warps * L.path_stride * DRT_WARP * 4;
-    off += (size_t)warps * (3 * (size_t)nslots + 2) * DRT_WARP * 4;   /* film parking */
+#define DRT_SMEM_NO_POINTER(T, NAME, AT)
+    DRT_RENDER_SMEM_CARVE(DRT_SMEM_NO_POINTER, f64_geometry ? sizeof(GeomT<double>) : sizeof(GeomT<float>), L.pool_words, warps, L.path_stride, nslots)
+#undef DRT_SMEM_NO_POINTER
     return off;
 }

@@ -1633,9 +1633,6 @@ static __device__ __noinline__ void dump_path(float *record_dump, float *path_du
 /* ALLFAST: every surface material of the scene is a two-lobe plastic and there is exactly one light (decided by the
  * host at scene upload: all shipped Cornell boxes except the gold/glass balls of cornell_plane_light).  The kernel then
  * contains neither the general lobe evaluators nor the general shader. */
-#ifndef DRT_PARK_GENERAL
-#define DRT_PARK_GENERAL 0   /* park the film of the general kernel too (pays off only if that buys resident warps) */
-#endif
 /* Phase clocks, diagnostic builds only (tools/build_variant.sh NAME -DDRT_PHASE_CLOCKS; tools/phase_split.py reads them through
  * drt_cuda_phase_clocks).  Each warp's timeline after the scene staging is cut at the boundaries of a batch, and the SM-clock cycles
  * since the previous cut go to the part that just ended: TRACE = phase 1 (film parking, the gate in front of it, trace_path), BOOK =
@@ -1653,8 +1650,7 @@ static __device__ __noinline__ void dump_path(float *record_dump, float *path_du
 #define DRT_PHASE_CUT(k) do {} while(0)
 #endif
 /* PAIRED: one pixel per task with all its samples (spp >= 32) against 32/spp whole pixels per task; see the task loop. */
-#define DRT_RENDER_BOUNDS(MODE) __launch_bounds__((MODE == 1 ? DRT_FAST_WARPS : MODE == 2 ? DRT_CLASSED_WARPS : DRT_CTA_WARPS) * DRT_WARP, \
-                                                  MODE == 1 ? DRT_MIN_CTAS : MODE == 2 ? DRT_CLASSED_CTAS : DRT_GENERAL_CTAS)
+#define DRT_RENDER_BOUNDS(MODE) __launch_bounds__(DRT_RENDER_SHAPE[MODE].warps * DRT_WARP, DRT_RENDER_SHAPE[MODE].min_ctas)
 template <typename R, int NS, int MODE, bool PAIRED, bool DEEP>
 __global__ void DRT_RENDER_BOUNDS(MODE) render_kernel(const RenderLaunch L)
 {

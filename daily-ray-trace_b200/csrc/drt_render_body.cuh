@@ -8,10 +8,10 @@
  * the tree as without it.  All adaptive code is behind `if constexpr(ADAPTIVE)`.
  */
     constexpr bool ALLFAST = MODE != 0;   /* compact records, film parked in shared memory while tracing */
-    /* LOCKSTEP (a kernel whose hot code does not fit the 32 KB instruction cache; DRT_LOCKSTEP says which modes): the warps of a CTA
+    /* LOCKSTEP (a kernel whose hot code does not fit the 32 KB instruction cache; DRT_RENDER_SHAPE says which modes): the warps of a CTA
      * run their phases together -- a gate (an mbarrier that every warp arrives at once per phase and leaves for good when it runs
      * out of pixels) in front of phase 1 and of phase 2 -- so that at any time the SM fetches the code of ONE phase. */
-    constexpr bool LOCKSTEP = MODE == 2 ? ((DRT_LOCKSTEP & 2) != 0) : MODE == 0 ? ((DRT_LOCKSTEP & 1) != 0) : ((DRT_LOCKSTEP & 4) != 0);
+    constexpr bool LOCKSTEP = DRT_RENDER_SHAPE[MODE].lockstep;
     __shared__ unsigned long long phase_bar;
     __shared__ uint32_t gates_off;
 #ifdef DRT_PHASE_CLOCKS
@@ -27,16 +27,9 @@
     }
     extern __shared__ __align__(16) unsigned char smem_raw[];
     GeomT<R> *sg = reinterpret_cast<GeomT<R> *>(smem_raw);
-    size_t off = (sizeof(GeomT<R>) + 15) & ~size_t(15);
-    SpdIndex *six = reinterpret_cast<SpdIndex *>(smem_raw + off);
-    off += (sizeof(SpdIndex) + 15) & ~size_t(15);
-    float *spool = reinterpret_cast<float *>(smem_raw + off);
-    off += (size_t)L.pool_words * 4;
-    unsigned long long *s_stats = reinterpret_cast<unsigned long long *>(smem_raw + off);
-    off += 16 * 8;
-    off = (off + 15) & ~size_t(15);
-    float *srec = reinterpret_cast<float *>(smem_raw + off);
-    float *spark = srec + (size_t)(blockDim.x >> 5) * L.path_stride * DRT_WARP;   /* film parking, (3 NS + 2) * 32 words per warp */
+#define DRT_SMEM_POINTER(T, NAME, AT) T *NAME = reinterpret_cast<T *>(smem_raw + (AT));
+    DRT_RENDER_SMEM_CARVE(DRT_SMEM_POINTER, sizeof(GeomT<R>), L.pool_words, blockDim.x >> 5, L.path_stride, NS)
+#undef DRT_SMEM_POINTER
 
     /* stage the scene once per (persistent) CTA */
     {
@@ -182,7 +175,7 @@
             /* ---- phase 1: lane = path ---- */
             DRT_PHASE_CUT(DRT_PHASE_OTHER);
             gate();
-            if((ALLFAST || DRT_PARK_GENERAL) && paired) film.park(park);
+            if(ALLFAST && paired) film.park(park);
             const uint32_t q = q0 + lane;
             uint32_t bin = 9, general = 0;
             uint32_t my_px = 0, my_s = q;      /* pixel of the batch and sample index inside the pixel */
@@ -209,7 +202,6 @@
             DRT_PHASE_CUT(DRT_PHASE_TRACE);
             gate();
             /* compact records: the film stays parked through the replay, which accumulates BatchStats instead */
-            if(!ALLFAST && DRT_PARK_GENERAL && paired) film.unpark(park);
             {
                 /* termination histogram: one shared-memory atomic per distinct bin of the batch (bin 9 = idle lane) */
                 const uint32_t peers = __match_any_sync(0xffffffffu, bin);

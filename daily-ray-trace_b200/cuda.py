@@ -117,6 +117,14 @@ def _check(rc):
         raise CudaError(rc, lib().drt_cuda_last_error().decode(errors="replace"))
 
 
+def _host_film(npix, n):
+    """Host planes for a film of npix pixels and n wavelengths: dict of numpy f32 arrays sum[npix, n], filter[npix], mean, m2, and the
+    Film over them."""
+    out = {"sum": np.empty((npix, n), np.float32), "filter": np.empty(npix, np.float32),
+           "mean": np.empty((npix, n), np.float32), "m2": np.empty((npix, n), np.float32)}
+    return out, Film(*(out[k].ctypes.data for k in ("sum", "filter", "mean", "m2")))
+
+
 def device_count():
     return lib().drt_cuda_device_count()
 
@@ -162,22 +170,15 @@ class Context:
 
     def render_host(self, params):
         """End-to-end call with host buffers: returns dict of numpy f32 arrays sum[H*W,N], filter[H*W], mean, m2."""
-        npix = max(params.width * params.height, 1)
-        n = self.n or 1     # before upload_scene the library reports DRT_CUDA_E_STATE; buffers only need to exist
-        out = {"sum": np.empty((npix, n), np.float32), "filter": np.empty(npix, np.float32),
-               "mean": np.empty((npix, n), np.float32), "m2": np.empty((npix, n), np.float32)}
-        film = Film(out["sum"].ctypes.data, out["filter"].ctypes.data, out["mean"].ctypes.data, out["m2"].ctypes.data)
+        # before upload_scene the library reports DRT_CUDA_E_STATE; buffers only need to exist
+        out, film = _host_film(max(params.width * params.height, 1), self.n or 1)
         _check(lib().drt_cuda_render_host(self._h, C.byref(params), C.byref(film)))
         return out
 
     def render_host_adaptive(self, params, rel_error, min_samples):
         """render_host with adaptive sampling (drt_cuda_render_host_adaptive): every pixel stops once the error bound of its luminance
         is <= rel_error times the luminance and it has >= min_samples samples; filter holds each pixel's count."""
-        npix = max(params.width * params.height, 1)
-        n = self.n or 1
-        out = {"sum": np.empty((npix, n), np.float32), "filter": np.empty(npix, np.float32),
-               "mean": np.empty((npix, n), np.float32), "m2": np.empty((npix, n), np.float32)}
-        film = Film(out["sum"].ctypes.data, out["filter"].ctypes.data, out["mean"].ctypes.data, out["m2"].ctypes.data)
+        out, film = _host_film(max(params.width * params.height, 1), self.n or 1)
         _check(lib().drt_cuda_render_host_adaptive(self._h, C.byref(params), C.byref(Adaptive(rel_error, min_samples)), C.byref(film)))
         return out
 
@@ -317,10 +318,7 @@ class Context:
 
 def render_host_multi(contexts, params):
     """render_host over several Context objects on distinct devices of this process: dict of numpy f32 arrays like Context.render_host."""
-    npix, n = params.width * params.height, contexts[0].n
-    out = {"sum": np.empty((npix, n), np.float32), "filter": np.empty(npix, np.float32),
-           "mean": np.empty((npix, n), np.float32), "m2": np.empty((npix, n), np.float32)}
-    film = Film(out["sum"].ctypes.data, out["filter"].ctypes.data, out["mean"].ctypes.data, out["m2"].ctypes.data)
+    out, film = _host_film(params.width * params.height, contexts[0].n)
     handles = (C.c_void_p * len(contexts))(*[c._h for c in contexts])
     _check(lib().drt_cuda_render_host_multi(handles, len(contexts), C.byref(params), C.byref(film)))
     return out
@@ -333,10 +331,7 @@ def render_host_multi_adaptive(contexts, params, rel_error, min_samples, film=No
     then None is returned."""
     out = None
     if film is None:
-        npix, n = params.width * params.height, contexts[0].n or 1
-        out = {"sum": np.empty((npix, n), np.float32), "filter": np.empty(npix, np.float32),
-               "mean": np.empty((npix, n), np.float32), "m2": np.empty((npix, n), np.float32)}
-        film = Film(out["sum"].ctypes.data, out["filter"].ctypes.data, out["mean"].ctypes.data, out["m2"].ctypes.data)
+        out, film = _host_film(params.width * params.height, contexts[0].n or 1)
     handles = (C.c_void_p * len(contexts))(*[c._h for c in contexts])
     _check(lib().drt_cuda_render_host_multi_adaptive(handles, len(contexts), C.byref(params), C.byref(Adaptive(rel_error, min_samples)),
                                                       C.byref(film)))
