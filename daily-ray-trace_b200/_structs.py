@@ -52,6 +52,10 @@ class Adaptive(C.Structure):
     _fields_ = [("rel_error", C.c_float), ("min_samples", C.c_uint32)]
 
 
+class Denoise(C.Structure):
+    _fields_ = [("search_radius", C.c_uint32), ("patch_radius", C.c_uint32), ("strength", C.c_float)]
+
+
 class Config(C.Structure):
     _paths = ["input_scene", "output_spd", "average_spd", "variance_spd", "output_bmp", "average_bmp", "variance_bmp",
               "white_spd", "cmf_x", "cmf_y", "cmf_z", "red_spd", "green_spd", "blue_spd", "cyan_spd", "magenta_spd",

@@ -66,6 +66,7 @@ extern "C" void drt_cuda_destroy(drt_cuda_context *ctx)
     cudaSetDevice(ctx->device);
     cudaFree(ctx->d_geom32); cudaFree(ctx->d_geom64); cudaFree(ctx->d_index); cudaFree(ctx->d_pool);
     cudaFree(ctx->d_rgb_tables); cudaFree(ctx->d_stats_ring); cudaFree(ctx->d_counter_ring); cudaFree(ctx->d_film); cudaFree(ctx->d_dump); cudaFree(ctx->d_slice); cudaFree(ctx->d_deep);
+    cudaFree(ctx->d_denoise);
     drt_exchange_release(ctx);
     if(ctx->band_render) cudaStreamDestroy(ctx->band_render);
     if(ctx->band_copy) cudaStreamDestroy(ctx->band_copy);
@@ -1108,6 +1109,71 @@ extern "C" int drt_cuda_film_merge(drt_cuda_context *ctx, const drt_film *dst, c
     drt_launch_film_merge(film_ptrs(*dst), film_ptrs(*src), (uint32_t)ctx->n, (size_t)width * height, ctx->num_sms * 8, (cudaStream_t)stream);
     CU(cudaGetLastError());
     ctx->launches += 2;
+    return DRT_CUDA_OK;
+}
+
+static bool overlaps(const float *a, size_t na, const float *b, size_t nb) { return a < b + nb && b < a + na; }
+
+/* argument checks of the denoise entry points (drt_cuda.h), before anything is copied or launched */
+static int denoise_args(const drt_cuda_context *ctx, const drt_film *film, uint32_t width, uint32_t height, const drt_denoise *opt, const float *out)
+{
+    if(!ctx || !film || !opt || !out) return fail(DRT_CUDA_E_ARG, "NULL argument");
+    if(!ctx->have_scene) return fail(DRT_CUDA_E_STATE, "upload a scene first");
+    if(!film->mean || !film->m2 || !film->filter) return fail(DRT_CUDA_E_ARG, "denoise: the film needs its mean, m2 and filter planes");
+    if(width == 0 || height == 0 || (uint64_t)width * height > 0xffffffffull)
+        return fail(DRT_CUDA_E_ARG, "denoise: width and height must be > 0, and width x height < 2^32 (got %u x %u)", width, height);
+    if(opt->search_radius < 1 || opt->search_radius > 15) return fail(DRT_CUDA_E_ARG, "denoise: search_radius must lie in 1..15 (got %u)", opt->search_radius);
+    if(opt->patch_radius > 4) return fail(DRT_CUDA_E_ARG, "denoise: patch_radius must lie in 0..4 (got %u)", opt->patch_radius);
+    if(!(opt->strength > 0.f) || !isfinite(opt->strength))
+        return fail(DRT_CUDA_E_ARG, "denoise: strength must be a finite number > 0 (got %g)", (double)opt->strength);
+    const size_t npix = (size_t)width * height, plane = npix * (size_t)ctx->n;
+    if(overlaps(out, plane, film->mean, plane) || overlaps(out, plane, film->m2, plane) || overlaps(out, plane, film->filter, npix))
+        return fail(DRT_CUDA_E_ARG, "denoise: mean_out overlaps the film's mean, m2 or filter plane");
+    return DRT_CUDA_OK;
+}
+
+/* guide, then filter, on `stream` (arguments checked) */
+static int denoise(drt_cuda_context *ctx, const drt_film *film, uint32_t width, uint32_t height, const drt_denoise *opt, float *out, cudaStream_t stream)
+{
+    const size_t npix = (size_t)width * height;
+    int rc = drt_ensure_buffer(&ctx->d_denoise, &ctx->denoise_bytes, 3 * npix * sizeof(float));
+    if(rc != DRT_CUDA_OK) return rc;
+    const float *yw = reinterpret_cast<const float *>(static_cast<const unsigned char *>(ctx->d_rgb_tables) + drt_rgb_tables_yw_offset());
+    drt_launch_denoise_guide(yw, film->mean, film->m2, film->filter, (uint32_t)npix, ctx->n, ctx->d_denoise, ctx->num_sms * 8, stream);
+    CU(cudaGetLastError());
+    CU(drt_launch_denoise_filter(film->mean, ctx->d_denoise, width, height, ctx->n, (int)opt->search_radius, (int)opt->patch_radius,
+                                 opt->strength, out, stream));
+    ctx->launches += 2;
+    return DRT_CUDA_OK;
+}
+
+extern "C" int drt_cuda_film_denoise(drt_cuda_context *ctx, const drt_film *film, uint32_t width, uint32_t height, const drt_denoise *opt,
+                                     float *mean_out, void *stream)
+{
+    int rc = denoise_args(ctx, film, width, height, opt, mean_out);
+    if(rc != DRT_CUDA_OK) return rc;
+    CU(cudaSetDevice(ctx->device));
+    return denoise(ctx, film, width, height, opt, mean_out, (cudaStream_t)stream);
+}
+
+/* The film goes up into the library-owned film (d_film): its mean, m2 and filter planes hold the input, its sum plane the output. */
+extern "C" int drt_cuda_film_denoise_host(drt_cuda_context *ctx, const drt_film *film, uint32_t width, uint32_t height, const drt_denoise *opt,
+                                          float *mean_out)
+{
+    int rc = denoise_args(ctx, film, width, height, opt, mean_out);
+    if(rc != DRT_CUDA_OK) return rc;
+    CU(cudaSetDevice(ctx->device));
+    const size_t npix = (size_t)width * height, bytes = npix * (size_t)ctx->n * sizeof(float);
+    drt_film f;
+    rc = drt_library_film(ctx, &ctx->d_film, &ctx->film_bytes, npix, &f);
+    if(rc != DRT_CUDA_OK) return rc;
+    CU(cudaMemcpyAsync(f.mean, film->mean, bytes, cudaMemcpyHostToDevice, 0));
+    CU(cudaMemcpyAsync(f.m2, film->m2, bytes, cudaMemcpyHostToDevice, 0));
+    CU(cudaMemcpyAsync(f.filter, film->filter, npix * sizeof(float), cudaMemcpyHostToDevice, 0));
+    rc = denoise(ctx, &f, width, height, opt, f.sum, 0);
+    if(rc != DRT_CUDA_OK) return rc;
+    CU(cudaMemcpyAsync(mean_out, f.sum, bytes, cudaMemcpyDeviceToHost, 0));
+    CU(cudaStreamSynchronize(0));
     return DRT_CUDA_OK;
 }
 

@@ -18,6 +18,12 @@ void        drt_launch_film_merge(FilmPtrs dst, FilmPtrs src, uint32_t n, size_t
 void        drt_launch_fma_peak(int packed, float *out, int iters, int grid, cudaStream_t stream);
 void        drt_launch_film_gather_merge(const void *tables, int count, const FilmPtrs *films, FilmPtrs dst, uint32_t pixel_begin, uint32_t pixel_end, uint32_t src_base, uint32_t dst_base,
                                          uint32_t *bgra_sum, uint32_t *bgra_mean, uint32_t *bgra_var, int grid, cudaStream_t stream);
+/* drt_denoise.cu: the guide planes (Y, v, usable as 1 / 0, npix each) of a film, then the filter of drt_cuda_film_denoise from them */
+void        drt_launch_denoise_guide(const float *yw, const float *mean, const float *m2, const float *filter, uint32_t npix, int n, float *guide,
+                                     int grid, cudaStream_t stream);
+cudaError_t drt_launch_denoise_filter(const float *mean, const float *guide, uint32_t width, uint32_t height, int n, int search_radius,
+                                      int patch_radius, float strength, float *out, cudaStream_t stream);
+size_t      drt_denoise_smem_bytes(int n, int search_radius, int patch_radius);
 size_t      drt_rgb_tables_bytes(void);
 size_t      drt_rgb_tables_yw_offset(void);   /* byte offset of the luminance weights cmf_y * ref_white (adaptive sampling) */
 void        drt_fill_rgb_tables(void *dst_host, const drt_tables *t);
@@ -60,6 +66,7 @@ struct drt_cuda_context
     float *d_dump = nullptr; size_t dump_bytes = 0;
     float *d_deep = nullptr; size_t deep_bytes = 0;     /* overflow rows of deep renders (RenderLaunch::deep) */
     float *d_slice = nullptr; size_t slice_bytes = 0;   /* merged planes of this rank's slice before they are copied to the root */
+    float *d_denoise = nullptr; size_t denoise_bytes = 0;   /* the denoise guide planes (drt_denoise.cu) */
     uint64_t launches = 0;
     size_t upload_bytes = 0;
     uint64_t last_launches = 0;

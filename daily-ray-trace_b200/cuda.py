@@ -8,7 +8,7 @@ import os
 import numpy as np
 
 from . import PACKAGE_DIR
-from ._structs import Adaptive, Camera, RenderParams, Scene, Tables
+from ._structs import Adaptive, Camera, Denoise, RenderParams, Scene, Tables
 
 GEOMETRY_F32, GEOMETRY_F64 = 0, 1
 
@@ -21,7 +21,7 @@ EXPORTS = ["drt_cuda_last_error", "drt_cuda_device_count", "drt_cuda_create", "d
            "drt_cuda_film_merge_slices_local", "drt_cuda_film_read_slice", "drt_cuda_flags_signal", "drt_cuda_flags_wait", "drt_cuda_flags_timeouts",
            "drt_cuda_host_alloc", "drt_cuda_host_free", "drt_cuda_render_host_multi_images", "drt_cuda_render_device_scatter_band", "drt_cuda_plan_scene",
            "drt_cuda_render_device_adaptive", "drt_cuda_render_host_adaptive", "drt_cuda_render_device_adaptive_rows", "drt_cuda_film_read_rows",
-           "drt_cuda_render_host_multi_adaptive"]
+           "drt_cuda_render_host_multi_adaptive", "drt_cuda_film_denoise", "drt_cuda_film_denoise_host"]
 
 
 class Film(C.Structure):
@@ -94,6 +94,8 @@ def lib():
         L.drt_cuda_film_to_rgb.argtypes = [C.c_void_p, C.POINTER(Film), C.c_uint32, C.c_uint32, C.c_int, C.c_void_p,
                                            C.c_void_p, C.c_void_p]
         L.drt_cuda_film_merge.argtypes = [C.c_void_p, C.POINTER(Film), C.POINTER(Film), C.c_uint32, C.c_uint32, C.c_void_p]
+        L.drt_cuda_film_denoise.argtypes = [C.c_void_p, C.POINTER(Film), C.c_uint32, C.c_uint32, C.POINTER(Denoise), C.c_void_p, C.c_void_p]
+        L.drt_cuda_film_denoise_host.argtypes = [C.c_void_p, C.POINTER(Film), C.c_uint32, C.c_uint32, C.POINTER(Denoise), C.c_void_p]
         L.drt_cuda_debug_records.argtypes = [C.c_void_p, C.POINTER(RenderParams)] + [C.c_uint32] * 4 + [C.c_void_p, C.c_size_t, C.POINTER(C.c_uint32)]
         L.drt_cuda_buffer_alloc.argtypes = [C.c_void_p, C.c_size_t, C.POINTER(C.c_void_p)]
         L.drt_cuda_buffer_free.argtypes = [C.c_void_p, C.c_void_p]
@@ -227,6 +229,31 @@ class Context:
 
     def film_merge(self, dst, src, width, height, stream=None):
         _check(lib().drt_cuda_film_merge(self._h, C.byref(dst), C.byref(src), width, height, stream))
+
+    def film_denoise(self, film, width, height, search_radius=7, patch_radius=3, strength=0.45, out=None, stream=None):
+        """Non-local-means denoising of a device film (drt_cuda_film_denoise, stream-ordered): writes the filtered mean plane [W*H*N] to the
+        device pointer `out` (which must not overlap the film), or to a new torch CUDA tensor, which is returned."""
+        t = None
+        if out is None:
+            import torch
+            t = torch.empty(width * height * (self.n or 1), dtype=torch.float32, device=f"cuda:{self.device}")
+            out = t.data_ptr()
+        _check(lib().drt_cuda_film_denoise(self._h, C.byref(film), width, height, C.byref(Denoise(search_radius, patch_radius, strength)),
+                                           out, stream))
+        return t
+
+    def film_denoise_host(self, film, width, height, search_radius=7, patch_radius=3, strength=0.45):
+        """drt_cuda_film_denoise on host planes: `film` is a dict of numpy f32 arrays like render_host returns (mean, m2, filter; sum
+        unused).  Returns the filtered mean as a new f32 array [W*H, N]."""
+        n = self.n or 1
+        planes = {k: np.ascontiguousarray(film[k], dtype=np.float32) for k in ("mean", "m2", "filter")}
+        if planes["filter"].size != width * height or planes["mean"].size != width * height * n or planes["m2"].size != width * height * n:
+            raise ValueError(f"film planes do not hold {width} x {height} pixels of {n} wavelengths")
+        out = np.empty((width * height, n), np.float32)
+        f = Film(None, planes["filter"].ctypes.data, planes["mean"].ctypes.data, planes["m2"].ctypes.data)
+        _check(lib().drt_cuda_film_denoise_host(self._h, C.byref(f), width, height, C.byref(Denoise(search_radius, patch_radius, strength)),
+                                                out.ctypes.data))
+        return out
 
     def buffer_alloc(self, nbytes):
         p = C.c_void_p()

@@ -6,7 +6,7 @@
  * (win32_main.c:129-152).  The render itself goes through the C ABI of include/drt_cuda.h; the timed region is the
  * reference's render_timer scope (sampling + film accumulation, daily_ray_trace.c:709-752; file I/O excluded).
  *
- *   drt_raytrace [config.cfg] [--device N] [--gpus G] [--seed S] [--strict] [--f64-geometry] [--cpu-images] [--adaptive REL [--min-spp M]]
+ *   drt_raytrace [config.cfg] [--device N] [--gpus G] [--seed S] [--strict] [--f64-geometry] [--cpu-images] [--adaptive REL [--min-spp M]] [--denoise]
  * --gpus G renders on devices N .. N+G-1: the samples of every pixel are split over them (drt_cuda_render_host_multi_images).
  * The three .bmp images come from the devices with the film (converted from the merged film there, fused into the multi-GPU merge
  * kernel); --cpu-images converts them the reference's way instead: by reading the .spd files back (spd_file_to_rgb_f64_pixels,
@@ -14,6 +14,8 @@
  * --adaptive REL samples adaptively (drt_cuda_render_host_adaptive): a pixel stops once the error bound of its luminance is at most REL
  * times the luminance and it has at least M samples (--min-spp, default 64, at most num_pixel_samples); num_pixel_samples is the cap.
  * One device only, and the .bmp images are converted from the .spd files as with --cpu-images.
+ * --denoise also filters the film with non-local means at the default parameters (drt_cuda_film_denoise_host on the first device) and
+ * writes denoised.spd (the format of average.spd) and denoised.bmp next to average.spd; the other files are those of a run without it.
  */
 #include <stdio.h>
 #include <stdlib.h>
@@ -45,7 +47,7 @@ static int spd_to_bmp(const char *spd, const char *bmp, const drt_tables *t)
 int main(int argc, char **argv)
 {
     const char *config_path = "config.cfg";
-    int device = 0, gpus = 1, flags = DRT_PARSE_LEGACY_COMPAT, precision = DRT_GEOMETRY_F32, cpu_images = 0, adaptive = 0;
+    int device = 0, gpus = 1, flags = DRT_PARSE_LEGACY_COMPAT, precision = DRT_GEOMETRY_F32, cpu_images = 0, adaptive = 0, denoise = 0;
     unsigned long long seed = 0;
     drt_adaptive ad = { 0.f, 64u };
     for(int i = 1; i < argc; i += 1)
@@ -56,6 +58,7 @@ int main(int argc, char **argv)
         else if(strcmp(argv[i], "--strict") == 0) flags = DRT_PARSE_STRICT;
         else if(strcmp(argv[i], "--f64-geometry") == 0) precision = DRT_GEOMETRY_F64;
         else if(strcmp(argv[i], "--cpu-images") == 0) cpu_images = 1;
+        else if(strcmp(argv[i], "--denoise") == 0) denoise = 1;
         else if(strcmp(argv[i], "--adaptive") == 0 && i + 1 < argc) { adaptive = 1; ad.rel_error = strtof(argv[++i], NULL); }
         else if(strcmp(argv[i], "--min-spp") == 0 && i + 1 < argc) ad.min_samples = (uint32_t)strtoul(argv[++i], NULL, 0);
         else config_path = argv[i];
@@ -154,6 +157,28 @@ int main(int argc, char **argv)
         if(drt_write_bmp(cfg.variance_bmp, prm.width, prm.height, images[2]) != DRT_OK) return die_host("variance bmp");
     }
     printf("Converted.\n");
+
+    if(denoise)
+    {
+        /* denoised.spd / .bmp in the directory of average_spd (a path of the config file: '\\' or '/' separated) */
+        char spd[80], bmp[80];
+        const char *slash = strrchr(cfg.average_spd, '\\'), *fwd = strrchr(cfg.average_spd, '/');
+        if(fwd && (!slash || fwd > slash)) slash = fwd;
+        const int dir = slash ? (int)(slash - cfg.average_spd) + 1 : 0;
+        snprintf(spd, sizeof(spd), "%.*sdenoised.spd", dir, cfg.average_spd);
+        snprintf(bmp, sizeof(bmp), "%.*sdenoised.bmp", dir, cfg.average_spd);
+        const size_t bytes = npix * n * 4;
+        float *out = (float *)malloc(bytes ? bytes : 4);
+        if(!out) { fprintf(stderr, "ERROR: out of host memory\n"); return 1; }
+        const drt_denoise opt = { 7u, 3u, 0.45f };
+        t0 = now_ms();
+        if(drt_cuda_film_denoise_host(ctxs[0], &film, prm.width, prm.height, &opt, out) != DRT_CUDA_OK) return die_cuda("denoise");
+        printf("Denoise time: %fms (non-local means, search radius %u, patch radius %u, strength %g)\n", now_ms() - t0, opt.search_radius,
+               opt.patch_radius, (double)opt.strength);
+        if(drt_write_spd_plain(spd, &tables, prm.width, prm.height, out, 0) != DRT_OK) return die_host("denoised spd");
+        if(spd_to_bmp(spd, bmp, &tables) != 0) return die_host("denoised bmp");
+        free(out);
+    }
 
     for(int i = 0; i < 7; i += 1) { if(pinned) drt_cuda_host_free(blocks[i]); else free(blocks[i]); }
     for(int g = 0; g < gpus; g += 1) drt_cuda_destroy(ctxs[g]);

@@ -206,6 +206,33 @@ int  drt_cuda_film_to_rgb(drt_cuda_context *ctx, const drt_film *film_device, ui
 int  drt_cuda_film_merge(drt_cuda_context *ctx, const drt_film *dst_device, const drt_film *src_device,
                          uint32_t width, uint32_t height, void *stream);
 
+/* Non-local-means denoising of a finished film, guided by its own mean and M2 (Rousselle, Knaus and Zwicker, "Adaptive rendering with
+ * non-local means filtering", SIGGRAPH Asia 2012).  Reads the mean, m2 and filter planes (sum is ignored and may be NULL) and writes the
+ * filtered mean plane [W*H*N] to mean_out, which must not overlap the film's planes; the film is not written.
+ *   usable pixel p:  count n_p = filter >= 2 and every mean and m2 value finite
+ *   guide:           Y_p = sum_l w_l mean_l(p),  v_p = (sum_l w_l sqrt(m2_l(p) / (n_p (n_p - 1))))^2  (w_l = cmf_y * ref_white, the
+ *                    adaptive rule's weights); Y_p = v_p = 0 for an unusable p (they only enter the patches of other pixels)
+ *   distance:        for q = p + d, d in [-r, r]^2, q inside the image and usable:
+ *                    D(a, b) = ((Y_a - Y_b)^2 - (v_a + min(v_a, v_b))) / (1e-10 + k^2 (v_a + v_b))
+ *                    d2(p, q) = mean over o in [-f, f]^2 of D(clamp(p + o), clamp(q + o))   (clamp replicates the border)
+ *   output:          wt(p, q) = exp(-max(0, d2(p, q))), wt(p, p) = 1;  out_l(p) = sum_q wt(p, q) mean_l(q) / sum_q wt(p, q) for a usable p;
+ *                    an unusable p is copied bit for bit.
+ * r = search_radius 1..15 (default 7), f = patch_radius 0..4 (default 3), k = strength finite and > 0 (default 0.45), else DRT_CUDA_E_ARG;
+ * also W, H > 0 and the planes present.  N and w come from the uploaded scene (DRT_CUDA_E_STATE without one).  f32 sums in a fixed order:
+ * the result is deterministic. */
+typedef struct
+{
+    uint32_t search_radius, patch_radius;
+    float    strength;
+} drt_denoise;
+
+/* Stream-ordered: film_device and mean_out_device are device planes. */
+int  drt_cuda_film_denoise(drt_cuda_context *ctx, const drt_film *film_device, uint32_t width, uint32_t height, const drt_denoise *opt,
+                           float *mean_out_device, void *stream);
+/* The same on host planes: copies the film up into library-owned device planes, filters, copies the result down and waits. */
+int  drt_cuda_film_denoise_host(drt_cuda_context *ctx, const drt_film *film_host, uint32_t width, uint32_t height, const drt_denoise *opt,
+                                float *mean_out_host);
+
 /* ---- multi-GPU: library-owned films that other processes / devices can map, and the fused merge epilogue ---- */
 
 /* Allocates the four planes of a W x H film with cudaMalloc (zero-filled) so that they can be exported over CUDA IPC. */
