@@ -67,6 +67,7 @@ extern "C" void drt_cuda_destroy(drt_cuda_context *ctx)
     cudaFree(ctx->d_geom32); cudaFree(ctx->d_geom64); cudaFree(ctx->d_index); cudaFree(ctx->d_pool);
     cudaFree(ctx->d_rgb_tables); cudaFree(ctx->d_stats_ring); cudaFree(ctx->d_counter_ring); cudaFree(ctx->d_film); cudaFree(ctx->d_dump); cudaFree(ctx->d_slice); cudaFree(ctx->d_deep);
     cudaFree(ctx->d_denoise);
+    if(ctx->denoise_done) cudaEventDestroy(ctx->denoise_done);
     drt_exchange_release(ctx);
     if(ctx->band_render) cudaStreamDestroy(ctx->band_render);
     if(ctx->band_copy) cudaStreamDestroy(ctx->band_copy);
@@ -1124,8 +1125,12 @@ static int denoise_args(const drt_cuda_context *ctx, const drt_film *film, uint3
         return fail(DRT_CUDA_E_ARG, "denoise: width and height must be > 0, and width x height < 2^32 (got %u x %u)", width, height);
     if(opt->search_radius < 1 || opt->search_radius > 15) return fail(DRT_CUDA_E_ARG, "denoise: search_radius must lie in 1..15 (got %u)", opt->search_radius);
     if(opt->patch_radius > 4) return fail(DRT_CUDA_E_ARG, "denoise: patch_radius must lie in 0..4 (got %u)", opt->patch_radius);
-    if(!(opt->strength > 0.f) || !isfinite(opt->strength))
-        return fail(DRT_CUDA_E_ARG, "denoise: strength must be a finite number > 0 (got %g)", (double)opt->strength);
+    /* the filter takes k^2 as an f32: it must be a normal number, so that neither 1e-10 + k^2 (v_a + v_b) nor its product overflows
+     * to inf or vanishes for every finite pair of variances */
+    const float kk = opt->strength * opt->strength;
+    if(!(opt->strength > 0.f) || !isnormal(kk))
+        return fail(DRT_CUDA_E_ARG, "denoise: strength must lie in [2^-63, 2^64), so that strength^2 is a normal f32 (got %g)",
+                    (double)opt->strength);
     const size_t npix = (size_t)width * height, plane = npix * (size_t)ctx->n;
     if(overlaps(out, plane, film->mean, plane) || overlaps(out, plane, film->m2, plane) || overlaps(out, plane, film->filter, npix))
         return fail(DRT_CUDA_E_ARG, "denoise: mean_out overlaps the film's mean, m2 or filter plane");
@@ -1139,10 +1144,13 @@ static int denoise(drt_cuda_context *ctx, const drt_film *film, uint32_t width, 
     int rc = drt_ensure_buffer(&ctx->d_denoise, &ctx->denoise_bytes, 3 * npix * sizeof(float));
     if(rc != DRT_CUDA_OK) return rc;
     const float *yw = reinterpret_cast<const float *>(static_cast<const unsigned char *>(ctx->d_rgb_tables) + drt_rgb_tables_yw_offset());
+    if(!ctx->denoise_done) CU(cudaEventCreateWithFlags(&ctx->denoise_done, cudaEventDisableTiming));
+    CU(cudaStreamWaitEvent(stream, ctx->denoise_done, 0));   /* the previous call's filter has read the guide planes */
     drt_launch_denoise_guide(yw, film->mean, film->m2, film->filter, (uint32_t)npix, ctx->n, ctx->d_denoise, ctx->num_sms * 8, stream);
     CU(cudaGetLastError());
     CU(drt_launch_denoise_filter(film->mean, ctx->d_denoise, width, height, ctx->n, (int)opt->search_radius, (int)opt->patch_radius,
                                  opt->strength, out, stream));
+    CU(cudaEventRecord(ctx->denoise_done, stream));
     ctx->launches += 2;
     return DRT_CUDA_OK;
 }

@@ -67,6 +67,9 @@ struct drt_cuda_context
     float *d_deep = nullptr; size_t deep_bytes = 0;     /* overflow rows of deep renders (RenderLaunch::deep) */
     float *d_slice = nullptr; size_t slice_bytes = 0;   /* merged planes of this rank's slice before they are copied to the root */
     float *d_denoise = nullptr; size_t denoise_bytes = 0;   /* the denoise guide planes (drt_denoise.cu) */
+    /* recorded after each denoise filter; the next denoise call's stream waits on it before its guide overwrites d_denoise, so calls
+     * on different streams take the guide planes one after the other */
+    cudaEvent_t denoise_done = nullptr;
     uint64_t launches = 0;
     size_t upload_bytes = 0;
     uint64_t last_launches = 0;

@@ -2,9 +2,9 @@
  * csrc/drt_denoise.cu -- non-local-means denoising of a finished film guided by the film's own statistics (Rousselle, Knaus and
  * Zwicker, "Adaptive rendering with non-local means filtering", 2012).  drt_cuda.h states the filter; this file computes it.
  *
- *   denoise_guide_kernel   per pixel: luminance Y = sum w_l mean_l, its variance bound v = (sum w_l sqrt(M2_l / (n (n - 1))))^2 and
- *                          whether the pixel is usable (n >= 2, finite mean and M2), into three planes of the context's scratch.
- *                          One warp per pixel, wavelengths across lanes (the adaptive rule's Y and err).
+ *   denoise_guide_kernel   per pixel: luminance Y = sum w_l mean_l, its variance bound v = (sum w_l sqrt(max(0, M2_l / (n (n - 1)))))^2
+ *                          and whether the pixel is usable (n >= 2, finite mean and M2, finite f32 Y and v), into three planes of the
+ *                          context's scratch.  One warp per pixel, wavelengths across lanes (the adaptive rule's Y and err).
  *   denoise_filter_kernel  a CTA takes a 32 x 4 tile of output pixels and stages the guide of the tile and its r + f halo in shared
  *                          memory (border replicated).  It walks the search window one row of offsets (dy) at a time: the patch
  *                          distances of all 2r + 1 offsets of the row come from one separable box sum over the tile and its f halo,
@@ -67,11 +67,11 @@ __global__ void __launch_bounds__(256) denoise_guide_kernel(const float *yw, con
             const float m = mean[(size_t)p * n + l], s = m2[(size_t)p * n + l];
             finite = finite && isfinite(m) && isfinite(s);
             y = fmaf(yw[l], m, y);
-            e = fmaf(yw[l], sqrtf(s * inv), e);
+            e = fmaf(yw[l], sqrtf(fmaxf(s * inv, 0.f)), e);   /* a negative M2 counts as zero variance */
         }
 #pragma unroll
         for(int o = 16; o > 0; o >>= 1) { y += __shfl_xor_sync(0xffffffffu, y, o); e += __shfl_xor_sync(0xffffffffu, e, o); }
-        const bool usable = __all_sync(0xffffffffu, finite) && cnt >= 2.f;
+        const bool usable = __all_sync(0xffffffffu, finite) && cnt >= 2.f && isfinite(y) && isfinite(e * e);
         if(lane == 0)
         {
             guide[p] = usable ? y : 0.f;
@@ -146,7 +146,8 @@ __global__ void __launch_bounds__(DN_THREADS) denoise_filter_kernel(const float 
             float s = 0.f;
             for(int j = 0; j < side; j += 1) s += h[j * DN_TX];
             const int dx = dxi - r, qx = x0 + vtx + dx, qy = y0 + vty + dy;
-            const bool in = qx >= 0 && qx < W && qy >= 0 && qy < H && gU[(vty + dy + R) * L.gx + vtx + dx + R] != 0.f;
+            /* a NaN distance (inf - inf of two guides near FLT_MAX) takes weight 0: fmaxf would turn it into 0, a weight of 1 */
+            const bool in = qx >= 0 && qx < W && qy >= 0 && qy < H && gU[(vty + dy + R) * L.gx + vtx + dx + R] != 0.f && !isnan(s);
             float w = in ? __expf(-fmaxf(0.f, s * inv_area)) : 0.f;
             if(dx == 0 && dy == 0) w = 1.f;
             wt[(dxi + DN_KP - 1) * DN_TP + vpix] = w;

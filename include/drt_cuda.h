@@ -209,15 +209,17 @@ int  drt_cuda_film_merge(drt_cuda_context *ctx, const drt_film *dst_device, cons
 /* Non-local-means denoising of a finished film, guided by its own mean and M2 (Rousselle, Knaus and Zwicker, "Adaptive rendering with
  * non-local means filtering", SIGGRAPH Asia 2012).  Reads the mean, m2 and filter planes (sum is ignored and may be NULL) and writes the
  * filtered mean plane [W*H*N] to mean_out, which must not overlap the film's planes; the film is not written.
- *   usable pixel p:  count n_p = filter >= 2 and every mean and m2 value finite
- *   guide:           Y_p = sum_l w_l mean_l(p),  v_p = (sum_l w_l sqrt(m2_l(p) / (n_p (n_p - 1))))^2  (w_l = cmf_y * ref_white, the
- *                    adaptive rule's weights); Y_p = v_p = 0 for an unusable p (they only enter the patches of other pixels)
+ *   usable pixel p:  count n_p = filter >= 2, every mean and m2 value finite, and |Y_p| and v_p at most FLT_MAX (finite as f32)
+ *   guide:           Y_p = sum_l w_l mean_l(p),  v_p = (sum_l w_l sqrt(max(0, m2_l(p) / (n_p (n_p - 1)))))^2  (w_l = cmf_y * ref_white,
+ *                    the adaptive rule's weights; a negative m2 counts as zero variance); Y_p = v_p = 0 for an unusable p (they only
+ *                    enter the patches of other pixels)
  *   distance:        for q = p + d, d in [-r, r]^2, q inside the image and usable:
  *                    D(a, b) = ((Y_a - Y_b)^2 - (v_a + min(v_a, v_b))) / (1e-10 + k^2 (v_a + v_b))
  *                    d2(p, q) = mean over o in [-f, f]^2 of D(clamp(p + o), clamp(q + o))   (clamp replicates the border)
- *   output:          wt(p, q) = exp(-max(0, d2(p, q))), wt(p, p) = 1;  out_l(p) = sum_q wt(p, q) mean_l(q) / sum_q wt(p, q) for a usable p;
- *                    an unusable p is copied bit for bit.
- * r = search_radius 1..15 (default 7), f = patch_radius 0..4 (default 3), k = strength finite and > 0 (default 0.45), else DRT_CUDA_E_ARG;
+ *   output:          wt(p, q) = exp(-max(0, d2(p, q))), or 0 where d2(p, q) is NaN; wt(p, p) = 1;
+ *                    out_l(p) = sum_q wt(p, q) mean_l(q) / sum_q wt(p, q) for a usable p; an unusable p is copied bit for bit.
+ * r = search_radius 1..15 (default 7), f = patch_radius 0..4 (default 3), k = strength in [2^-63, 2^64) so that k^2 is a normal f32
+ * (default 0.45), else DRT_CUDA_E_ARG;
  * also W, H > 0 and the planes present.  N and w come from the uploaded scene (DRT_CUDA_E_STATE without one).  f32 sums in a fixed order:
  * the result is deterministic. */
 typedef struct
@@ -226,7 +228,8 @@ typedef struct
     float    strength;
 } drt_denoise;
 
-/* Stream-ordered: film_device and mean_out_device are device planes. */
+/* Stream-ordered: film_device and mean_out_device are device planes.  Calls on one context may run on different streams: each waits for
+ * the previous call's filter before it overwrites the context's guide scratch. */
 int  drt_cuda_film_denoise(drt_cuda_context *ctx, const drt_film *film_device, uint32_t width, uint32_t height, const drt_denoise *opt,
                            float *mean_out_device, void *stream);
 /* The same on host planes: copies the film up into library-owned device planes, filters, copies the result down and waits. */
