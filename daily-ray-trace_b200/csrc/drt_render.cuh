@@ -80,6 +80,7 @@ template <> struct Num<float>
     static __device__ __forceinline__ float fudge() { return 0.0001f; }
     /* rng() of rng.c:2-7: r31 / RAND_MAX, rounded once to f32 */
     static __device__ __forceinline__ float unit(uint32_t r31) { return __uint2float_rn(r31) * 4.6566128752457969e-10f; }
+    static __device__ __forceinline__ float norm_min() { return 0x1p-126f; }   /* the smallest normal number */
 };
 template <> struct Num<double>
 {
@@ -87,6 +88,7 @@ template <> struct Num<double>
     static __device__ __forceinline__ double inf() { return CUDART_INF; }
     static __device__ __forceinline__ double fudge() { return 0.0001; }
     static __device__ __forceinline__ double unit(uint32_t r31) { return (double)r31 / 2147483647.0; }
+    static __device__ __forceinline__ double norm_min() { return 0x1p-1022; }
 };
 
 /* a / b and 1 / sqrt(x) for operands known to be in range: f32 uses the bare MUFU.RCP / MUFU.RSQ (<= 1-2 ulp) instead of the
@@ -126,16 +128,23 @@ template <typename R> __device__ __forceinline__ V3<R> transmit(V3<R> v, V3<R> n
 }
 
 /* find_rotation_between_vectors((0,0,1), n) applied to q (geometry.c:263-295), in closed form:
- * R q = q + a x q + a x (a x q) / (1 + c) with a = (0,0,1) x n, c = n.z; antiparallel -> -q (Q14). */
+ * R q = q + a x q + a x (a x q) / (1 + c) with a = (0,0,1) x n, c = n.z; antiparallel -> -q (Q14).
+ * The factor is taken as 2 / ((1 + c)^2 + a.a), the same number for a unit n (a.a = 1 - c^2): 1 / (1 + c) cancels near -z, where
+ * in f32 n.z rounds to -1 within 2.4e-4 rad while a.a is still 6e-8.  The antiparallel test is made on the same denominator: below
+ * the normal range (n within 2^-63 rad of -z in f32) the factor would overflow, and -q serves the hemisphere samplers as well as any
+ * rotation.  Without branches and with the a.z = 0 terms dropped, this is shorter than the reference's form.  tests/test_frame_model.py
+ * models this function. */
 template <typename R> __device__ __forceinline__ V3<R> rotate_from_z(V3<R> n, V3<R> q)
 {
     V3<R> a = mk<R>(-n.y, n.x, R(0));
     R c = n.z;
-    if(dot(a, a) == R(0) && c <= R(0)) return neg(q);
-    V3<R> aq = cross(a, q);
-    V3<R> aaq = cross(a, aq);
-    R f = r_div(R(1), R(1) + c);
-    return (q + aq) + aaq * f;
+    R p = R(1) + c;
+    R d = p * p + dot(a, a);
+    V3<R> aq = mk<R>(a.y * q.z, -(a.x * q.z), a.x * q.y - a.y * q.x);        /* cross(a, q) */
+    V3<R> aaq = mk<R>(a.y * aq.z, -(a.x * aq.z), a.x * aq.y - a.y * aq.x);   /* cross(a, aq) */
+    V3<R> r = (q + aq) + aaq * r_div(R(2), d);
+    bool anti = d < Num<R>::norm_min() && c <= R(0);
+    return mk<R>(anti ? -q.x : r.x, anti ? -q.y : r.y, anti ? -q.z : r.z);
 }
 
 /* ------------------------------------------------------------------ per-path random stream (include/drt_rng.h) */

@@ -705,3 +705,11 @@ void drt_oracle_bdsf(const drt_scene *scene, uint32_t surface_material, uint32_t
     p.transmit_material = &scene->materials[transmit_material];
     bdsf(&c, result, &p, v3_make(in_dir));
 }
+
+/* The hemisphere samplers' frame: q (a sample about +z) rotated onto the normal n, as sample_direction does it. */
+void drt_oracle_rotate_from_z(const double *normal, const double *q, double *result)
+{
+    const v3 plus_z = { 0.0, 0.0, 1.0 };
+    v3 v = m3_apply(rotation_between(plus_z, v3_make(normal)), v3_make(q));
+    result[0] = v.x; result[1] = v.y; result[2] = v.z;
+}

@@ -41,6 +41,8 @@ def lib():
         L.drt_oracle_primary_material.argtypes = [C.POINTER(_structs.Scene), C.POINTER(_structs.Camera), C.POINTER(_structs.RenderParams),
                                                   C.c_uint32, C.c_uint32, C.c_uint32]
         L.drt_oracle_primary_material.restype = C.c_int
+        L.drt_oracle_rotate_from_z.argtypes = [dp, dp, dp]
+        L.drt_oracle_rotate_from_z.restype = None
         _lib = L
     return _lib
 
@@ -70,6 +72,14 @@ def bdsf(scene, surf_mat, inc_mat, trans_mat, normal, out_dir, in_dir):
     a = [np.ascontiguousarray(v, dtype=np.float64) for v in (normal, out_dir, in_dir)]
     res = np.zeros(scene.num_wavelengths)
     lib().drt_oracle_bdsf(C.byref(scene), surf_mat, inc_mat, trans_mat, _p(a[0]), _p(a[1]), _p(a[2]), _p(res))
+    return res
+
+
+def rotate_from_z(normal, q):
+    """q, a direction about +z, rotated onto `normal` by the reference's frame (rotation_between((0,0,1), normal))."""
+    a = [np.ascontiguousarray(v, dtype=np.float64) for v in (normal, q)]
+    res = np.zeros(3)
+    lib().drt_oracle_rotate_from_z(_p(a[0]), _p(a[1]), _p(res))
     return res
 
 
